@@ -1,6 +1,6 @@
 """bench.py -- skinned-Chamfer forward+backward throughput of the reart energy evaluation on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg3_16k]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg3_16k] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE full optimisation iteration of the relaxation model (run_robot.py:154-221, --model=base,
@@ -45,7 +45,7 @@ FLOP_PER_PAIR = 8.0                   # 3 FSUB + 1 FMUL + 2 FFMA (BASELINE.md se
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline workload (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg3_16k", choices=sorted(WORKLOADS))
@@ -54,7 +54,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the per-config sweep (N=1) / candidate fits (N>1)")
     ap.add_argument("--sustained-s", type=float, default=10.0, help="seconds of back-to-back steps after the timed region (0: skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, skinned cloud, updated parameters; rank 0's shard) "
+                         "as DIR/<name>.npy in float32, at most 60 MiB in all, for comparing two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times the CPU port, not the engine)")
+    return args
 
 
 def config_dict(args, T, N, P, world):
@@ -356,6 +364,27 @@ def time_engine_steps(engine, ctx, K, W, flush, n_iter=15000, sampler=None):
     return float(tmax.item()) / K, wall, loss
 
 
+DUMP_BYTES = 60 << 20                # under 64 MB with the .npy headers
+
+
+def dump_outputs(engine, loss, out_dir):
+    """What one engine step hands its caller: the loss, the skinned cloud and the parameters after the Adam update, as
+    float32 .npy files.  Beyond DUMP_BYTES in all, the skinned cloud keeps a fixed sample of its points (seed 0, sorted
+    indices), so that two runs with the same arguments write the same arrays."""
+    import numpy as np
+    arrays = {"loss": loss.detach().reshape(1), "skinned": engine.skinned}
+    arrays.update({"param_" + n: p for n, p in engine.model.named_parameters() if p.requires_grad})
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    sk = arrays["skinned"]
+    T, N, _ = sk.shape
+    keep = (DUMP_BYTES - sum(a.nbytes for k, a in arrays.items() if k != "skinned")) // (T * 3 * 4)
+    if keep < N:
+        arrays["skinned"] = sk[:, np.sort(np.random.default_rng(0).choice(N, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
+
+
 def search_kernel_timing(engine, flush, reps=5):
     """The dominant kernel (chamfer_sym_kernel) alone on this rank's shard: CUDA events on the launch stream, L2 flushed."""
     import torch
@@ -573,11 +602,13 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     sampler = ClockSampler(ctx.local_rank, uuid) if ctx.is_main else None
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     ms_per_step, wall_s, loss = time_engine_steps(engine, ctx, K, W, flush, sampler=sampler)
     clocks = sampler.stop() if sampler else None
     value = pairs_per_step / (ms_per_step * 1e-3)
     final_loss = float(loss.item())
+    if args.dump_outputs and ctx.is_main:                # before any later section steps the engine again
+        dump_outputs(engine, loss, args.dump_outputs)
 
     # ---- e2e: host buffers in, loss out, every step.  The H2D of step i+1 (pinned host clouds -> staging buffer, copy
     # stream) runs while step i computes; each step then takes its clouds from the staging buffer (D2D), re-packs the

@@ -61,7 +61,7 @@ def gen_nao(ref):
     out.update(katA_pose=pose.numpy(), katA_part=part.numpy().astype(np.int16), katA_skinned_s16=skinned.numpy()[:, ::16],
                katA_sum_fwd=np.float64(d_f.double().sum().item()), katA_sum_bwd=np.float64(d_b.double().sum().item()),
                katA_idx_fwd=i_f.numpy().astype(np.int16), katA_idx_bwd=i_b.numpy().astype(np.int16),
-               katA_d_fwd=d_f.numpy(), katA_d_bwd=d_b.numpy())
+               katA_d_fwd=d_f.numpy())      # d_b is not stored: no test reads it, and it would take nao.npz past 1 MB
 
     # KAT-B: raw frames 0 <-> 1, bidirectional
     tot, i01, i10 = cd(complete[0:1], complete[1:2], bidirectional=True, return_index=True)

@@ -11,21 +11,14 @@ Golden rows (reference Python on CPU, oracle/make_golden.py::gen_nao_eval, 3 dec
 The relaxation rows are device dependent IN THE REFERENCE: its CPU FPS fallback starts at torch.randint, its CUDA kernel
 at index 0 (SURVEY Q13), and the merging / spanning-tree stage that precedes the rows consumes those samples.  On a GPU
 the reference -- and this package -- follow the CUDA semantics, so the base test is pinned on the fps0 rows.
-
-The companion test at the bottom drives the UNMODIFIED reference script over ``dropin.install()`` when a staged copy of
-the reference is present (``baseline/_ref/reart``, git-ignored, made by scripts/stage_reference.py); it is skipped
-otherwise.
 """
 import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, load_golden
+from conftest import load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -124,28 +117,3 @@ def test_kat_e_base_rows(nao):
     pred = compute_pc_transform(cano, trans_list, seg_part)
     rows = _rows(pred, cano, cano_idx, seg_part, ev)
     _check(rows, golden, ("recon_err", "flow_epe", "flow_acc5", "flow_acc10", "flow_angle", "seg_ri"))
-
-
-STAGED = os.path.join(ROOT, "baseline", "_ref", "reart")
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(STAGED, "utils")),
-                    reason="no staged reference copy (scripts/stage_reference.py makes baseline/_ref/reart)")
-def test_unmodified_run_robot_over_dropin_reproduces_kat_e(tmp_path):
-    """The reference's own run_robot.py, byte for byte, with chamferdist._C / knn_cuda / pointnet2_cuda answered by
-    libreart_b200.so: result.txt must carry the KAT-E rows and the native entry points must have been called."""
-    ev = load_golden("nao_eval.npz")
-    golden = json.loads(str(ev["kin_rows_json"]))
-    summ = tmp_path / "summary.json"
-    cmd = [sys.executable, os.path.join(ROOT, "scripts", "run_reference_dropin.py"), "--backend", "dropin", "--ref-root",
-           STAGED, "--summary", str(summ), "--", f"--seq_path={STAGED}/demo_data/data/nao", f"--save_root={tmp_path}",
-           "--cano_idx=2", "--evaluate", "--model=kinematic",
-           f"--resume={STAGED}/demo_data/pretrained/nao/kinematic-2/model.pth.tar"]
-    subprocess.run(cmd, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=900)
-    s = json.load(open(summ))
-    assert s["status"] == "ok" and s["cuda"]
-    assert s["native_calls"].get("knn_cuda.KNN.__call__", 0) > 0, s["native_calls"]
-    assert any("libreart_b200.so" in p for p in s["native_so_loaded"])
-    rows = s["result_txt"]
-    _check(rows, golden, ("recon_err", "flow_epe", "flow_acc5", "flow_acc10", "flow_angle", "seg_ri"))
-    assert abs(rows["retarget_err"] - golden["retarget_err"]) <= RETARGET_TOL
