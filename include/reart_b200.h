@@ -147,6 +147,26 @@ REART_API int reart_skinned_chamfer_fwd_bwd_culled(const float* cano, const floa
                                                    float* d_fwd, int64_t* i_fwd, float* d_bwd, int64_t* i_bwd,
                                                    int32_t* nn_rows, int32_t* nn_cols, uint64_t* cull_stats,
                                                    void* workspace, int64_t workspace_bytes, void* stream);
+/* The culled evaluation on the CALLER's point order, bit-identical to reart_skinned_chamfer_fwd_bwd_ex on the same
+ * arguments (cano, W, R, tr, tgt in caller order; every output in caller order).  Only the search runs in a permuted order,
+ * where consecutive points are spatially compact: row_order [N] (search position -> caller row of cano) with its inverse
+ * row_inv, tgt_order [T,M] (per frame: search position -> caller target) with tgt_inv; tgt_search [T,M,3] = tgt in
+ * tgt_order, tgt_search_packed its reart_pack_cloud copy.  Culling is exact for any order, and index ties are exact: the
+ * search marks every point whose minimum is reached in two of its chunks, and those take the lowest caller index among
+ * all points at exactly that distance -- the brute force's answer.  Points ordered by caller index inside every 256-row
+ * block and 32-target chunk of the search order are required for the others: a chunk's first match is then its lowest
+ * caller index.  nn_rows [T,N] / nn_cols [T,M] (device, int32, SEARCH order and search indices) are the culling seeds as in
+ * reart_skinned_chamfer_fwd_bwd_culled (-1 / any value: still exact) and are overwritten with this evaluation's arg-mins.
+ * stats (optional, device, [3] uint64, caller-zeroed): += (warp, chunk) pairs evaluated, offered, points resolved by the
+ * tie path. */
+REART_API int reart_skinned_chamfer_fwd_bwd_ordered(const float* cano, const float* W, const float* R, const float* tr,
+                                                    const float* tgt, const float* tgt_search, const float* tgt_search_packed,
+                                                    int64_t T, int64_t N, int64_t M, int64_t P, const int32_t* row_order,
+                                                    const int32_t* row_inv, const int32_t* tgt_order, const int32_t* tgt_inv,
+                                                    float* skinned, double* loss, float* gW, float* gR, float* gtr,
+                                                    float* g_skinned, int compute_grad, float* d_fwd, int64_t* i_fwd,
+                                                    float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
+                                                    uint64_t* stats, void* workspace, int64_t workspace_bytes, void* stream);
 /* The same energy with the skinning FUSED INTO THE PRODUCER SIDE OF THE SEARCH (the composition networks/model.py:63-69 ->
  * utils/chamfer.py:78-94 in one kernel): every search CTA skins its own 2048 canonical points in its prologue and the
  * skinned cloud / x-sorted copy are emitted as by-products, so there is no skinning launch and the cloud is not re-read.

@@ -228,7 +228,7 @@ int64_t reart_energy_workspace_bytes(int64_t T, int64_t N, int64_t M) {
            align_up(T * round_up(N, 256)) + align_up(xq_floats(T, round_up(N, 256)) * 4) +
            align_up(T * N * 24 + 64) + align_up(2 * (int64_t)energy_max_blocks() * 8) +
            align_up(skin_bwd_workspace_floats(T, N, 32) * 4) + align_up(T * (padded_points(M) / kChunk) * 32) +
-           align_up(T * ceil_div(N, 256) * 4) + kAlign;
+           align_up(T * ceil_div(N, 256) * 4) + align_up(T * N * 12) + align_up(T * (N + M) * 4) + kAlign;
 }
 
 int reart_skinned_chamfer_fwd_bwd(const float* cano, const float* W, const float* R, const float* tr, const float* tgt,
@@ -251,11 +251,18 @@ int reart_skinned_chamfer_fwd_bwd_ex(const float* cano, const float* W, const fl
                                                 workspace_bytes, stream_);
 }
 
+// The search order of reart_skinned_chamfer_fwd_bwd_ordered (null everywhere else).
+struct SearchOrder {
+    const int32_t* row_order; const int32_t* row_inv; const int32_t* tgt_order; const int32_t* tgt_inv;
+    const float* tgt_search;      // [T,M,3] the observed frames in tgt_order (tgt_packed is then its packed copy)
+};
+
 static int energy_pipeline(const float* cano, const float* W, const float* hot, const float* R, const float* tr,
                            const float* tgt, const float* tgt_packed, int64_t T, int64_t N, int64_t M, int64_t P,
                            float* skinned, double* loss, float* gW, float* gR, float* gtr, float* g_skinned, int compute_grad,
                            float* d_fwd, int64_t* i_fwd, float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
-                           uint64_t* cull_stats, void* workspace, int64_t workspace_bytes, void* stream_);
+                           uint64_t* cull_stats, void* workspace, int64_t workspace_bytes, void* stream_,
+                           const SearchOrder* order = nullptr);
 
 int reart_skinned_chamfer_fwd_bwd_culled(const float* cano, const float* W, const float* R, const float* tr,
                                          const float* tgt, const float* tgt_packed, int64_t T, int64_t N, int64_t M,
@@ -267,6 +274,22 @@ int reart_skinned_chamfer_fwd_bwd_culled(const float* cano, const float* W, cons
     return energy_pipeline(cano, W, nullptr, R, tr, tgt, tgt_packed, T, N, M, P, skinned, loss, gW, gR, gtr, g_skinned,
                            compute_grad, d_fwd, i_fwd, d_bwd, i_bwd, nn_rows, nn_cols, cull_stats, workspace, workspace_bytes,
                            stream_);
+}
+
+int reart_skinned_chamfer_fwd_bwd_ordered(const float* cano, const float* W, const float* R, const float* tr,
+                                          const float* tgt, const float* tgt_search, const float* tgt_search_packed,
+                                          int64_t T, int64_t N, int64_t M, int64_t P, const int32_t* row_order,
+                                          const int32_t* row_inv, const int32_t* tgt_order, const int32_t* tgt_inv,
+                                          float* skinned, double* loss, float* gW, float* gR, float* gtr, float* g_skinned,
+                                          int compute_grad, float* d_fwd, int64_t* i_fwd, float* d_bwd, int64_t* i_bwd,
+                                          int32_t* nn_rows, int32_t* nn_cols, uint64_t* stats, void* workspace,
+                                          int64_t workspace_bytes, void* stream_) {
+    REART_ENTRY();
+    if (!tgt_search || !row_order || !row_inv || !tgt_order || !tgt_inv || !nn_rows || !nn_cols) return REART_ERR_INVALID_ARG;
+    const SearchOrder order = {row_order, row_inv, tgt_order, tgt_inv, tgt_search};
+    return energy_pipeline(cano, W, nullptr, R, tr, tgt, tgt_search_packed, T, N, M, P, skinned, loss, gW, gR, gtr, g_skinned,
+                           compute_grad, d_fwd, i_fwd, d_bwd, i_bwd, nn_rows, nn_cols, stats, workspace, workspace_bytes,
+                           stream_, &order);
 }
 
 int reart_skinned_chamfer_fwd_bwd_fused(const float* cano, const float* hot, const float* W, const float* R,
@@ -286,7 +309,8 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
                            const float* tgt, const float* tgt_packed, int64_t T, int64_t N, int64_t M, int64_t P,
                            float* skinned, double* loss, float* gW, float* gR, float* gtr, float* g_skinned, int compute_grad,
                            float* d_fwd, int64_t* i_fwd, float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
-                           uint64_t* cull_stats, void* workspace, int64_t workspace_bytes, void* stream_) {
+                           uint64_t* cull_stats, void* workspace, int64_t workspace_bytes, void* stream_,
+                           const SearchOrder* order) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     if (T <= 0 || N <= 0 || M <= 0 || P <= 0 || P > 32 || !fits_int(T) || !fits_int(padded_points(N)) ||
         !fits_int(padded_points(M)))
@@ -310,6 +334,9 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
     const bool cull = nn_rows != nullptr && nn_cols != nullptr;
     float* colbox = cull ? ws.take<float>(T * (padded_points(M) / kChunk) * 8) : nullptr;
     float* rowbound = cull ? ws.take<float>(T * ceil_div(N, 256)) : nullptr;
+    // ordered search: the skinned rows in the search order, and the tie words [T,N] | [T,M] of both sides
+    float* skinned_search = order ? ws.take<float>(T * N * 3) : nullptr;
+    unsigned* tie = order ? ws.take<unsigned>(T * (N + M)) : nullptr;
     if (!ws.ok) return REART_ERR_WORKSPACE;
     long long* acc = reinterpret_cast<long long*>(zero);
     unsigned* ticket = reinterpret_cast<unsigned*>(zero + T * N * 24);
@@ -327,13 +354,18 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
         sp.sk_cano = cano; sp.sk_hot = hot; sp.sk_R = R; sp.sk_tr = tr; sp.sk_P = (int)P; sp.sk_npad = (int)n_pad_sorted;
         sp.sk_out = skinned; sp.sk_sorted = psrc; sp.sk_perm = perm; sp.sk_xq = xq;
     } else {
-        rc = launch_skin_fwd_sorted(cano, W, R, tr, T, N, P, skinned, psrc, perm, xq, n_pad_sorted, stream);
+        rc = launch_skin_fwd_sorted(cano, W, R, tr, T, N, P, skinned, psrc, perm, xq, n_pad_sorted, stream,
+                                    order ? order->row_order : nullptr, skinned_search);
         if (rc) return rc;
+    }
+    if (order) {
+        sp.a = skinned_search;
+        sp.tie_a = tie; sp.tie_b = tie + T * N;
     }
     if (cull) {
         // seeds = the arg-mins of the previous evaluation (nn_* = -1: none, brute force); bounds, then the culled search
         CullParams cp = {};
-        cp.a = skinned; cp.b = tgt; cp.nn_rows = nn_rows; cp.nn_cols = nn_cols;
+        cp.a = sp.a; cp.b = order ? order->tgt_search : tgt; cp.nn_rows = nn_rows; cp.nn_cols = nn_cols;
         cp.B = (int)T; cp.na = (int)N; cp.nb = (int)M; cp.nb_pad = (int)padded_points(M);
         cp.colbox = colbox; cp.rowbound = rowbound;
         cp.coarse = (N >= 8192 && M >= 8192 && N <= 800000 && M <= 800000) ? 1 : 0;   // small clouds: the pass costs more than it saves
@@ -352,6 +384,11 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
     ep.d_fwd = d_fwd; ep.i_fwd = i_fwd; ep.d_bwd = d_bwd; ep.i_bwd = i_bwd;
     ep.nn_rows = nn_rows; ep.nn_cols = nn_cols;                      // the next evaluation's seeds
     ep.src_perm = perm; ep.src_xq = xq; ep.acc = acc; ep.col_bound = col_bound; ep.partials = partials; ep.ticket = ticket;
+    if (order) {
+        ep.row_order = order->row_order; ep.row_inv = order->row_inv; ep.tgt_order = order->tgt_order; ep.tgt_inv = order->tgt_inv;
+        ep.tie_a = sp.tie_a; ep.tie_b = sp.tie_b;
+        ep.ties = cull_stats ? reinterpret_cast<unsigned long long*>(cull_stats) + 2 : nullptr;
+    }
     rc = launch_energy_bwd(ep, stream);
     if (rc || !compute_grad) return rc;
     return launch_skin_bwd(cano, W, R, tr, gs, T, N, P, gW, gR, gtr, bwd_partials, stream);

@@ -352,12 +352,21 @@ __global__ void __launch_bounds__(kSymThreads, 2) chamfer_sym_kernel(const SymPa
 //     issues the next TMA into it, so the warps drift apart by up to kCullStages - 1 tiles and the per-tile maxima
 //     average out.
 // Same keys as the brute force, bit for bit (tests/test_cull_gpu.py).
+//
+// TIES = true also leaves a per-point TIE WORD (p.tie_a / p.tie_b, 0xffffffff on entry): the smallest distance, as bits, at
+// which two DIFFERENT chunks were seen to reach the same value.  A search over a permuted copy of the clouds needs it: a
+// key names the first chunk of the SEARCH order that reaches the minimum, while the caller's semantics is the lowest
+// index of the CALLER's order, so a point whose minimum is reached in two chunks (tie word == final distance) must be
+// resolved exactly by the consumer (energy.cu).  Detection is exact: a row folds every chunk into a chunk-local minimum
+// (same min3 count as the running one) and compares it with the running minimum at the chunk's end; partial results of
+// different work items meet through atomicMin, whose returned old value shows a tie -- of two minimum-attaining chunks,
+// the one that merges second sees the first one's value.  A skipped chunk cannot hold a minimum (the skip test is strict).
 constexpr int kCullStages = 6;
 constexpr int kCullTileChunks = 16;
 constexpr int kCullTileBytes = kCullTileChunks * kChunk * 12;
 constexpr int kCullStageBytes = kCullTileBytes + kCullTileChunks * kBoxFloats * 4;
 
-template <int NT>
+template <int NT, bool TIES>
 __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const SymParams p) {
     constexpr int kWarps = NT / 32;
     constexpr int R = 8;
@@ -401,8 +410,9 @@ __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const Sy
     }
 
     u64 QX[R], QY[R], QZ[R];
-    float best[R], prev[R];
+    float best[R], prev[R];                                    // TIES: prev is the chunk-local minimum
     unsigned bch[R];
+    unsigned tied = 0u;                                        // TIES: bit r = row r's running minimum is reached in two chunks
     float rlx = INFINITY, rly = INFINITY, rlz = INFINITY, rhx = -INFINITY, rhy = -INFINITY, rhz = -INFINITY;
 #pragma unroll
     for (int r = 0; r < R; ++r) {
@@ -448,6 +458,10 @@ __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const Sy
             ++evaluated;
             const float4* __restrict__ cg = tile + c * (kChunk / 4 * 3);
             unsigned mine = 0x7f800000u;                       // the warp's minimum for target (this lane) of the chunk
+            if (TIES) {
+#pragma unroll
+                for (int r = 0; r < R; ++r) prev[r] = INFINITY;
+            }
 #pragma unroll
             for (int g = 0; g < kChunk / 4; ++g) {
                 const float4 X = cg[3 * g], Y = cg[3 * g + 1], Z = cg[3 * g + 2];
@@ -460,8 +474,9 @@ __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const Sy
                     float a0, a1, a2, a3;
                     unpack2(sqdist_pair(QX[r], QY[r], QZ[r], X01, Y01, Z01), a0, a1);
                     unpack2(sqdist_pair(QX[r], QY[r], QZ[r], X23, Y23, Z23), a2, a3);
-                    best[r] = min3(best[r], a0, a1);
-                    best[r] = min3(best[r], a2, a3);
+                    float& acc = TIES ? prev[r] : best[r];
+                    acc = min3(acc, a0, a1);
+                    acc = min3(acc, a2, a3);
                     if (r == 0) { c0 = a0; c1 = a1; c2 = a2; c3 = a3; }
                     else { c0 = fminf(c0, a0); c1 = fminf(c1, a1); c2 = fminf(c2, a2); c3 = fminf(c3, a3); }
                 }
@@ -474,12 +489,18 @@ __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const Sy
             const unsigned gid = (unsigned)(chunk0 + k * kCullTileChunks + c);
 #pragma unroll
             for (int r = 0; r < R; ++r) {
-                if (best[r] < prev[r]) bch[r] = gid;
-                prev[r] = best[r];
+                if (TIES) {
+                    if (prev[r] < best[r]) { best[r] = prev[r]; bch[r] = gid; tied &= ~(1u << r); }
+                    else if (prev[r] == best[r]) tied |= 1u << r;
+                } else {
+                    if (best[r] < prev[r]) bch[r] = gid;
+                    prev[r] = best[r];
+                }
             }
             const int j = (int)gid * kChunk + lane;
             if (j < p.nb && mine <= __float_as_uint(b1.z)) {   // <=: a tie with the bound can still be the final minimum
-                atomicMin(&keys_col[j], ((u64)mine << 32) | colchunk);
+                const u64 old = atomicMin(&keys_col[j], ((u64)mine << 32) | colchunk);
+                if (TIES && (unsigned)(old >> 32) == mine) atomicMin(p.tie_b + (int64_t)b * p.nb + j, mine);   // another row chunk
                 if (mine < 0x7f800000u) cmax = max(cmax, mine);
             }
         }
@@ -511,9 +532,16 @@ __global__ void __launch_bounds__(NT, 512 / NT) chamfer_sym_cull_kernel(const Sy
     for (int r = 0; r < R; ++r) {
         const int i = qbase + warp * (32 * R) + lane * R + r;
         if (i < p.na) {
-            const u64 key = ((u64)__float_as_uint(best[r]) << 32) | (u64)bch[r];
-            if (p.splits == 1) keys_row[i] = key;
-            else atomicMin(&keys_row[i], key);
+            const unsigned d = __float_as_uint(best[r]);
+            const u64 key = ((u64)d << 32) | (u64)bch[r];
+            unsigned tie = ((tied >> r) & 1u) ? d : 0xffffffffu;
+            if (p.splits == 1) {
+                keys_row[i] = key;
+            } else {
+                const u64 old = atomicMin(&keys_row[i], key);
+                if (TIES && (unsigned)(old >> 32) == d) tie = d;     // the other split's chunks are different chunks
+            }
+            if (TIES && tie != 0xffffffffu) atomicMin(p.tie_a + (int64_t)b * p.na + i, tie);
         }
     }
 }
@@ -604,6 +632,8 @@ static int launch_sym_cull(SymParams& p, cudaStream_t stream) {
     const int64_t items = (int64_t)p.B * p.qblocks * p.splits;
     if (items <= 0) return kOk;
     if (items > 0x7fffffff) return kErrUnsupported;
+    if (p.tie_a && cudaMemsetAsync(p.tie_a, 0xff, sizeof(unsigned) * (size_t)p.B * (p.na + p.nb), stream) != cudaSuccess)
+        return kErrLaunch;                                     // [tie_a | tie_b] are one array
     if (!p.keys_preset) {
         // every column key is merged by atomicMin here (no CTA-level fold), row keys when the targets are split
         const size_t bytes_a = sizeof(u64) * (size_t)p.B * p.na, bytes_b = sizeof(u64) * (size_t)p.B * p.nb;
@@ -617,8 +647,13 @@ static int launch_sym_cull(SymParams& p, cudaStream_t stream) {
         }
     }
     const size_t smem = (size_t)kCullStages * kCullStageBytes;
-    if (nt == 256) chamfer_sym_cull_kernel<256><<<(unsigned)items, 256, smem, stream>>>(p);
-    else chamfer_sym_cull_kernel<128><<<(unsigned)items, 128, smem, stream>>>(p);
+    if (p.tie_a) {
+        if (nt == 256) chamfer_sym_cull_kernel<256, true><<<(unsigned)items, 256, smem, stream>>>(p);
+        else chamfer_sym_cull_kernel<128, true><<<(unsigned)items, 128, smem, stream>>>(p);
+    } else {
+        if (nt == 256) chamfer_sym_cull_kernel<256, false><<<(unsigned)items, 256, smem, stream>>>(p);
+        else chamfer_sym_cull_kernel<128, false><<<(unsigned)items, 128, smem, stream>>>(p);
+    }
     REART_CHECK_LAUNCH();
     return kOk;
 }
@@ -634,7 +669,7 @@ int launch_chamfer_sym(SymParams& p, cudaStream_t stream) {
         return launch_sym_rs<8, 1, false, true>(p, stream);
     }
     if (p.cull) {
-        if (!p.colbox || !p.rowbound) return kErrInvalidArg;
+        if (!p.colbox || !p.rowbound || (p.tie_a && p.tie_b != p.tie_a + (int64_t)p.B * p.na)) return kErrInvalidArg;
         p.row_chunks = (int)ceil_div(p.na, 256);
         if (p.variant == 1) return launch_sym_rs<8, 1, true>(p, stream);      // the barrier-per-tile culled kernel (comparison)
         return launch_sym_cull(p, stream);

@@ -50,6 +50,8 @@ struct SymParams {
     const float* rowbound;        // [B, ceil(na/256)]: upper bound of the final minima of each 256-row chunk
     int row_chunks;               // filled by the launcher
     unsigned long long* cull_stats;   // null, or [2] (zero on entry): (warp, chunk) pairs evaluated / offered
+    unsigned* tie_a;              // null, or [B,na] followed by tie_b [B,nb]: tie words of the culled search (chamfer_sym.cu
+    unsigned* tie_b;              // TIES), set to 0xffffffff by the launcher
     // fused producer (chamfer_sym.cu SKIN = true): sk_cano != null -> `a` is not read, the rows are skinned in the kernel
     const float* sk_cano;         // [na,3] canonical cloud
     const float* sk_hot;          // [na,2] one-hot weights in compact form: (part as int bits, weight value)
@@ -89,9 +91,11 @@ int launch_chamfer_bidir_bwd(const float* src, const float* tgt, const int64_t* 
 
 int launch_skin_fwd(const float* cano, const float* W, const float* R, const float* tr, int64_t T, int64_t N, int64_t P,
                     float* out, float* out_packed, cudaStream_t stream);
+// order != null: the sorted copy (and out_search [T,N,3], AoS) holds the points in the order `order` [N] (search position ->
+// caller point); `out` stays in caller order
 int launch_skin_fwd_sorted(const float* cano, const float* W, const float* R, const float* tr, int64_t T, int64_t N,
                            int64_t P, float* out, float* out_packed, unsigned char* perm, float* xq, int64_t n_pad,
-                           cudaStream_t stream);
+                           cudaStream_t stream, const int32_t* order = nullptr, float* out_search = nullptr);
 int64_t skin_bwd_workspace_floats(int64_t T, int64_t N, int64_t P);
 int launch_skin_bwd(const float* cano, const float* W, const float* R, const float* tr, const float* g, int64_t T,
                     int64_t N, int64_t P, float* gW, float* gR, float* gtr, float* partials, cudaStream_t stream);
@@ -141,6 +145,15 @@ struct EnergyParams {
     int32_t* nn_rows; int32_t* nn_cols;   // optional [B,N] / [B,M]: the arg-mins, kept as the next evaluation's culling seeds
     float* d_fwd; int64_t* i_fwd; // optional [B,N]
     float* d_bwd; int64_t* i_bwd; // optional [B,M]
+    // search in a permuted order (all null: the keys are in caller order).  The search ran on row_order / tgt_order copies
+    // (src_packed, tgt_packed, keys, tie words and nn_* are in that order); both passes still iterate in caller order.
+    const int32_t* row_order;     // [N]   search position -> caller row
+    const int32_t* row_inv;       // [N]   caller row -> search position
+    const int32_t* tgt_order;     // [B,M] per frame: search position -> caller target
+    const int32_t* tgt_inv;       // [B,M]
+    const unsigned* tie_a;        // [B,N] / [B,M] tie words of the search (SymParams::tie_a)
+    const unsigned* tie_b;
+    unsigned long long* ties;     // null, or [1]: += number of points resolved by the exact tie path
 };
 int energy_max_blocks();
 int launch_energy_bwd(const EnergyParams& p, cudaStream_t stream);

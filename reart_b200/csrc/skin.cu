@@ -88,7 +88,9 @@ int launch_skin_fwd(const float* cano, const float* W, const float* R, const flo
 // sorted position k and xq[t][block][16] = x at sorted positions 15, 31, ..., 255 (the quantile index the column-side
 // index recovery probes first, common.cuh rescan_sorted_chunk_q).  The recovery then looks at the x window
 // |b.x - a.x| <= sqrt(dmin) instead of testing all 256 candidates.
-// The AoS output keeps the original order -- it is what the search and every consumer read.
+// The AoS output keeps the original order -- it is what the search and every consumer read.  With a search order
+// (`order`, the ordered pipeline of capi.cu) the blocks are 256 consecutive points OF THAT ORDER, and the same points are
+// also written in that order to out_search: the rows of a search over permuted copies.
 constexpr int kSortBlock = 256;
 
 __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted_kernel(const float* __restrict__ cano,
@@ -98,7 +100,9 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted_kernel(const float
                                                                      float* __restrict__ out,
                                                                      float* __restrict__ out_packed,
                                                                      unsigned char* __restrict__ perm,
-                                                                     float* __restrict__ xq, int n_pad, int fpb) {
+                                                                     float* __restrict__ xq, int n_pad, int fpb,
+                                                                     const int32_t* __restrict__ order,
+                                                                     float* __restrict__ out_search) {
     extern __shared__ __align__(16) unsigned char sm_raw[];
     u64* xchg = reinterpret_cast<u64*>(sm_raw);                               // [256]
     float* sx = reinterpret_cast<float*>(xchg + kSortBlock);                  // [3][256]
@@ -113,11 +117,12 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted_kernel(const float
     __syncthreads();
     const int i = threadIdx.x;
     const int base = blockIdx.x * kSortBlock;
-    const int n = base + i;
+    const int n = base + i;                                                   // position in the sorted copy's order
     const bool real = n < N;
+    const int c = (order && real) ? order[n] : n;                             // the caller's point
     float cx = 0.f, cy = 0.f, cz = 0.f;
-    if (real) { cx = cano[3 * n]; cy = cano[3 * n + 1]; cz = cano[3 * n + 2]; }
-    const float* __restrict__ w = W + (int64_t)(real ? n : 0) * P;
+    if (real) { cx = cano[3 * c]; cy = cano[3 * c + 1]; cz = cano[3 * c + 2]; }
+    const float* __restrict__ w = W + (int64_t)(real ? c : 0) * P;
     const int nblk = n_pad / kSortBlock;
     for (int f = 0; f < nt; ++f) {
         float ax = INFINITY, ay = INFINITY, az = INFINITY;                    // padding sorts last
@@ -134,8 +139,12 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted_kernel(const float
                     az = __fmaf_rn(wp, skin_axis(cx, cy, cz, m[6], m[7], m[8], m[11]), az);
                 }
             }
-            float* o = out + ((int64_t)(t0 + f) * N + n) * 3;
+            float* o = out + ((int64_t)(t0 + f) * N + c) * 3;
             o[0] = ax; o[1] = ay; o[2] = az;
+            if (out_search) {
+                float* os = out_search + ((int64_t)(t0 + f) * N + n) * 3;
+                os[0] = ax; os[1] = ay; os[2] = az;
+            }
         }
         sx[i] = ax; sx[kSortBlock + i] = ay; sx[2 * kSortBlock + i] = az;      // visible after the sort's first barrier
         const u64 key = block_bitonic_sort256(((u64)orderable_bits(ax) << 32) | (u64)i, xchg);
@@ -162,7 +171,9 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted8_kernel(const floa
                                                                       float* __restrict__ out,
                                                                       float* __restrict__ out_packed,
                                                                       unsigned char* __restrict__ perm,
-                                                                      float* __restrict__ xq, int n_pad) {
+                                                                      float* __restrict__ xq, int n_pad,
+                                                                      const int32_t* __restrict__ order,
+                                                                      float* __restrict__ out_search) {
     extern __shared__ __align__(16) unsigned char sm_raw[];
     float* sx = reinterpret_cast<float*>(sm_raw);                             // [8 frames][3][256]
     float* sm_tf = sx + kSortFrames * 3 * kSortBlock;                         // [8][P][12]
@@ -176,11 +187,12 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted8_kernel(const floa
     __syncthreads();
     const int i = threadIdx.x;
     const int base = blockIdx.x * kSortBlock;
-    const int n = base + i;
+    const int n = base + i;                                                   // position in the sorted copy's order
     const bool real = n < N;
+    const int c = (order && real) ? order[n] : n;                             // the caller's point
     float cx = 0.f, cy = 0.f, cz = 0.f;
-    if (real) { cx = cano[3 * n]; cy = cano[3 * n + 1]; cz = cano[3 * n + 2]; }
-    const float* __restrict__ w = W + (int64_t)(real ? n : 0) * P;
+    if (real) { cx = cano[3 * c]; cy = cano[3 * c + 1]; cz = cano[3 * c + 2]; }
+    const float* __restrict__ w = W + (int64_t)(real ? c : 0) * P;
     // the weight row is read ONCE: rows with at most two non-zeros (one-hot / straight-through rows have one) are kept in
     // registers for all 8 frames; denser rows re-read it per frame.  Non-zeros are applied in increasing p either way.
     int p0 = 0, p1 = 0, nnz = 0;
@@ -224,8 +236,12 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted8_kernel(const floa
                     }
                 }
             }
-            float* o = out + ((int64_t)(t0 + f) * N + n) * 3;
+            float* o = out + ((int64_t)(t0 + f) * N + c) * 3;
             o[0] = ax; o[1] = ay; o[2] = az;
+            if (out_search) {
+                float* os = out_search + ((int64_t)(t0 + f) * N + n) * 3;
+                os[0] = ax; os[1] = ay; os[2] = az;
+            }
         }
         float* s = sx + f * 3 * kSortBlock;
         s[i] = ax; s[kSortBlock + i] = ay; s[2 * kSortBlock + i] = az;
@@ -257,7 +273,7 @@ __global__ void __launch_bounds__(kSortBlock) skin_fwd_sorted8_kernel(const floa
 
 int launch_skin_fwd_sorted(const float* cano, const float* W, const float* R, const float* tr, int64_t T, int64_t N,
                            int64_t P, float* out, float* out_packed, unsigned char* perm, float* xq, int64_t n_pad,
-                           cudaStream_t stream) {
+                           cudaStream_t stream, const int32_t* order, float* out_search) {
     if (T <= 0 || N <= 0) return kOk;
     if (P <= 0 || P > 32 || n_pad % kSortBlock != 0 || n_pad < N) return kErrUnsupported;
     int fpb = kSkinFramesPerBlock;
@@ -266,14 +282,14 @@ int launch_skin_fwd_sorted(const float* cano, const float* W, const float* R, co
         dim3 grid8((unsigned)(n_pad / kSortBlock), (unsigned)ceil_div(T, kSortFrames));
         const size_t smem8 = ((size_t)kSortFrames * 3 * kSortBlock + (size_t)kSortFrames * P * 12) * sizeof(float);
         skin_fwd_sorted8_kernel<<<grid8, kSortBlock, smem8, stream>>>(cano, W, R, tr, (int)T, (int)N, (int)P, out, out_packed,
-                                                                      perm, xq, (int)n_pad);
+                                                                      perm, xq, (int)n_pad, order, out_search);
         REART_CHECK_LAUNCH();
         return kOk;
     }
     dim3 grid((unsigned)(n_pad / kSortBlock), (unsigned)ceil_div(T, fpb));
     const size_t smem = (size_t)kSortBlock * (8 + 12) + (size_t)fpb * P * 12 * sizeof(float);
     skin_fwd_sorted_kernel<<<grid, kSortBlock, smem, stream>>>(cano, W, R, tr, (int)T, (int)N, (int)P, out, out_packed,
-                                                               perm, xq, (int)n_pad, fpb);
+                                                               perm, xq, (int)n_pad, fpb, order, out_search);
     REART_CHECK_LAUNCH();
     return kOk;
 }

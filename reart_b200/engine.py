@@ -39,6 +39,9 @@ class _EngineBase:
             self.cano.copy_(cano_src)
             self.frames.copy_(frames_src)
             ops.pack_cloud(self.frames, out=self.frames_packed)
+            if getattr(self, "search_culled", False):
+                torch.gather(self.frames, 1, self._search_gather, out=self.frames_search)
+                ops.pack_cloud(self.frames_search, out=self.frames_search_packed)
         if getattr(self, "native", False):
             return self._run_iteration_native()
         if getattr(self, "sink", None) is not None:
@@ -169,6 +172,11 @@ class _EngineBase:
         pass
 
 
+# search="auto" runs the culled search from this many points per cloud on (both clouds): the coarse bounds of cull.cu
+# start culling there
+SEARCH_CULLED_MIN_POINTS = 8192
+
+
 class RelaxationEngine(_EngineBase):
     """Relaxation model (networks/model.py BaseModel) + recon loss, frame-sharded."""
 
@@ -176,14 +184,18 @@ class RelaxationEngine(_EngineBase):
                  trans_lr: float = 1e-2, seg_lr: float = 1e-3, weight_decay: float = 0.0, use_graph: bool = True,
                  seed: int = 2, flow_ref=None, cano_idx: int = 0, lambda_flow: float = 1.0, robust_flow: bool = False,
                  native: Optional[bool] = None, betas=(0.9, 0.999), eps: float = 1e-8, assign: Optional[dict] = None,
-                 cull: Optional[bool] = None, fuse_producer: bool = False):
+                 cull: Optional[bool] = None, fuse_producer: bool = False, search: str = "auto"):
         """assign: optional dict(downsample=4, assign_gap=5, lambda_assign=0.3, assign_iter=0, mode="add"|"replace")
         enabling the assignment loss (run_robot.py:164-187): from iteration ``assign_iter`` on it is ADDED to the Chamfer
         loss (run_real.py / run_sapien.py) or REPLACES it (run_robot.py's if/else, SURVEY Q12); assignments are refreshed
         on the GPU (``reart_lap``) at ``assign_iter`` and whenever ``i % assign_gap == 0``, inside the captured iteration.
         flow_ref: optional ``flow_utils.FlowReference`` (run_robot.py:78-84) enabling the flow loss of
         run_robot.py:194-213.  Consecutive frames couple across shard boundaries: under frame sharding each rank
-        receives one skinned frame per iteration from the previous rank (``dist.halo_from_previous_rank``)."""
+        receives one skinned frame per iteration from the previous rank (``dist.halo_from_previous_rank``).
+        search: "brute" evaluates every pair; "culled" runs the exact culled search on k-d ordered copies of the clouds
+        while everything else stays in the caller's order -- bit-identical to "brute" (native fused iteration only);
+        "auto" picks "culled" from ``SEARCH_CULLED_MIN_POINTS`` points per cloud on, where the coarse bounds of cull.cu make
+        it faster.  ``cull=True`` (the engine reorders the caller's clouds) and ``fuse_producer=True`` search brute force."""
         super().__init__(ctx, use_graph)
         self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
         # the flow loss couples consecutive frames: under frame sharding each rank evaluates the pairs whose second
@@ -197,11 +209,11 @@ class RelaxationEngine(_EngineBase):
         self.total_frames = int(frames.shape[0])
         self.cano = cano.float().contiguous()
         self.frames = frames[lo:hi].float().contiguous()          # local shard of the observed frames
-        # Exact tile culling (csrc/cull.cu), opt-in (cull=True; native fused iteration only).  The loss is invariant to the
-        # order of the points inside a cloud, so both clouds are put into k-d leaf order ONCE here (256-point leaves for
-        # the canonical cloud = one warp of the search, 32-point leaves for the observed frames = one target chunk);
-        # ``perm_cano`` / ``perm_frames`` map engine order -> caller order (engine.skinned[:, k] is caller point perm_cano[k]).
-        # The brute-force search stays the default: it is the kernel the roofline is quoted on and the order-preserving path.
+        # cull=True: the engine's own clouds are put into k-d leaf order ONCE here (256-point leaves for the canonical
+        # cloud = one warp of the search, 32-point leaves for the observed frames = one target chunk); ``perm_cano`` /
+        # ``perm_frames`` map engine order -> caller order (engine.skinned[:, k] is caller point perm_cano[k]).  Every
+        # order-dependent float sum then associates differently: the same optimisation, not the same bits.  The default
+        # (search="auto") culls without this: only the search runs on k-d ordered copies (search_order_rows / _tgt).
         self.cull = bool(cull) if cull is not None else False
         # fuse_producer: skin inside the search kernel's prologue (reart_skinned_chamfer_fwd_bwd_fused; SURVEY N1).  Bit-identical,
         # one launch less, but measured SLOWER than the separate skin kernel on B200 (profiles/r02_fused_producer.md), so opt-in.
@@ -209,6 +221,14 @@ class RelaxationEngine(_EngineBase):
         if self.cull and (flow_ref is not None or native is False):
             raise ValueError("exact tile culling runs on the native fused iteration (recon / assignment losses)")
         self.perm_cano = self.perm_frames = None
+        if search not in ("auto", "brute", "culled"):
+            raise ValueError("search must be 'auto', 'brute' or 'culled'")
+        native_path = (flow_ref is None) if native is None else bool(native)
+        can_order = native_path and not self.cull and not self.fuse_producer
+        if search == "culled" and not can_order:
+            raise ValueError("search='culled' runs on the native fused iteration, without cull=True or fuse_producer=True")
+        self.search_culled = can_order and (search == "culled" or (
+            search == "auto" and min(self.cano.shape[0], self.frames.shape[1]) >= SEARCH_CULLED_MIN_POINTS))
         cano_orig, frames_orig = self.cano, self.frames
         if self.cull:
             # k-d order refined well below the chunk sizes of the search (256 rows / 32 targets): the chunks stay the same
@@ -218,6 +238,22 @@ class RelaxationEngine(_EngineBase):
             self.cano = self.cano[self.perm_cano].contiguous()
             self.frames = torch.gather(self.frames, 1, self.perm_frames[:, :, None].expand(-1, -1, 3)).contiguous()
         self.frames_packed = ops.pack_cloud(self.frames)          # constant over the optimisation: packed once
+        self.search_order_rows = self.search_order_tgt = None
+        if self.search_culled:
+            # the culled search's own order, fixed here (256-row blocks = one warp of the search, 32-target chunks); the
+            # engine's clouds, outputs and every sum stay in the caller's order.  Any order is exact, a stale one (after
+            # step(ingest=...)) only culls less.
+            self.search_order_rows = ops.search_order(self.cano[None], 256)[0].int()
+            self.search_order_tgt = ops.search_order(self.frames, 32).int()
+            self.search_inv_rows = torch.empty_like(self.search_order_rows)
+            self.search_inv_rows[self.search_order_rows.long()] = torch.arange(
+                self.cano.shape[0], dtype=torch.int32, device=dev)
+            self.search_inv_tgt = torch.empty_like(self.search_order_tgt)
+            self.search_inv_tgt.scatter_(1, self.search_order_tgt.long(), torch.arange(
+                self.frames.shape[1], dtype=torch.int32, device=dev)[None].expand_as(self.search_order_tgt).contiguous())
+            self._search_gather = self.search_order_tgt.long()[:, :, None].expand(-1, -1, 3)
+            self.frames_search = torch.gather(self.frames, 1, self._search_gather).contiguous()
+            self.frames_search_packed = ops.pack_cloud(self.frames_search)
         torch.manual_seed(seed)                                    # identical init + gumbel draws on every rank
         torch.cuda.manual_seed_all(seed)
         self.model = BaseModel(num_parts=num_parts, pose_len=hi - lo).to(dev)
@@ -293,10 +329,11 @@ class RelaxationEngine(_EngineBase):
         b["bucket"] = torch.zeros(nseg + 1, **f32)
         b["loss_out"] = torch.zeros(1, **f32)
         b["dims"] = (T, N, M, P, H)
-        if self.cull:                                            # arg-mins carried from step to step (-1: none yet)
+        if self.cull or self.search_culled:                      # arg-mins carried from step to step (-1: none yet)
             b["nn_rows"] = torch.full((T, N), -1, dtype=torch.int32, device=dev)
             b["nn_cols"] = torch.full((T, M), -1, dtype=torch.int32, device=dev)
-            b["cull_stats"] = torch.zeros(2, dtype=torch.int64, device=dev)
+            # evaluated / offered (warp, chunk) pairs; ordered search: + points resolved by the exact tie path
+            b["cull_stats"] = torch.zeros(3 if self.search_culled else 2, dtype=torch.int64, device=dev)
         red = self.sink.reducer if self.sink is not None else None
         self.model.seg_head.grad_sink = None                     # the autograd sink is not used on this path
         oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
@@ -334,7 +371,7 @@ class RelaxationEngine(_EngineBase):
 
     def _aux_state_tensors(self):
         aux = [self.assign.col4row, self.assign.dual_u] if self.assign is not None else []
-        if self.native and self.cull:
+        if self.native and (self.cull or self.search_culled):
             aux += [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
         return aux
 
@@ -363,7 +400,14 @@ class RelaxationEngine(_EngineBase):
         step's arg-mins (bit-identical results)."""
         from ._lib import check, ptr, stream_ptr
         m = self.model
-        if self.cull:
+        if self.search_culled:
+            check(L.reart_skinned_chamfer_fwd_bwd_ordered(
+                ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_search),
+                ptr(self.frames_search_packed), T, N, M, P, ptr(self.search_order_rows), ptr(self.search_inv_rows),
+                ptr(self.search_order_tgt), ptr(self.search_inv_tgt), ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR),
+                ptr(gtr), ptr(g_skinned), compute_grad, None, None, None, None, ptr(b["nn_rows"]), ptr(b["nn_cols"]),
+                ptr(b["cull_stats"]), ptr(b["ws"]), b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_ordered")
+        elif self.cull:
             check(L.reart_skinned_chamfer_fwd_bwd_culled(
                 ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_packed), T, N, M, P,
                 ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr), ptr(g_skinned), compute_grad, None, None, None,
@@ -383,11 +427,20 @@ class RelaxationEngine(_EngineBase):
 
     def culling_stats(self):
         """(evaluated, offered) (warp, 32-target chunk) pairs since the last call; resets the counters.  Host sync."""
-        if not (self.native and self.cull):
+        if not (self.native and (self.cull or self.search_culled)):
             return None
-        ev, off = (int(x) for x in self._nat["cull_stats"].tolist())
-        self._nat["cull_stats"].zero_()
+        ev, off = (int(x) for x in self._nat["cull_stats"][:2].tolist())
+        self._nat["cull_stats"][:2].zero_()
         return ev, off
+
+    def flagged_ties(self):
+        """Points the culled search saw reach their minimum in two of its chunks, resolved by the exact tie path, since
+        the last call (resets the counter; None unless search is culled).  Host sync."""
+        if not self.search_culled:
+            return None
+        n = int(self._nat["cull_stats"][2])
+        self._nat["cull_stats"][2].zero_()
+        return n
 
     def _run_iteration_native(self):
         """head -> [memset, skin (x-sorted copy), search, energy columns, energy rows, skin backward, reduce] -> tail."""

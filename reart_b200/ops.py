@@ -501,6 +501,16 @@ def kd_order(points: torch.Tensor, leaf: int) -> torch.Tensor:
     return idx
 
 
+def search_order(points: torch.Tensor, leaf: int) -> torch.Tensor:
+    """``kd_order`` [B,N] with the points of every leaf (``leaf`` consecutive positions) put back in ascending caller index.
+    Leaf membership, and so what the culled search skips, is unchanged; the first exact match inside a leaf is then the
+    lowest caller index, which is what ``reart_skinned_chamfer_fwd_bwd_ordered`` needs to return the brute force's ties."""
+    order = kd_order(points, leaf)
+    n = order.shape[1]
+    leaf_of = torch.arange(n, device=order.device) // leaf
+    return torch.sort(leaf_of[None] * n + order, dim=1).values % n
+
+
 def fp32_probe(variant: int, iters: int = 2000, blocks: int | None = None, device=None):
     """Run one FP32 pipe micro-benchmark; returns (ms, lane_ops_total)."""
     L = _lib.lib()
