@@ -241,6 +241,46 @@ REART_API int64_t reart_relax_tail_ticket_words(int64_t N);
 REART_API int reart_relax_tail(const reart_relax_tail_args* args, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * One iteration of the kinematic (projection) model (run_robot.py's second model, --model=kinematic), fused around the
+ * energy (reart_skinned_chamfer_fwd_bwd / _ordered with the constant one-hot weights of the label transfer).
+ * head: KinematicModel.transforms (networks/model.py:151-159): tree forward kinematics of reart_fk_fwd
+ *       (utils/kinematic_utils.py:151-198, same tree arrays, same device arithmetic) followed by the optional learned
+ *       root pose root @ fk, root = [rotation_6d_to_matrix(root_6d) | root_t] (networks/model.py:155-158).
+ *       axis, moment [E,3], theta [T,E], distance [T,E] or NULL, joint_type [E] or NULL; root_6d [T,6] and root_t [T,3]
+ *       both or neither -> R [T,P,3,3], tr [T,P,3] (the energy's pose inputs; without a root pose bit-identical to
+ *       reart_fk_fwd's [..., :3, :3] / [..., :3, 3]) and fk [T,P,12] (the 3x4 poses before the root pose, for the tail).
+ * tail: the backward of head given d loss / d (R, tr) from the energy (dual-number screw derivatives, frame sums in frame
+ *       order -- no float atomics, bit-reproducible), [frames sharded over `world` ranks: the one-shot peer-memory
+ *       all-reduce of reart_allreduce_oneshot, inline, on grad[0 .. 6E]] and Adam with torch.optim.Adam semantics and one
+ *       learning rate (run_robot.py:146-150, 219-221 as the kinematic run builds it) on every parameter, in ONE launch.
+ *       grad (written) = [g_axis 3E | g_moment 3E | loss | g_theta T*E | g_distance T*E (with distance) | g_root_6d 6T,
+ *       g_root_t 3T (with a root pose)]; m, v: Adam moments in the same layout; step [1] counts completed steps.
+ *       phase 0: everything; 1: gradients only (the caller reduces grad[0 .. 6E], e.g. with NCCL); 2: Adam from grad.
+ * P <= 32; joint_type values as in reart_fk_fwd.
+ * ------------------------------------------------------------------------------------------- */
+REART_API int reart_kin_head(const float* axis, const float* moment, const float* theta, const float* distance,
+                             const int32_t* order, const int32_t* parent, const int32_t* edge, const int32_t* joint_type,
+                             const float* root_6d, const float* root_t, int64_t T, int64_t P, float* R, float* tr, float* fk,
+                             void* stream);
+typedef struct reart_kin_tail_args {
+    const float* fk;
+    const float* gR; const float* gtr;
+    const double* loss_local;
+    const int32_t* order; const int32_t* parent; const int32_t* edge; const int32_t* joint_type;
+    float* axis; float* moment; float* theta; float* distance; float* root_6d; float* root_t;
+    float* grad; float* m; float* v;
+    float* step;
+    float lr, beta1, beta2, eps, weight_decay;
+    float* partials;              /* reart_kin_tail_workspace_bytes(T,P) */
+    float* loss_out;
+    const uint64_t* peer_base; uint32_t* epoch; int32_t rank, world, n_pad;
+    int32_t phase;
+    int64_t T, P;
+} reart_kin_tail_args;
+REART_API int64_t reart_kin_tail_workspace_bytes(int64_t T, int64_t P);
+REART_API int reart_kin_tail(const reart_kin_tail_args* args, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * 6D rotation representation -> matrix (Gram-Schmidt).
  * Replaces screw_se3/geo_utils.py:632-651 (rotation_6d_to_matrix); d6 [B,6] -> R [B,3,3].
  * Backward: gR [B,3,3] -> gd6 [B,6].

@@ -82,7 +82,20 @@ class RelaxTailArgs(ctypes.Structure):
                [(n, _c_i64) for n in ("N", "H", "P", "T")]
 
 
+class KinTailArgs(ctypes.Structure):
+    """reart_kin_tail_args of include/reart_b200.h (field for field)."""
+    _fields_ = [(n, _vp) for n in ("fk", "gR", "gtr", "loss_local", "order", "parent", "edge", "joint_type", "axis", "moment",
+                                   "theta", "distance", "root_6d", "root_t", "grad", "m", "v", "step")] + \
+               [(n, ctypes.c_float) for n in ("lr", "beta1", "beta2", "eps", "weight_decay")] + \
+               [(n, _vp) for n in ("partials", "loss_out", "peer_base", "epoch")] + \
+               [(n, ctypes.c_int32) for n in ("rank", "world", "n_pad", "phase")] + \
+               [(n, _c_i64) for n in ("T", "P")]
+
+
 SIGNATURES.update({
+    "reart_kin_head": (_c_int, [_vp] * 10 + [_c_i64, _c_i64] + [_vp] * 4),
+    "reart_kin_tail_workspace_bytes": (_c_i64, [_c_i64, _c_i64]),
+    "reart_kin_tail": (_c_int, [ctypes.POINTER(KinTailArgs), _vp]),
     "reart_relax_head": (_c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "reart_skinned_chamfer_fwd_bwd_fused": (_c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _c_i64, _vp, _vp, _vp,
                                                      _vp, _vp, _vp, _c_int, _vp, _c_i64, _vp]),

@@ -479,6 +479,46 @@ int reart_relax_tail(const reart_relax_tail_args* x, void* stream_) {
     return launch_relax_tail(a, static_cast<cudaStream_t>(stream_));
 }
 
+int reart_kin_head(const float* axis, const float* moment, const float* theta, const float* distance, const int32_t* order,
+                   const int32_t* parent, const int32_t* edge, const int32_t* joint_type, const float* root_6d,
+                   const float* root_t, int64_t T, int64_t P, float* R, float* tr, float* fk, void* stream_) {
+    REART_ENTRY();
+    if (T < 0 || P < 1 || !fits_int(T * P * 12)) return REART_ERR_INVALID_ARG;
+    if (P > 32) return REART_ERR_UNSUPPORTED;
+    if (T == 0) return REART_OK;
+    if (!order || !parent || !edge || !R || !tr || !fk || (P > 1 && (!axis || !moment || !theta)) || (!root_6d != !root_t))
+        return REART_ERR_INVALID_ARG;
+    FkParams p = {axis, moment, theta, distance, order, parent, edge, joint_type, (int)T, (int)P};
+    return launch_kin_head(p, root_6d, root_t, R, tr, fk, static_cast<cudaStream_t>(stream_));
+}
+
+int64_t reart_kin_tail_workspace_bytes(int64_t T, int64_t P) {
+    if (T < 0 || P < 1) return -1;
+    return align_up(kin_tail_workspace_floats(T, P) * 4) + kAlign;
+}
+
+int reart_kin_tail(const reart_kin_tail_args* x, void* stream_) {
+    REART_ENTRY();
+    if (!x || x->T <= 0 || x->P < 1 || !fits_int(x->T * x->P * 12)) return REART_ERR_INVALID_ARG;
+    if (x->P > 32) return REART_ERR_UNSUPPORTED;
+    if (!x->fk || !x->gR || !x->gtr || !x->loss_local || !x->order || !x->parent || !x->edge || !x->theta ||
+        (x->P > 1 && (!x->axis || !x->moment)) || (!x->root_6d != !x->root_t) || !x->grad || !x->m || !x->v || !x->step ||
+        !x->partials || !x->loss_out || x->phase < 0 || x->phase > 2 || x->world < 1 || x->rank < 0 || x->rank >= x->world)
+        return REART_ERR_INVALID_ARG;
+    KinTail a = {};
+    a.fk = x->fk; a.gR = x->gR; a.gtr = x->gtr; a.loss_local = x->loss_local;
+    a.order = x->order; a.parent = x->parent; a.edge = x->edge; a.joint_type = x->joint_type;
+    a.axis = x->axis; a.moment = x->moment; a.theta = x->theta; a.distance = x->distance;
+    a.root_6d = x->root_6d; a.root_t = x->root_t;
+    a.grad = x->grad; a.m = x->m; a.v = x->v; a.step = x->step;
+    a.lr = x->lr; a.beta1 = x->beta1; a.beta2 = x->beta2; a.eps = x->eps; a.wd = x->weight_decay;
+    a.partials = x->partials; a.loss_out = x->loss_out;
+    a.peer_base = reinterpret_cast<const unsigned long long*>(x->peer_base); a.epoch = x->epoch;
+    a.rank = x->rank; a.world = x->world; a.n_pad = x->n_pad; a.phase = x->phase;
+    a.T = (int)x->T; a.P = (int)x->P;
+    return launch_kin_tail(a, static_cast<cudaStream_t>(stream_));
+}
+
 int reart_rot6d_fwd(const float* d6, int64_t B, float* R, void* stream_) {
     REART_ENTRY();
     if (B < 0) return REART_ERR_INVALID_ARG;

@@ -216,6 +216,30 @@ int64_t relax_tail_workspace_floats(int64_t N, int64_t H, int64_t P);
 int64_t relax_tail_ticket_words(int64_t N);
 int launch_relax_tail(const RelaxTail& a, cudaStream_t stream);
 
+// Fused head / tail of one kinematic-model iteration around the energy (kin.cu).
+int launch_kin_head(const FkParams& p, const float* root_6d, const float* root_t, float* R, float* tr, float* fk,
+                    cudaStream_t stream);
+struct KinTail {
+    const float* fk;              // [T,P,12] per-part poses before the root pose (kin_head)
+    const float* gR; const float* gtr;            // [T,P,9], [T,P,3] d loss / d (R, tr) from the energy
+    const double* loss_local;     // [1] this rank's loss
+    const int32_t* order; const int32_t* parent; const int32_t* edge; const int32_t* joint_type;   // FkParams' tree
+    float* axis; float* moment;   // [E,3] shared parameters -- updated in place
+    float* theta; float* distance;                // [T,E]; distance may be null
+    float* root_6d; float* root_t;                // [T,6], [T,3]; both null without a learned root pose
+    float* grad;                  // [6E | loss | T*E theta | (T*E distance) | (6T root_6d, 3T root_t)]; [0, 6E] is the bucket
+    float* m; float* v;           // Adam moments, same layout as grad (the loss slot is unused)
+    float* step;                  // [1] completed optimisation steps (advanced by the kernel)
+    float lr, beta1, beta2, eps, wd;
+    float* partials;              // [kin_tail_workspace_floats(T,P)]
+    float* loss_out;              // [1] all-rank loss of the step
+    const unsigned long long* peer_base; unsigned* epoch; int rank, world, n_pad;   // one-shot all-reduce (world > 1)
+    int phase;                    // 0 everything; 1 gradients only; 2 Adam from an (externally reduced) bucket
+    int T, P;
+};
+int64_t kin_tail_workspace_floats(int64_t T, int64_t P);
+int launch_kin_tail(const KinTail& a, cudaStream_t stream);
+
 int launch_allreduce_oneshot(const unsigned long long* peer_base, int rank, int world, int64_t n, int64_t n_pad,
                              unsigned* epoch, float* data, cudaStream_t stream);
 

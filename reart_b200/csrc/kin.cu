@@ -1,0 +1,225 @@
+// kin.cu -- one iteration of the kinematic (projection) model, run_robot.py's second model (--model=kinematic,
+// networks/model.py:73-166), around the fused energy of capi.cu:
+//
+//   head = tree forward kinematics (utils/kinematic_utils.py:151-198) + the optional learned root pose
+//          (networks/model.py:151-159): R [T,P,3,3], tr [T,P,3] for the energy, the per-part poses before the root pose
+//          for the backward.  The arithmetic is fk_fwd_kernel's (screw_eval<float>, mat34_mul), so without a root pose
+//          R / tr are bit-identical to reart_fk_fwd.
+//   tail = root-pose backward + FK backward (the dual-number screw of fk_bwd_kernel) + the frame sums of the shared
+//          gradients in frame order + [the one-shot all-reduce of allreduce.cu, inline, when frames are sharded]
+//          + Adam (torch.optim.Adam semantics, one parameter group) on every parameter.
+// The work is T*P small dependent steps: the tail is ONE CTA striding over frames.  No float atomics anywhere, so a step
+// is bit-reproducible (fk_bwd_kernel's atomicAdd over frames is what the autograd path does instead).
+#include "common.cuh"
+#include "kernels.h"
+#include "se3_device.cuh"
+#include "tail_device.cuh"
+
+namespace reart {
+
+// ============================================================================================ head
+constexpr int kKinHeadThreads = 32;                          // one thread per frame, as fk_fwd_kernel
+
+__global__ void __launch_bounds__(kKinHeadThreads) kin_head_kernel(const FkParams p, const float* __restrict__ root_6d,
+                                                                   const float* __restrict__ root_t, float* __restrict__ R,
+                                                                   float* __restrict__ tr, float* __restrict__ fk) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= p.T) return;
+    const bool has_root = root_6d != nullptr;
+    float root[12];                                           // [R_root | t_root], 3x4
+    if (has_root) {
+        float in[6], Rr[9];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) in[k] = root_6d[(int64_t)t * 6 + k];
+        rot6d_eval<float>(in, Rr);
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            root[4 * i] = Rr[3 * i]; root[4 * i + 1] = Rr[3 * i + 1]; root[4 * i + 2] = Rr[3 * i + 2];
+            root[4 * i + 3] = root_t[(int64_t)t * 3 + i];
+        }
+    }
+    for (int oi = 0; oi < p.P; ++oi) {
+        const int c = p.order[oi];
+        const int par = p.parent[c];
+        float M[12];
+        if (par < 0) {
+            for (int k = 0; k < 12; ++k) M[k] = (k % 5 == 0) ? 1.f : 0.f;
+        } else {
+            const int e = p.edge[c];
+            float th, dd; bool tv, dv;
+            fk_joint_inputs(p, t, e, th, dd, tv, dv);
+            float L[3] = {p.axis[3 * e], p.axis[3 * e + 1], p.axis[3 * e + 2]};
+            float Mo[3] = {p.moment[3 * e], p.moment[3 * e + 1], p.moment[3 * e + 2]};
+            float rel[12];
+            screw_eval<float>(L, Mo, th, dd, rel);
+            mat34_mul(fk + ((int64_t)t * p.P + par) * 12, rel, M);
+        }
+        float* F = fk + ((int64_t)t * p.P + c) * 12;
+        for (int k = 0; k < 12; ++k) F[k] = M[k];
+        float out[12];
+        if (has_root) mat34_mul(root, M, out);                // networks/model.py:157-158: root @ fk
+        else for (int k = 0; k < 12; ++k) out[k] = M[k];
+        for (int i = 0; i < 3; ++i) {
+            for (int j = 0; j < 3; ++j) R[((int64_t)t * p.P + c) * 9 + 3 * i + j] = out[4 * i + j];
+            tr[((int64_t)t * p.P + c) * 3 + i] = out[4 * i + 3];
+        }
+    }
+}
+
+int launch_kin_head(const FkParams& p, const float* root_6d, const float* root_t, float* R, float* tr, float* fk,
+                    cudaStream_t stream) {
+    if (p.T <= 0) return kOk;
+    if (p.P <= 0 || p.P > 32) return kErrUnsupported;
+    kin_head_kernel<<<(unsigned)ceil_div(p.T, kKinHeadThreads), kKinHeadThreads, 0, stream>>>(p, root_6d, root_t, R, tr, fk);
+    REART_CHECK_LAUNCH();
+    return kOk;
+}
+
+// ============================================================================================ tail
+constexpr int kKinTailThreads = 256;
+
+int64_t kin_tail_workspace_floats(int64_t T, int64_t P) { return T * 6 * (P - 1) + T * P * 12; }
+
+__global__ void __launch_bounds__(kKinTailThreads) kin_tail_kernel(const KinTail a) {
+    __shared__ int s_ok;
+    const int T = a.T, P = a.P, E = P - 1;
+    const int nshared = 6 * E;                                // [g_axis | g_moment], then the loss
+    const int o_theta = nshared + 1;
+    const int o_dist = o_theta + T * E;
+    const int o_d6 = o_dist + (a.distance ? T * E : 0);
+    const int o_rt = o_d6 + 6 * T;
+    const int n_grad = o_d6 + (a.root_6d ? 9 * T : 0);
+    float* g = a.grad;
+    float* fpart = a.partials;                                // [T][6E] per-frame shared-gradient terms
+    float* work = a.partials + (int64_t)T * nshared;          // [T][P][12] dL/d (pose before the root pose)
+    if (a.phase != 2) {
+        const FkParams fp = {a.axis, a.moment, a.theta, a.distance, a.order, a.parent, a.edge, a.joint_type, T, P};
+        for (int t = threadIdx.x; t < T; t += blockDim.x) {
+            float* gw = work + (int64_t)t * P * 12;
+            const float* gR = a.gR + (int64_t)t * P * 9;
+            const float* gT = a.gtr + (int64_t)t * P * 3;
+            if (a.root_6d) {
+                // out_c = [Rr | tr] [F_c; 0001]:  dL/dF_c = Rr^T G_c,  dL/dRr = sum_c G_c F_c^T (3x4 . 4x3),  dL/dtr = sum_c G_c[:,3]
+                Dual<6> in[6], Rr[9];
+#pragma unroll
+                for (int k = 0; k < 6; ++k) in[k] = Dual<6>::var(a.root_6d[(int64_t)t * 6 + k], k);
+                rot6d_eval<Dual<6>>(in, Rr);
+                float gRr[9], gtr[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+                for (int k = 0; k < 9; ++k) gRr[k] = 0.f;
+                for (int c = 0; c < P; ++c) {
+                    const float* F = a.fk + ((int64_t)t * P + c) * 12;
+                    float G[12];
+#pragma unroll
+                    for (int i = 0; i < 3; ++i) {
+                        G[4 * i] = gR[c * 9 + 3 * i]; G[4 * i + 1] = gR[c * 9 + 3 * i + 1]; G[4 * i + 2] = gR[c * 9 + 3 * i + 2];
+                        G[4 * i + 3] = gT[c * 3 + i];
+                    }
+#pragma unroll
+                    for (int i = 0; i < 3; ++i) {
+#pragma unroll
+                        for (int k = 0; k < 3; ++k)
+                            gRr[3 * i + k] += G[4 * i] * F[4 * k] + G[4 * i + 1] * F[4 * k + 1] + G[4 * i + 2] * F[4 * k + 2] +
+                                              G[4 * i + 3] * F[4 * k + 3];
+                        gtr[i] += G[4 * i + 3];
+                    }
+#pragma unroll
+                    for (int k = 0; k < 3; ++k)
+#pragma unroll
+                        for (int j = 0; j < 4; ++j)
+                            gw[c * 12 + 4 * k + j] = Rr[k].v * G[j] + Rr[3 + k].v * G[4 + j] + Rr[6 + k].v * G[8 + j];
+                }
+                float g6[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+                for (int o = 0; o < 9; ++o)
+#pragma unroll
+                    for (int k = 0; k < 6; ++k) g6[k] += gRr[o] * Rr[o].d[k];
+#pragma unroll
+                for (int k = 0; k < 6; ++k) g[o_d6 + t * 6 + k] = g6[k];
+#pragma unroll
+                for (int i = 0; i < 3; ++i) g[o_rt + t * 3 + i] = gtr[i];
+            } else {
+                for (int c = 0; c < P; ++c)
+#pragma unroll
+                    for (int i = 0; i < 3; ++i) {
+                        gw[c * 12 + 4 * i] = gR[c * 9 + 3 * i]; gw[c * 12 + 4 * i + 1] = gR[c * 9 + 3 * i + 1];
+                        gw[c * 12 + 4 * i + 2] = gR[c * 9 + 3 * i + 2]; gw[c * 12 + 4 * i + 3] = gT[c * 3 + i];
+                    }
+            }
+            // the tree walk of fk_bwd_kernel, leaves first; the shared terms go to this frame's row instead of atomics
+            for (int oi = P - 1; oi >= 0; --oi) {
+                const int c = a.order[oi];
+                const int par = a.parent[c];
+                if (par < 0) continue;
+                const int e = a.edge[c];
+                float th, dd; bool tv, dv;
+                fk_joint_inputs(fp, t, e, th, dd, tv, dv);
+                Dual<8> L[3], Mo[3], rel[12];
+                for (int k = 0; k < 3; ++k) { L[k] = Dual<8>::var(a.axis[3 * e + k], k); Mo[k] = Dual<8>::var(a.moment[3 * e + k], 3 + k); }
+                screw_eval<Dual<8>>(L, Mo, Dual<8>::var(th, 6), Dual<8>::var(dd, 7), rel);
+                const float* A = a.fk + ((int64_t)t * P + par) * 12;   // parent pose
+                const float* G = gw + c * 12;                         // dL/d fk[c] (complete: children were folded already)
+                float* Gp = gw + par * 12;
+                float g8[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+                for (int i = 0; i < 3; ++i) {
+                    for (int j = 0; j < 4; ++j) {
+                        const float dT = A[i] * G[j] + A[4 + i] * G[4 + j] + A[8 + i] * G[8 + j];
+                        for (int k = 0; k < 8; ++k) g8[k] += dT * rel[4 * i + j].d[k];
+                    }
+                }
+                for (int i = 0; i < 3; ++i) {
+                    for (int j = 0; j < 4; ++j) {
+                        float s = 0.f;
+                        if (j < 3) s = G[4 * i] * rel[4 * j].v + G[4 * i + 1] * rel[4 * j + 1].v + G[4 * i + 2] * rel[4 * j + 2].v +
+                                       G[4 * i + 3] * rel[4 * j + 3].v;
+                        else s = G[4 * i + 3];
+                        Gp[4 * i + j] += s;
+                    }
+                }
+                float* row = fpart + (int64_t)t * nshared;
+                for (int k = 0; k < 3; ++k) { row[3 * e + k] = g8[k]; row[3 * E + 3 * e + k] = g8[3 + k]; }
+                g[o_theta + t * E + e] = tv ? g8[6] : 0.f;
+                if (a.distance) g[o_dist + t * E + e] = dv ? g8[7] : 0.f;
+            }
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < nshared; i += blockDim.x) {   // sum over frames in frame order
+            float s = 0.f;
+            for (int t = 0; t < T; ++t) s += fpart[(int64_t)t * nshared + i];
+            g[i] = s;
+        }
+        if (threadIdx.x == 0) g[nshared] = (float)*a.loss_local;
+        __syncthreads();
+    }
+    if (a.phase == 1) return;                                 // the caller all-reduces g[0 .. 6E] (NCCL), then phase 2
+    if (a.phase == 0 && a.world > 1)
+        cta_allreduce_oneshot(a.peer_base, a.rank, a.world, nshared + 1, a.n_pad, a.epoch, g, &s_ok);
+    const float step = *a.step + 1.0f;                        // 1-based index of this optimisation step
+    const AdamCoef c = adam_coef(a.lr, a.beta1, a.beta2, a.eps, a.wd, step);
+    for (int i = threadIdx.x; i < n_grad; i += blockDim.x) {
+        if (i == nshared) continue;                           // the loss slot
+        float* prm = i < 3 * E ? a.axis + i
+                   : i < nshared ? a.moment + (i - 3 * E)
+                   : i < o_dist ? a.theta + (i - o_theta)
+                   : i < o_d6 ? a.distance + (i - o_dist)
+                   : i < o_rt ? a.root_6d + (i - o_d6)
+                   : a.root_t + (i - o_rt);
+        adam_update(prm, a.m + i, a.v + i, g[i], c);
+    }
+    __syncthreads();                                          // every thread has read *a.step
+    if (threadIdx.x == 0) {
+        *a.loss_out = g[nshared];
+        *a.step = step;
+    }
+}
+
+int launch_kin_tail(const KinTail& a, cudaStream_t stream) {
+    if (a.T <= 0 || a.P <= 0) return kErrInvalidArg;
+    if (a.P > 32) return kErrUnsupported;
+    if (a.world > 1 && a.phase == 0 && (a.world > kKinTailThreads || !a.peer_base || !a.epoch)) return kErrInvalidArg;
+    kin_tail_kernel<<<1, kKinTailThreads, 0, stream>>>(a);
+    REART_CHECK_LAUNCH();
+    return kOk;
+}
+
+}  // namespace reart

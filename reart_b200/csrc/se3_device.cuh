@@ -1,6 +1,8 @@
-// se3_device.cuh -- forward-mode dual numbers and the 6D -> R evaluation shared by se3.cu and relax.cu.
+// se3_device.cuh -- forward-mode dual numbers, 6D -> R, screw -> 3x4 and the forward-kinematics pieces shared by se3.cu,
+// relax.cu and kin.cu.
 #pragma once
 #include "common.cuh"
+#include "kernels.h"
 
 namespace reart {
 
@@ -128,5 +130,71 @@ __device__ __forceinline__ void rot6d_eval(const S* d6, S* R) {
     R[8] = b1[0] * b2[1] - b1[1] * b2[0];
 }
 
+
+// ----------------------------------------------------------------------------- screw -> 4x4
+// M (row-major 3x4: [R | t]) from (l, m, theta, d): screw_se3/screw_utils.py:6-30 over geo_utils.py:90-222, with the
+// reference's quirks (se3.cu header)
+template <typename S>
+__device__ __forceinline__ void screw_eval(const S* l, const S* m, const S& theta, const S& d, S* M) {
+    const float eps = 1e-6f;
+    const float pi_f = 3.14159265358979323846f;
+    const float th = val(theta);
+    const bool no_rot = (fabsf(th) < eps) || (fabsf(th - pi_f) < eps);
+    S w[3], v[3];
+    if (!no_rot) {
+        S q[3] = {l[1] * m[2] - l[2] * m[1], l[2] * m[0] - l[0] * m[2], l[0] * m[1] - l[1] * m[0]};
+        S h = d / theta;
+        S c[3] = {q[1] * l[2] - q[2] * l[1], q[2] * l[0] - q[0] * l[2], q[0] * l[1] - q[1] * l[0]};
+        for (int k = 0; k < 3; ++k) { w[k] = l[k] * theta; v[k] = (c[k] + h * l[k]) * theta; }
+    } else {
+        for (int k = 0; k < 3; ++k) { w[k] = lit<S>(0.f) * theta; v[k] = l[k] * theta; }
+    }
+    S nrm = w[0] * w[0] + w[1] * w[1] + w[2] * w[2];
+    S ang = dsqrt(dclamp_min(nrm, 1e-4f));
+    S one = lit<S>(1.0f);
+    S inv = one / ang;
+    S sn = dsin(ang), cs = dcos(ang);
+    S fac1 = inv * sn;
+    S fac2 = inv * inv * (one - cs);
+    S facV1 = (one - cs) / (ang * ang);
+    S facV2 = (ang - sn) / (ang * ang * ang);
+    S zero = lit<S>(0.f);
+    S K[9] = {zero, -w[2], w[1], w[2], zero, -w[0], -w[1], w[0], zero};
+    S K2[9];
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) K2[3 * i + j] = K[3 * i] * K[j] + K[3 * i + 1] * K[3 + j] + K[3 * i + 2] * K[6 + j];
+    for (int i = 0; i < 3; ++i) {
+        S Vr[3];
+        for (int j = 0; j < 3; ++j) {
+            S I = lit<S>(i == j ? 1.f : 0.f);
+            M[4 * i + j] = fac1 * K[3 * i + j] + fac2 * K2[3 * i + j] + I;
+            Vr[j] = I + K[3 * i + j] * facV1 + K2[3 * i + j] * facV2;
+        }
+        M[4 * i + 3] = Vr[0] * v[0] + Vr[1] * v[1] + Vr[2] * v[2];
+    }
+}
+
+// ----------------------------------------------------------------------------- forward kinematics (tree walk pieces)
+__device__ __forceinline__ void mat34_mul(const float* A, const float* Bm, float* C) {   // [A;0001]*[B;0001], 3x4 blocks
+    for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 4; ++j) {
+            float s = A[4 * i] * Bm[j] + A[4 * i + 1] * Bm[4 + j] + A[4 * i + 2] * Bm[8 + j];
+            if (j == 3) s += A[4 * i + 3];
+            C[4 * i + j] = s;
+        }
+    }
+}
+
+__device__ __forceinline__ void fk_joint_inputs(const FkParams& p, int t, int e, float& th, float& dd, bool& th_var,
+                                                bool& d_var) {
+    const int E = p.P - 1;
+    const int jt = p.joint_type ? p.joint_type[e] : 0;
+    th = p.theta[(int64_t)t * E + e];
+    th_var = true;
+    d_var = p.distance != nullptr;
+    dd = d_var ? p.distance[(int64_t)t * E + e] : 1e-6f;
+    if (jt == 1) { dd = 1e-6f; d_var = false; }              // revolute  (kinematic_utils.py:181-184)
+    if (jt == 2) { th = 1e-6f; th_var = false; }             // prismatic (kinematic_utils.py:176-179)
+}
 
 }  // namespace reart

@@ -6,7 +6,8 @@ seg MLP -> straight-through gumbel weights -> 6D -> R -> fused [skin -> bidirect
 captured once in a CUDA graph (NCCL all-reduce included) and replayed, so neither Python nor the ~4 host syncs
 per iteration of the reference loop (SURVEY Q20) sit on the critical path.
 
-``KinematicEngine.step`` is the same for ``--model=kinematic`` (fused tree FK instead of the 6D proposals).
+``KinematicEngine.step`` is the same for ``--model=kinematic`` (fused tree FK instead of the 6D proposals); its native
+iteration (``native=True``) is kin_head -> fused energy -> kin_tail on library kernels.
 Frames are sharded across ranks by ``DistContext``; per-frame parameters stay local to their rank.
 """
 from __future__ import annotations
@@ -171,6 +172,79 @@ class _EngineBase:
     def _after_replay(self, variant):
         pass
 
+    # ------------------------------------------------------------------------------------------ search of the energy
+    def _setup_search(self, search: str, can_order: bool, why: str):
+        """search="brute" | "culled" | "auto" of the native iterations.  "culled" runs the exact culled search on k-d ordered
+        copies of the clouds while everything else stays in the caller's order: bit-identical to "brute".  "auto" picks it
+        from ``SEARCH_CULLED_MIN_POINTS`` points per cloud on, where the coarse bounds of cull.cu make it faster.
+        ``can_order``: this engine's configuration can run it (else "culled" raises ValueError(why))."""
+        if search not in ("auto", "brute", "culled"):
+            raise ValueError("search must be 'auto', 'brute' or 'culled'")
+        if search == "culled" and not can_order:
+            raise ValueError(why)
+        self.search_culled = can_order and (search == "culled" or (
+            search == "auto" and min(self.cano.shape[0], self.frames.shape[1]) >= SEARCH_CULLED_MIN_POINTS))
+        self.search_order_rows = self.search_order_tgt = None
+        if self.search_culled:
+            # the culled search's own order, fixed here (256-row blocks = one warp of the search, 32-target chunks); the
+            # engine's clouds, outputs and every sum stay in the caller's order.  Any order is exact, a stale one (after
+            # step(ingest=...)) only culls less.
+            dev = self.cano.device
+            self.search_order_rows = ops.search_order(self.cano[None], 256)[0].int()
+            self.search_order_tgt = ops.search_order(self.frames, 32).int()
+            self.search_inv_rows = torch.empty_like(self.search_order_rows)
+            self.search_inv_rows[self.search_order_rows.long()] = torch.arange(
+                self.cano.shape[0], dtype=torch.int32, device=dev)
+            self.search_inv_tgt = torch.empty_like(self.search_order_tgt)
+            self.search_inv_tgt.scatter_(1, self.search_order_tgt.long(), torch.arange(
+                self.frames.shape[1], dtype=torch.int32, device=dev)[None].expand_as(self.search_order_tgt).contiguous())
+            self._search_gather = self.search_order_tgt.long()[:, :, None].expand(-1, -1, 3)
+            self.frames_search = torch.gather(self.frames, 1, self._search_gather).contiguous()
+            self.frames_search_packed = ops.pack_cloud(self.frames_search)
+
+    def _search_buffers(self, b, T, N, M):
+        """The culled search's state carried from step to step, in the native buffers ``b``."""
+        dev = self.cano.device
+        b["nn_rows"] = torch.full((T, N), -1, dtype=torch.int32, device=dev)      # arg-mins of the last step (-1: none yet)
+        b["nn_cols"] = torch.full((T, M), -1, dtype=torch.int32, device=dev)
+        # evaluated / offered (warp, chunk) pairs; ordered search: + points resolved by the exact tie path
+        b["cull_stats"] = torch.zeros(3 if self.search_culled else 2, dtype=torch.int64, device=dev)
+
+    def _search_energy(self, L, b, W, R, tr, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
+        """The fused energy on skinning weights W and poses (R, tr): brute-force search, or the exact culled one in the
+        search order seeded by the previous step's arg-mins (bit-identical results).  Writes b["skinned"], b["loss64"]."""
+        from ._lib import check, ptr, stream_ptr
+        if self.search_culled:
+            check(L.reart_skinned_chamfer_fwd_bwd_ordered(
+                ptr(self.cano), ptr(W), ptr(R), ptr(tr), ptr(self.frames), ptr(self.frames_search),
+                ptr(self.frames_search_packed), T, N, M, P, ptr(self.search_order_rows), ptr(self.search_inv_rows),
+                ptr(self.search_order_tgt), ptr(self.search_inv_tgt), ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR),
+                ptr(gtr), ptr(g_skinned), compute_grad, None, None, None, None, ptr(b["nn_rows"]), ptr(b["nn_cols"]),
+                ptr(b["cull_stats"]), ptr(b["ws"]), b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_ordered")
+        else:
+            check(L.reart_skinned_chamfer_fwd_bwd(
+                ptr(self.cano), ptr(W), ptr(R), ptr(tr), ptr(self.frames), ptr(self.frames_packed), T, N, M, P,
+                ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr), ptr(g_skinned), compute_grad, ptr(b["ws"]),
+                b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd")
+
+    def culling_stats(self):
+        """(evaluated, offered) (warp, 32-target chunk) pairs since the last call; resets the counters.  Host sync."""
+        b = getattr(self, "_nat", None)
+        if not getattr(self, "native", False) or b is None or "cull_stats" not in b:
+            return None
+        ev, off = (int(x) for x in b["cull_stats"][:2].tolist())
+        b["cull_stats"][:2].zero_()
+        return ev, off
+
+    def flagged_ties(self):
+        """Points the culled search saw reach their minimum in two of its chunks, resolved by the exact tie path, since
+        the last call (resets the counter; None unless search is culled).  Host sync."""
+        if not self.search_culled:
+            return None
+        n = int(self._nat["cull_stats"][2])
+        self._nat["cull_stats"][2].zero_()
+        return n
+
 
 # search="auto" runs the culled search from this many points per cloud on (both clouds): the coarse bounds of cull.cu
 # start culling there
@@ -221,14 +295,9 @@ class RelaxationEngine(_EngineBase):
         if self.cull and (flow_ref is not None or native is False):
             raise ValueError("exact tile culling runs on the native fused iteration (recon / assignment losses)")
         self.perm_cano = self.perm_frames = None
-        if search not in ("auto", "brute", "culled"):
-            raise ValueError("search must be 'auto', 'brute' or 'culled'")
         native_path = (flow_ref is None) if native is None else bool(native)
-        can_order = native_path and not self.cull and not self.fuse_producer
-        if search == "culled" and not can_order:
-            raise ValueError("search='culled' runs on the native fused iteration, without cull=True or fuse_producer=True")
-        self.search_culled = can_order and (search == "culled" or (
-            search == "auto" and min(self.cano.shape[0], self.frames.shape[1]) >= SEARCH_CULLED_MIN_POINTS))
+        self._setup_search(search, native_path and not self.cull and not self.fuse_producer,
+                           "search='culled' runs on the native fused iteration, without cull=True or fuse_producer=True")
         cano_orig, frames_orig = self.cano, self.frames
         if self.cull:
             # k-d order refined well below the chunk sizes of the search (256 rows / 32 targets): the chunks stay the same
@@ -238,22 +307,6 @@ class RelaxationEngine(_EngineBase):
             self.cano = self.cano[self.perm_cano].contiguous()
             self.frames = torch.gather(self.frames, 1, self.perm_frames[:, :, None].expand(-1, -1, 3)).contiguous()
         self.frames_packed = ops.pack_cloud(self.frames)          # constant over the optimisation: packed once
-        self.search_order_rows = self.search_order_tgt = None
-        if self.search_culled:
-            # the culled search's own order, fixed here (256-row blocks = one warp of the search, 32-target chunks); the
-            # engine's clouds, outputs and every sum stay in the caller's order.  Any order is exact, a stale one (after
-            # step(ingest=...)) only culls less.
-            self.search_order_rows = ops.search_order(self.cano[None], 256)[0].int()
-            self.search_order_tgt = ops.search_order(self.frames, 32).int()
-            self.search_inv_rows = torch.empty_like(self.search_order_rows)
-            self.search_inv_rows[self.search_order_rows.long()] = torch.arange(
-                self.cano.shape[0], dtype=torch.int32, device=dev)
-            self.search_inv_tgt = torch.empty_like(self.search_order_tgt)
-            self.search_inv_tgt.scatter_(1, self.search_order_tgt.long(), torch.arange(
-                self.frames.shape[1], dtype=torch.int32, device=dev)[None].expand_as(self.search_order_tgt).contiguous())
-            self._search_gather = self.search_order_tgt.long()[:, :, None].expand(-1, -1, 3)
-            self.frames_search = torch.gather(self.frames, 1, self._search_gather).contiguous()
-            self.frames_search_packed = ops.pack_cloud(self.frames_search)
         torch.manual_seed(seed)                                    # identical init + gumbel draws on every rank
         torch.cuda.manual_seed_all(seed)
         self.model = BaseModel(num_parts=num_parts, pose_len=hi - lo).to(dev)
@@ -329,11 +382,8 @@ class RelaxationEngine(_EngineBase):
         b["bucket"] = torch.zeros(nseg + 1, **f32)
         b["loss_out"] = torch.zeros(1, **f32)
         b["dims"] = (T, N, M, P, H)
-        if self.cull or self.search_culled:                      # arg-mins carried from step to step (-1: none yet)
-            b["nn_rows"] = torch.full((T, N), -1, dtype=torch.int32, device=dev)
-            b["nn_cols"] = torch.full((T, M), -1, dtype=torch.int32, device=dev)
-            # evaluated / offered (warp, chunk) pairs; ordered search: + points resolved by the exact tie path
-            b["cull_stats"] = torch.zeros(3 if self.search_culled else 2, dtype=torch.int64, device=dev)
+        if self.cull or self.search_culled:
+            self._search_buffers(b, T, N, M)
         red = self.sink.reducer if self.sink is not None else None
         self.model.seg_head.grad_sink = None                     # the autograd sink is not used on this path
         oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
@@ -396,51 +446,24 @@ class RelaxationEngine(_EngineBase):
         return getattr(self, "_cur_variant", None) or self._phase()
 
     def _energy_call(self, L, b, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
-        """The fused energy evaluation of this step: brute-force search, or the exact culled one seeded by the previous
-        step's arg-mins (bit-identical results)."""
+        """The fused energy evaluation of this step: brute-force or culled search (``_search_energy``), the culled search on
+        the engine's own k-d order (cull=True), or the skinning fused into the search (fuse_producer=True)."""
         from ._lib import check, ptr, stream_ptr
         m = self.model
-        if self.search_culled:
-            check(L.reart_skinned_chamfer_fwd_bwd_ordered(
-                ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_search),
-                ptr(self.frames_search_packed), T, N, M, P, ptr(self.search_order_rows), ptr(self.search_inv_rows),
-                ptr(self.search_order_tgt), ptr(self.search_inv_tgt), ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR),
-                ptr(gtr), ptr(g_skinned), compute_grad, None, None, None, None, ptr(b["nn_rows"]), ptr(b["nn_cols"]),
-                ptr(b["cull_stats"]), ptr(b["ws"]), b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_ordered")
-        elif self.cull:
+        if self.cull:
             check(L.reart_skinned_chamfer_fwd_bwd_culled(
                 ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_packed), T, N, M, P,
                 ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr), ptr(g_skinned), compute_grad, None, None, None,
                 None, ptr(b["nn_rows"]), ptr(b["nn_cols"]), ptr(b["cull_stats"]), ptr(b["ws"]), b["ws_bytes"], stream_ptr()),
                 "reart_skinned_chamfer_fwd_bwd_culled")
         elif not self.fuse_producer:
-            check(L.reart_skinned_chamfer_fwd_bwd(
-                ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_packed), T, N, M, P,
-                ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr), ptr(g_skinned), compute_grad, ptr(b["ws"]),
-                b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd")
+            self._search_energy(L, b, b["W"], b["R"], m.proposal_t, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad)
         else:
             # skinning fused into the producer side of the search (the weights are one-hot: the head wrote them in compact form)
             check(L.reart_skinned_chamfer_fwd_bwd_fused(
                 ptr(self.cano), ptr(b["hot"]), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(self.frames), ptr(self.frames_packed),
                 T, N, M, P, ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr), ptr(g_skinned), compute_grad, ptr(b["ws"]),
                 b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_fused")
-
-    def culling_stats(self):
-        """(evaluated, offered) (warp, 32-target chunk) pairs since the last call; resets the counters.  Host sync."""
-        if not (self.native and (self.cull or self.search_culled)):
-            return None
-        ev, off = (int(x) for x in self._nat["cull_stats"][:2].tolist())
-        self._nat["cull_stats"][:2].zero_()
-        return ev, off
-
-    def flagged_ties(self):
-        """Points the culled search saw reach their minimum in two of its chunks, resolved by the exact tie path, since
-        the last call (resets the counter; None unless search is culled).  Host sync."""
-        if not self.search_culled:
-            return None
-        n = int(self._nat["cull_stats"][2])
-        self._nat["cull_stats"][2].zero_()
-        return n
 
     def _run_iteration_native(self):
         """head -> [memset, skin (x-sorted copy), search, energy columns, energy rows, skin backward, reduce] -> tail."""
@@ -548,7 +571,11 @@ class KinematicEngine(_EngineBase):
 
     def __init__(self, model_kwargs: dict, seg_part: torch.Tensor, cano: torch.Tensor, frames: torch.Tensor,
                  ctx: Optional[DistContext] = None, lr: float = 1e-2, weight_decay: float = 0.0,
-                 use_graph: bool = True):
+                 use_graph: bool = True, native: bool = False, search: str = "auto", betas=(0.9, 0.999), eps: float = 1e-8):
+        """native=True runs the iteration on library kernels -- kin_head -> fused energy -> kin_tail (FK backward, frame
+        sums in a fixed order, [all-reduce], the library's Adam) -- with no autograd: the same optimisation as the default
+        autograd composition, bit-reproducible.  search: "brute" | "culled" | "auto" as for ``RelaxationEngine`` (native
+        iteration only; "culled" is bit-identical to "brute")."""
         super().__init__(ctx, use_graph)
         from .knn_module import KNN
         dev = cano.device
@@ -559,6 +586,8 @@ class KinematicEngine(_EngineBase):
         self.cano = cano.float().contiguous()
         self.frames = frames[lo:hi].float().contiguous()
         self.frames_packed = ops.pack_cloud(self.frames)
+        self.native = bool(native)
+        self._setup_search(search, self.native, "search='culled' runs on the native fused iteration (native=True)")
         kw = dict(model_kwargs)
         for k in ("theta_list", "distance_list", "root_trans"):
             if k in kw:
@@ -566,12 +595,17 @@ class KinematicEngine(_EngineBase):
         self.model = KinematicModel(pose_len=hi - lo, seg_part=seg_part, cano_pc=self.cano,
                                     knn=KNN(k=1, transpose_mode=True), **kw).to(dev)
         self.tau = torch.ones((), device=dev)
-        params = [p for p in self.model.parameters() if p.requires_grad]
-        self.optimizer = torch.optim.Adam(params, lr=lr, weight_decay=weight_decay, capturable=use_graph, fused=True)
-        self.bucket = GradBucket([self.model.axis_list, self.model.moment_list], extra_scalars=1)
         with torch.no_grad():                                       # constant label transfer (SURVEY Q27)
             self.weight = F.one_hot(self.model._labels(self.model.cano_pc), num_classes=self.model.num_parts).float()
         self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
+        if self.native:
+            self.optimizer = self.bucket = None
+            self._init_native(lr, weight_decay, betas, eps)
+        else:
+            params = [p for p in self.model.parameters() if p.requires_grad]
+            self.optimizer = torch.optim.Adam(params, lr=lr, weight_decay=weight_decay, betas=betas, eps=eps,
+                                              capturable=use_graph, fused=True)
+            self.bucket = GradBucket([self.model.axis_list, self.model.moment_list], extra_scalars=1)
 
     def _iteration(self):
         trans = self.model.transforms()
@@ -580,6 +614,112 @@ class KinematicEngine(_EngineBase):
                                                  unit_grad=True)
         self.skinned = skinned.detach()
         return loss
+
+    # ------------------------------------------------------------------------------------------ native fused iteration
+    def _init_native(self, lr, weight_decay, betas, eps):
+        from . import _lib
+        from ._lib import ptr
+        L = _lib.lib()
+        m = self.model
+        dev = self.cano.device
+        T, P = m.theta_list.shape[0], m.num_parts
+        E = P - 1
+        N, M = self.cano.shape[0], self.frames.shape[1]
+        tree = m.tree(dev)
+        if P > 32:
+            raise ValueError("the native kinematic iteration supports up to 32 parts")
+        params = self._opt_params()
+        for q in params:                                            # raw pointers below: float32, contiguous, updated in place
+            if q.dtype != torch.float32 or not q.is_contiguous():
+                q.data = q.data.float().contiguous()
+        distance = getattr(m, "distance_list", None)
+        has_root = hasattr(m, "root_6d") and hasattr(m, "root_t")
+        f32 = dict(dtype=torch.float32, device=dev)
+        b = self._nat = {}
+        b["dims"] = (T, N, M, P)
+        b["fk"] = torch.empty(T, P, 12, **f32)
+        b["R"], b["tr"] = torch.empty(T, P, 3, 3, **f32), torch.empty(T, P, 3, **f32)
+        b["gpose"] = torch.empty(T * P * 12, **f32)
+        b["gR"], b["gtr"] = b["gpose"][:T * P * 9], b["gpose"][T * P * 9:]
+        b["gW"] = torch.empty(N, P, **f32)                          # the weights are constant: scratch
+        b["skinned"] = torch.empty(T, N, 3, **f32)
+        b["loss64"] = torch.zeros(1, dtype=torch.float64, device=dev)
+        b["ws_bytes"] = int(L.reart_energy_workspace_bytes(T, N, M))
+        b["ws"] = _lib.workspace(b["ws_bytes"], dev)
+        b["tail_ws"] = _lib.workspace(int(L.reart_kin_tail_workspace_bytes(T, P)), dev)
+        # [g_axis | g_moment | loss | g_theta | (g_distance) | (g_root_6d, g_root_t)]; the first 6E + 1 are the all-reduce bucket
+        n_grad = 6 * E + 1 + T * E + (T * E if distance is not None else 0) + (9 * T if has_root else 0)
+        b["grad"], b["m"], b["v"] = torch.zeros(n_grad, **f32), torch.zeros(n_grad, **f32), torch.zeros(n_grad, **f32)
+        b["bucket"] = b["grad"][:6 * E + 1]
+        b["step"] = torch.zeros(1, **f32)
+        b["loss_out"] = torch.zeros(1, **f32)
+        if self.search_culled:
+            self._search_buffers(b, T, N, M)
+        self.weight = self.weight.contiguous()
+        red = make_small_all_reduce(self.ctx, 6 * E + 1, dev)
+        oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
+        b["nccl"] = red is not None and oneshot is None
+        b["head"] = (ptr(m.axis_list), ptr(m.moment_list), ptr(m.theta_list), ptr(distance), ptr(tree.order), ptr(tree.parent),
+                     ptr(tree.edge), ptr(tree.joint_type), ptr(m.root_6d) if has_root else None,
+                     ptr(m.root_t) if has_root else None, T, P, ptr(b["R"]), ptr(b["tr"]), ptr(b["fk"]))
+        a = _lib.KinTailArgs()
+        a.fk, a.gR, a.gtr, a.loss_local = ptr(b["fk"]), ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"])
+        a.order, a.parent, a.edge, a.joint_type = ptr(tree.order), ptr(tree.parent), ptr(tree.edge), ptr(tree.joint_type)
+        a.axis, a.moment, a.theta, a.distance = ptr(m.axis_list), ptr(m.moment_list), ptr(m.theta_list), ptr(distance)
+        a.root_6d, a.root_t = (ptr(m.root_6d), ptr(m.root_t)) if has_root else (None, None)
+        a.grad, a.m, a.v, a.step = ptr(b["grad"]), ptr(b["m"]), ptr(b["v"]), ptr(b["step"])
+        a.lr, a.beta1, a.beta2, a.eps, a.weight_decay = lr, betas[0], betas[1], eps, weight_decay
+        a.partials, a.loss_out = ptr(b["tail_ws"]), ptr(b["loss_out"])
+        a.rank, a.world = (self.ctx.rank, self.ctx.world_size) if oneshot is not None else (0, 1)
+        if oneshot is not None:
+            assert oneshot.n == 6 * E + 1
+            a.peer_base, a.epoch, a.n_pad = ptr(oneshot.peer_base), ptr(oneshot.epoch), oneshot.n_pad
+        a.phase = 0
+        a.T, a.P = T, P
+        b["args"] = a
+        b["keep"] = (tree, oneshot)
+
+    def _opt_params(self):
+        if not self.native:
+            return super()._opt_params()
+        m = self.model
+        names = ["axis_list", "moment_list", "theta_list", "distance_list", "root_6d", "root_t"]
+        return [getattr(m, n) for n in names if hasattr(m, n)]
+
+    def _opt_state_tensors(self):
+        if self.native:
+            return [self._nat[k] for k in ("m", "v", "step")]
+        return super()._opt_state_tensors()
+
+    def _aux_state_tensors(self):
+        if self.native and self.search_culled:
+            return [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
+        return []
+
+    def _run_iteration_native(self):
+        """kin_head -> [memset, skin (x-sorted copy), (cull bounds,) search, energy columns, energy rows, skin backward,
+        reduce] -> kin_tail."""
+        import ctypes
+        from . import _lib
+        from ._lib import check, stream_ptr
+        L = _lib.lib()
+        b = self._nat
+        T, N, M, P = b["dims"]
+        with torch.cuda.device(self.cano.device):
+            check(L.reart_kin_head(*b["head"], stream_ptr()), "reart_kin_head")
+            self._search_energy(L, b, self.weight, b["R"], b["tr"], T, N, M, P, b["gW"], b["gR"], b["gtr"], None, 1)
+            a = b["args"]
+            if not b["nccl"]:
+                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
+            else:                                                 # no peer memory: gradients -> bucket, NCCL, Adam
+                a.phase = 1
+                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
+                self.ctx.all_reduce_sum_(b["bucket"])
+                a.phase = 2
+                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
+                a.phase = 0
+        self.skinned = b["skinned"]
+        return b["loss_out"][0]
 
 
 def tau_schedule(i: int, n_iter: int, start_tau: float, end_tau: float) -> float:
