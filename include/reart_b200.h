@@ -280,6 +280,24 @@ typedef struct reart_kin_tail_args {
 REART_API int64_t reart_kin_tail_workspace_bytes(int64_t T, int64_t P);
 REART_API int reart_kin_tail(const reart_kin_tail_args* args, void* stream);
 
+/* The assignment loss of the kinematic model (run_robot.py:181-187) straight into the pose gradients, between the energy
+ * (or reart_skin_fwd) and reart_kin_tail.  Premise: the skinning weights are ONE-HOT rows (the kinematic model's label
+ * transfer), so the gradient w.r.t. (R, tr) of part p in frame t is a sum over the samples of part p alone:
+ *   d = skinned[t, src_idx[i]] - tgt[t, col4row[t,i]],  x = cano[src_idx[i]]
+ *   loss += lambda sum |d|^2,  gR[t,p] += 2 lambda sum d x^T,  gtr[t,p] += 2 lambda sum d.
+ * skinned [T,N,3] (read, not recomputed), cano [N,3], src_idx [n] int64, tgt [T,n,3] (the sampled targets), col4row [T,n]
+ * (reart_lap); sample_order [n]: the sample indices stably sorted by the part of cano[src_idx[i]], part_offsets [P+1]: part
+ * p owns sample_order[part_offsets[p] .. part_offsets[p+1]).  gR [T,P,3,3], gtr [T,P,3], loss [1] double: accumulate != 0
+ * adds to them (after the energy wrote its Chamfer gradients), else overwrites them (a part without samples gets zeros;
+ * with accumulate its gradient is left untouched).  No float atomics: bit-reproducible.  workspace:
+ * reart_kin_assign_workspace_bytes(T,P), zero before the FIRST call (the kernel re-arms it).  P <= 32, n <= 4096 as reart_lap.
+ * ------------------------------------------------------------------------------------------- */
+REART_API int64_t reart_kin_assign_workspace_bytes(int64_t T, int64_t P);
+REART_API int reart_kin_assign(const float* skinned, const float* cano, const int64_t* src_idx, const float* tgt,
+                               const int32_t* col4row, const int32_t* sample_order, const int32_t* part_offsets,
+                               float lambda, int64_t T, int64_t N, int64_t n, int64_t P, float* gR, float* gtr,
+                               double* loss, int accumulate, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * 6D rotation representation -> matrix (Gram-Schmidt).
  * Replaces screw_se3/geo_utils.py:632-651 (rotation_6d_to_matrix); d6 [B,6] -> R [B,3,3].

@@ -519,6 +519,36 @@ int reart_kin_tail(const reart_kin_tail_args* x, void* stream_) {
     return launch_kin_tail(a, static_cast<cudaStream_t>(stream_));
 }
 
+int64_t reart_kin_assign_workspace_bytes(int64_t T, int64_t P) {
+    if (T < 0 || P < 1 || P > 32) return -1;
+    return align_up(kin_assign_blocks(T, P) * 8) + align_up(4) + kAlign;
+}
+
+int reart_kin_assign(const float* skinned, const float* cano, const int64_t* src_idx, const float* tgt,
+                     const int32_t* col4row, const int32_t* sample_order, const int32_t* part_offsets, float lambda, int64_t T,
+                     int64_t N, int64_t n, int64_t P, float* gR, float* gtr, double* loss, int accumulate, void* workspace,
+                     int64_t workspace_bytes, void* stream_) {
+    REART_ENTRY();
+    if (T < 0 || N < 0 || n < 0 || P < 1 || !fits_int(T * P * 12) || !fits_int(T * N * 3) || !fits_int(T * n * 3))
+        return REART_ERR_INVALID_ARG;
+    if (P > 32) return REART_ERR_UNSUPPORTED;
+    if (T == 0) return REART_OK;
+    if (n == 0 || N == 0 || !skinned || !cano || !src_idx || !tgt || !col4row || !sample_order || !part_offsets || !gR ||
+        !gtr || !loss)
+        return REART_ERR_INVALID_ARG;
+    Carver ws(workspace, workspace_bytes);
+    double* partials = ws.take<double>(kin_assign_blocks(T, P));
+    unsigned* ticket = ws.take<unsigned>(1);
+    if (!ws.ok) return REART_ERR_WORKSPACE;
+    KinAssign a = {};
+    a.skinned = skinned; a.cano = cano; a.src_idx = src_idx; a.tgt = tgt; a.col4row = col4row;
+    a.sample_order = sample_order; a.part_offsets = part_offsets; a.lambda = lambda;
+    a.gR = gR; a.gtr = gtr; a.loss = loss; a.accumulate = accumulate ? 1 : 0;
+    a.partials = partials; a.ticket = ticket;
+    a.T = (int)T; a.N = (int)N; a.n = (int)n; a.P = (int)P;
+    return launch_kin_assign(a, static_cast<cudaStream_t>(stream_));
+}
+
 int reart_rot6d_fwd(const float* d6, int64_t B, float* R, void* stream_) {
     REART_ENTRY();
     if (B < 0) return REART_ERR_INVALID_ARG;

@@ -239,6 +239,25 @@ struct KinTail {
 };
 int64_t kin_tail_workspace_floats(int64_t T, int64_t P);
 int launch_kin_tail(const KinTail& a, cudaStream_t stream);
+// Assignment loss of the kinematic model straight into the pose gradients (one-hot skinning weights).
+struct KinAssign {
+    const float* skinned;         // [T,N,3]
+    const float* cano;            // [N,3]
+    const int64_t* src_idx;       // [n] sampled canonical points
+    const float* tgt;             // [T,n,3] sampled target points
+    const int32_t* col4row;       // [T,n] target sample matched to source sample i
+    const int32_t* sample_order;  // [n] sample indices grouped by part (stable)
+    const int32_t* part_offsets;  // [P+1] part p owns sample_order[part_offsets[p] .. part_offsets[p+1])
+    float lambda;
+    float* gR; float* gtr;        // [T,P,9], [T,P,3]
+    double* loss;                 // [1]
+    int accumulate;               // add to gR / gtr / loss, else overwrite them
+    double* partials;             // [kin_assign_blocks(T,P)]
+    unsigned* ticket;             // [1] zero before the FIRST call; the kernel re-arms it
+    int T, N, n, P;
+};
+int64_t kin_assign_blocks(int64_t T, int64_t P);
+int launch_kin_assign(const KinAssign& a, cudaStream_t stream);
 
 int launch_allreduce_oneshot(const unsigned long long* peer_base, int rank, int world, int64_t n, int64_t n_pad,
                              unsigned* epoch, float* data, cudaStream_t stream);

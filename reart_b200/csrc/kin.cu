@@ -222,4 +222,90 @@ int launch_kin_tail(const KinTail& a, cudaStream_t stream) {
     return kOk;
 }
 
+// ============================================================================================ assignment loss
+// The matched-pair loss of run_robot.py:181-187 and its gradient w.r.t. the poses.  The kinematic model's skinning
+// weights are one-hot rows (the label transfer), so d loss / d (R, tr) of part p in frame t is a plain sum over the
+// samples of that part -- reading only the T*n sampled points instead of a [T,N,3] gradient through the full skin backward:
+//   d = skinned[t, src_idx[i]] - tgt[t, col4row[t,i]],  x = cano[src_idx[i]],  g = 2 lambda d
+//   loss += lambda sum |d|^2 ;  gR[t,p] += sum g x^T ;  gtr[t,p] += sum g.
+// One warp per (frame, part): lane l takes the part's samples l, l+32, ... (sample_order groups them by part), then a
+// fixed xor tree.  The loss: per-CTA partials, the last CTA (ticket) adds them in index order and re-arms the ticket.
+constexpr int kKinAssignWarps = 4;
+
+int64_t kin_assign_blocks(int64_t T, int64_t P) { return T * ceil_div(P, (int64_t)kKinAssignWarps); }
+
+__global__ void __launch_bounds__(32 * kKinAssignWarps) kin_assign_kernel(const KinAssign a) {
+    __shared__ double s_loss[kKinAssignWarps];
+    __shared__ bool s_last;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int t = blockIdx.x, p = blockIdx.y * kKinAssignWarps + w;
+    double loss = 0.0;
+    if (p < a.P) {
+        const int k0 = a.part_offsets[p], k1 = a.part_offsets[p + 1];
+        const float s = 2.0f * a.lambda;
+        float acc[12];
+#pragma unroll
+        for (int k = 0; k < 12; ++k) acc[k] = 0.f;
+        for (int k = k0 + lane; k < k1; k += 32) {
+            const int i = a.sample_order[k];
+            const int64_t si = a.src_idx[i];
+            const int j = a.col4row[(int64_t)t * a.n + i];
+            const float* sp = a.skinned + ((int64_t)t * a.N + si) * 3;
+            const float* tp = a.tgt + ((int64_t)t * a.n + (j >= 0 ? j : 0)) * 3;
+            const float* x = a.cano + si * 3;
+            const float dx = sp[0] - tp[0], dy = sp[1] - tp[1], dz = sp[2] - tp[2];
+            loss += (double)(dx * dx + dy * dy + dz * dz);
+            const float g[3] = {s * dx, s * dy, s * dz};
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                acc[3 * r] += g[r] * x[0]; acc[3 * r + 1] += g[r] * x[1]; acc[3 * r + 2] += g[r] * x[2];
+                acc[9 + r] += g[r];
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 12; ++k)
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+        const int64_t tp = (int64_t)t * a.P + p;
+        if (lane < 12 && (k1 > k0 || !a.accumulate)) {          // a part without samples keeps its gradient (or gets zeros)
+            float v = 0.f;
+#pragma unroll
+            for (int k = 0; k < 12; ++k) v = lane == k ? acc[k] : v;
+            float* o = lane < 9 ? a.gR + tp * 9 + lane : a.gtr + tp * 3 + (lane - 9);
+            *o = a.accumulate ? *o + v : v;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) loss += __shfl_xor_sync(0xffffffffu, loss, o);
+    if (lane == 0) s_loss[w] = loss;
+    __syncthreads();
+    const int nblk = gridDim.x * gridDim.y, blk = blockIdx.y * gridDim.x + blockIdx.x;
+    if (threadIdx.x == 0) {
+        double c = 0.0;
+#pragma unroll
+        for (int q = 0; q < kKinAssignWarps; ++q) c += s_loss[q];
+        a.partials[blk] = c;
+        __threadfence();
+        s_last = atomicAdd(a.ticket, 1u) == (unsigned)nblk - 1u;
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x == 0) {
+        __threadfence();
+        const volatile double* v = a.partials;
+        double tot = 0.0;
+        for (int b = 0; b < nblk; ++b) tot += v[b];
+        *a.loss = a.accumulate ? *a.loss + (double)a.lambda * tot : (double)a.lambda * tot;
+        *a.ticket = 0u;                                       // re-armed for the next launch (graph replay)
+    }
+}
+
+int launch_kin_assign(const KinAssign& a, cudaStream_t stream) {
+    if (a.T <= 0) return kOk;
+    if (a.P <= 0 || a.P > 32) return kErrUnsupported;
+    dim3 grid((unsigned)a.T, (unsigned)ceil_div(a.P, kKinAssignWarps));
+    kin_assign_kernel<<<grid, 32 * kKinAssignWarps, 0, stream>>>(a);
+    REART_CHECK_LAUNCH();
+    return kOk;
+}
+
 }  // namespace reart

@@ -84,11 +84,44 @@ class _EngineBase:
 
     def _aux_state_tensors(self):
         """Other device state an iteration carries from step to step (restored after a capture's warm-up)."""
-        return []
+        aux = [self.assign.col4row, self.assign.dual_u] if self.assign is not None else []
+        if getattr(self, "native", False) and (getattr(self, "cull", False) or self.search_culled):
+            aux += [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
+        return aux
+
+    # ------------------------------------------------------------------------------------------ iteration flavours
+    def _setup_assign(self, assign: Optional[dict], sample=None):
+        """assign: None or dict(downsample, assign_gap, lambda_assign, assign_iter, mode="add"|"replace") -> self.assign
+        (an ``AssignLoss`` on the engine's clouds), self.assign_iter, self.assign_mode.  ``sample(n)`` -> (src_idx, tgt_idx):
+        the FPS samples when the engine's clouds are not in the caller's order."""
+        self.assign = None
+        if assign is None:
+            return
+        from .assign import AssignLoss
+        cfg = dict(assign)
+        self.assign_iter = int(cfg.pop("assign_iter", 0))
+        self.assign_mode = cfg.pop("mode", "add")
+        if self.assign_mode not in ("add", "replace"):
+            raise ValueError("assign mode must be 'add' (run_real/run_sapien) or 'replace' (run_robot)")
+        if sample is not None:
+            cfg["src_idx"], cfg["tgt_idx"] = sample(self.cano.shape[0] // int(cfg.get("downsample", 4)))
+        self.assign = AssignLoss(self.cano, self.frames, **cfg)
+
+    def _phase(self):
+        """(use_chamfer, use_assign, refresh) of the iteration that is about to run (self.iteration is 1-based)."""
+        if self.assign is None:
+            return True, False, False
+        i = self.iteration - 1
+        if i < self.assign_iter:
+            return True, False, False
+        return self.assign_mode == "add", True, self.assign.due(i, self.assign_iter)
 
     def _variant(self):
         """Which flavour of the iteration the NEXT step runs (hashable); one CUDA graph is captured per flavour."""
-        return None
+        return self._phase()
+
+    def _step_phase(self):
+        return getattr(self, "_cur_variant", None) or self._phase()
 
     def _capture(self, variant):
         """Warm up (allocator, library handles, NCCL communicator, lazily created Adam state), capture one
@@ -170,7 +203,8 @@ class _EngineBase:
             self._ingest_src = None
 
     def _after_replay(self, variant):
-        pass
+        if variant[2]:
+            self.assign.have_assignment = True
 
     # ------------------------------------------------------------------------------------------ search of the energy
     def _setup_search(self, search: str, can_order: bool, why: str):
@@ -323,25 +357,17 @@ class RelaxationEngine(_EngineBase):
         self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
         # recon-only iterations run on the fused head / energy / tail kernels with the library's own Adam (8 launches per
         # step, no autograd); extra losses on the skinned cloud (flow) keep the autograd composition
-        self.assign = None
-        if assign is not None:
-            from .assign import AssignLoss
-            cfg = dict(assign)
-            self.assign_iter = int(cfg.pop("assign_iter", 0))
-            self.assign_mode = cfg.pop("mode", "add")
-            if self.assign_mode not in ("add", "replace"):
-                raise ValueError("assign mode must be 'add' (run_real/run_sapien) or 'replace' (run_robot)")
-            if self.cull:
-                # sample the clouds in the CALLER's order (FPS starts at the caller's point 0, like the reference's
-                # kernel), then express the samples in engine order
-                from .assign import farthest_point_sample
-                n_fps = self.cano.shape[0] // int(cfg.get("downsample", 4))
-                inv_c = torch.empty_like(self.perm_cano); inv_c[self.perm_cano] = torch.arange(len(inv_c), device=dev)
-                inv_f = torch.empty_like(self.perm_frames)
-                inv_f.scatter_(1, self.perm_frames, torch.arange(inv_f.shape[1], device=dev)[None].expand_as(inv_f))
-                cfg["src_idx"] = inv_c[farthest_point_sample(cano_orig[None], n_fps)[0]]
-                cfg["tgt_idx"] = torch.gather(inv_f, 1, farthest_point_sample(frames_orig, n_fps))
-            self.assign = AssignLoss(self.cano, self.frames, **cfg)
+        def sample_in_caller_order(n_fps):
+            # sample the clouds in the CALLER's order (FPS starts at the caller's point 0, like the reference's kernel),
+            # then express the samples in engine order
+            from .assign import farthest_point_sample
+            inv_c = torch.empty_like(self.perm_cano); inv_c[self.perm_cano] = torch.arange(len(inv_c), device=dev)
+            inv_f = torch.empty_like(self.perm_frames)
+            inv_f.scatter_(1, self.perm_frames, torch.arange(inv_f.shape[1], device=dev)[None].expand_as(inv_f))
+            return (inv_c[farthest_point_sample(cano_orig[None], n_fps)[0]],
+                    torch.gather(inv_f, 1, farthest_point_sample(frames_orig, n_fps)))
+
+        self._setup_assign(assign, sample_in_caller_order if self.cull else None)
         self.native = (flow_ref is None) if native is None else bool(native)
         if self.native:
             if flow_ref is not None:
@@ -418,32 +444,6 @@ class RelaxationEngine(_EngineBase):
         if self.native:
             return [self._nat[k] for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr", "step")]
         return super()._opt_state_tensors()
-
-    def _aux_state_tensors(self):
-        aux = [self.assign.col4row, self.assign.dual_u] if self.assign is not None else []
-        if self.native and (self.cull or self.search_culled):
-            aux += [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
-        return aux
-
-    # ------------------------------------------------------------------------------------------ iteration flavours
-    def _phase(self):
-        """(use_chamfer, use_assign, refresh) of the iteration that is about to run (self.iteration is 1-based)."""
-        if self.assign is None:
-            return True, False, False
-        i = self.iteration - 1
-        if i < self.assign_iter:
-            return True, False, False
-        return self.assign_mode == "add", True, self.assign.due(i, self.assign_iter)
-
-    def _variant(self):
-        return self._phase()
-
-    def _after_replay(self, variant):
-        if variant[2]:
-            self.assign.have_assignment = True
-
-    def _step_phase(self):
-        return getattr(self, "_cur_variant", None) or self._phase()
 
     def _energy_call(self, L, b, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
         """The fused energy evaluation of this step: brute-force or culled search (``_search_energy``), the culled search on
@@ -566,16 +566,20 @@ class RelaxationEngine(_EngineBase):
 
 
 class KinematicEngine(_EngineBase):
-    """Projection model (networks/model.py KinematicModel) + recon loss, frame-sharded.
+    """Projection model (networks/model.py KinematicModel) + recon loss (+ the optional assignment loss), frame-sharded.
     axis/moment are shared (all-reduced); theta/distance/root pose are per frame."""
 
     def __init__(self, model_kwargs: dict, seg_part: torch.Tensor, cano: torch.Tensor, frames: torch.Tensor,
                  ctx: Optional[DistContext] = None, lr: float = 1e-2, weight_decay: float = 0.0,
-                 use_graph: bool = True, native: bool = False, search: str = "auto", betas=(0.9, 0.999), eps: float = 1e-8):
+                 use_graph: bool = True, native: bool = False, search: str = "auto", betas=(0.9, 0.999), eps: float = 1e-8,
+                 assign: Optional[dict] = None):
         """native=True runs the iteration on library kernels -- kin_head -> fused energy -> kin_tail (FK backward, frame
         sums in a fixed order, [all-reduce], the library's Adam) -- with no autograd: the same optimisation as the default
         autograd composition, bit-reproducible.  search: "brute" | "culled" | "auto" as for ``RelaxationEngine`` (native
-        iteration only; "culled" is bit-identical to "brute")."""
+        iteration only; "culled" is bit-identical to "brute").
+        assign: the assignment loss, dict(downsample, assign_gap, lambda_assign, assign_iter, mode="add"|"replace") as for
+        ``RelaxationEngine``; the native iteration adds its pose gradients with ``reart_kin_assign``.  The frames' samples are
+        taken once here, so ``step(ingest=...)`` is not available with it."""
         super().__init__(ctx, use_graph)
         from .knn_module import KNN
         dev = cano.device
@@ -596,8 +600,12 @@ class KinematicEngine(_EngineBase):
                                     knn=KNN(k=1, transpose_mode=True), **kw).to(dev)
         self.tau = torch.ones((), device=dev)
         with torch.no_grad():                                       # constant label transfer (SURVEY Q27)
-            self.weight = F.one_hot(self.model._labels(self.model.cano_pc), num_classes=self.model.num_parts).float()
+            self.labels = self.model._labels(self.model.cano_pc)
+            self.weight = F.one_hot(self.labels, num_classes=self.model.num_parts).float()
         self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
+        if assign is not None and self.cano.shape[0] // int(assign.get("downsample", 4)) < 1:
+            raise ValueError(f"downsample leaves no assignment samples of {self.cano.shape[0]} points")
+        self._setup_assign(assign)
         if self.native:
             self.optimizer = self.bucket = None
             self._init_native(lr, weight_decay, betas, eps)
@@ -607,11 +615,25 @@ class KinematicEngine(_EngineBase):
                                               capturable=use_graph, fused=True)
             self.bucket = GradBucket([self.model.axis_list, self.model.moment_list], extra_scalars=1)
 
+    def step(self, tau: Optional[float] = None, ingest=None) -> torch.Tensor:
+        if ingest is not None and self.assign is not None:
+            raise ValueError("ingest is not available with the assignment loss: the frames' samples are taken once at set-up")
+        return super().step(tau, ingest)
+
     def _iteration(self):
+        use_chamfer, use_assign, refresh = self._step_phase()
         trans = self.model.transforms()
-        loss, skinned = ops.skinned_chamfer_loss(self.cano, self.weight, trans[:, :, :3, :3].contiguous(),
-                                                 trans[:, :, :3, 3].contiguous(), self.frames, self.frames_packed,
-                                                 unit_grad=True)
+        R, tr = trans[:, :, :3, :3].contiguous(), trans[:, :, :3, 3].contiguous()
+        if use_chamfer:
+            loss, skinned = ops.skinned_chamfer_loss(self.cano, self.weight, R, tr, self.frames, self.frames_packed,
+                                                     unit_grad=True)
+        else:                                                       # run_robot.py:164-192: assignment only
+            skinned = ops.skin(self.cano, self.weight, R, tr)
+            loss = skinned.new_zeros(())
+        if use_assign:
+            if refresh:
+                self.assign.refresh(skinned)
+            loss = loss + self.assign.loss(skinned)
         self.skinned = skinned.detach()
         return loss
 
@@ -655,6 +677,13 @@ class KinematicEngine(_EngineBase):
         b["loss_out"] = torch.zeros(1, **f32)
         if self.search_culled:
             self._search_buffers(b, T, N, M)
+        if self.assign is not None:
+            # the samples grouped by part, once: reart_kin_assign sums each (frame, part) over its own samples
+            sample_part = self.labels[self.assign.src_idx]
+            b["sample_order"] = torch.argsort(sample_part, stable=True).int()
+            b["part_offsets"] = torch.cat((sample_part.new_zeros(1), torch.bincount(sample_part, minlength=P).cumsum(0))).int()
+            b["assign_ws_bytes"] = int(L.reart_kin_assign_workspace_bytes(T, P))
+            b["assign_ws"] = torch.zeros(b["assign_ws_bytes"], dtype=torch.uint8, device=dev)
         self.weight = self.weight.contiguous()
         red = make_small_all_reduce(self.ctx, 6 * E + 1, dev)
         oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
@@ -691,23 +720,32 @@ class KinematicEngine(_EngineBase):
             return [self._nat[k] for k in ("m", "v", "step")]
         return super()._opt_state_tensors()
 
-    def _aux_state_tensors(self):
-        if self.native and self.search_culled:
-            return [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
-        return []
-
     def _run_iteration_native(self):
         """kin_head -> [memset, skin (x-sorted copy), (cull bounds,) search, energy columns, energy rows, skin backward,
-        reduce] -> kin_tail."""
+        reduce] -> kin_tail.  With the assignment loss: kin_head -> energy ("add") or skin ("replace") -> [reart_lap on
+        refresh steps] -> kin_assign -> kin_tail."""
         import ctypes
         from . import _lib
-        from ._lib import check, stream_ptr
+        from ._lib import check, ptr, stream_ptr
         L = _lib.lib()
         b = self._nat
         T, N, M, P = b["dims"]
+        use_chamfer, use_assign, refresh = self._step_phase()
         with torch.cuda.device(self.cano.device):
             check(L.reart_kin_head(*b["head"], stream_ptr()), "reart_kin_head")
-            self._search_energy(L, b, self.weight, b["R"], b["tr"], T, N, M, P, b["gW"], b["gR"], b["gtr"], None, 1)
+            if use_chamfer:
+                self._search_energy(L, b, self.weight, b["R"], b["tr"], T, N, M, P, b["gW"], b["gR"], b["gtr"], None, 1)
+            else:                                                 # run_robot.py:164-192: the assignment loss REPLACES Chamfer
+                check(L.reart_skin_fwd(ptr(self.cano), ptr(self.weight), ptr(b["R"]), ptr(b["tr"]), T, N, P, ptr(b["skinned"]),
+                                       stream_ptr()), "reart_skin_fwd")
+            if use_assign:
+                if refresh:
+                    self.assign.refresh(b["skinned"])
+                s = self.assign
+                check(L.reart_kin_assign(ptr(b["skinned"]), ptr(self.cano), ptr(s.src_idx), ptr(s.pc_tgt), ptr(s.col4row),
+                                         ptr(b["sample_order"]), ptr(b["part_offsets"]), s.lambda_assign, T, N, s.num_fps, P,
+                                         ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), 1 if use_chamfer else 0,
+                                         ptr(b["assign_ws"]), b["assign_ws_bytes"], stream_ptr()), "reart_kin_assign")
             a = b["args"]
             if not b["nccl"]:
                 check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
