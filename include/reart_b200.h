@@ -214,6 +214,9 @@ REART_API int reart_gumbel_st_bwd(const float* ysoft, const float* tau, const fl
  *       first call only (the kernel re-arms them).
  *       phase 0: everything; phase 1: gradients -> bucket only (caller reduces the bucket, e.g. with NCCL);
  *       phase 2: Adam from the reduced bucket.
+ * limits: P <= 32 for both.  The head stages w0/b0/w2 in shared memory and rejects H*(8+PMAX)*4 > 48 KB with
+ *       REART_ERR_UNSUPPORTED, PMAX being P rounded up to 8, 16 or 32 (e.g. P > 16 with H > 307 is unsupported).  The tail
+ *       supports H <= 256 (REART_ERR_UNSUPPORTED above that).
  * ------------------------------------------------------------------------------------------- */
 REART_API int reart_relax_head(const float* cano, const float* w0, const float* b0, const float* w2, const float* expo,
                                const int64_t* noise_index, const float* tau, const float* d6, int64_t N, int64_t H, int64_t P, int64_t T,

@@ -221,14 +221,17 @@ __global__ void __launch_bounds__(NT) lap_jv_kernel(const float* __restrict__ sr
 
 template <int NT>
 static int launch_lap_nt(const float* src_base, const int64_t* src_idx, int64_t src_stride, const float* tgt, int64_t B,
-                         int64_t n, int* col4row, double* total, double* dual_u, int warm, cudaStream_t stream) {
+                         int64_t n, int n_max, int* col4row, double* total, double* dual_u, int warm, cudaStream_t stream) {
     const size_t smem = (size_t)n * (16 + 8 + 8 + 4 * 4);
     static bool attr_done[64] = {};
     int devid = 0;
     cudaGetDevice(&devid);
-    // static shared memory (reduction slots) comes on top of the dynamic part: opt in well below the 48 KB default limit
+    // static shared memory (reduction slots) comes on top of the dynamic part: opt in well below the 48 KB default limit.
+    // smem grows with n, so the opt-in is made once per device for the bucket's LARGEST n: a later call with a larger n
+    // than the first must not exceed what was opted in
     if (smem > 32 * 1024 && (devid < 0 || devid >= 64 || !attr_done[devid])) {
-        if (cudaFuncSetAttribute(lap_jv_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+        const size_t smem_max = (size_t)n_max * (16 + 8 + 8 + 4 * 4);
+        if (cudaFuncSetAttribute(lap_jv_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max) != cudaSuccess)
             return kErrUnsupported;
         if (devid >= 0 && devid < 64) attr_done[devid] = true;
     }
@@ -242,10 +245,10 @@ int launch_lap(const float* src_base, const int64_t* src_idx, int64_t src_stride
                int* col4row, double* total, double* dual_u, int warm, cudaStream_t stream) {
     if (B <= 0 || n <= 0) return kOk;
     if (n > 4096) return kErrUnsupported;
-    if (n <= 512) return launch_lap_nt<128>(src_base, src_idx, src_stride, tgt, B, n, col4row, total, dual_u, warm, stream);
-    if (n <= 1024) return launch_lap_nt<256>(src_base, src_idx, src_stride, tgt, B, n, col4row, total, dual_u, warm, stream);
-    if (n <= 2048) return launch_lap_nt<512>(src_base, src_idx, src_stride, tgt, B, n, col4row, total, dual_u, warm, stream);
-    return launch_lap_nt<1024>(src_base, src_idx, src_stride, tgt, B, n, col4row, total, dual_u, warm, stream);
+    if (n <= 512) return launch_lap_nt<128>(src_base, src_idx, src_stride, tgt, B, n, 512, col4row, total, dual_u, warm, stream);
+    if (n <= 1024) return launch_lap_nt<256>(src_base, src_idx, src_stride, tgt, B, n, 1024, col4row, total, dual_u, warm, stream);
+    if (n <= 2048) return launch_lap_nt<512>(src_base, src_idx, src_stride, tgt, B, n, 2048, col4row, total, dual_u, warm, stream);
+    return launch_lap_nt<1024>(src_base, src_idx, src_stride, tgt, B, n, 4096, col4row, total, dual_u, warm, stream);
 }
 
 // ---------------------------------------------------------------------------------------------- matched-pair loss

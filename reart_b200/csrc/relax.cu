@@ -386,14 +386,17 @@ int launch_relax_tail(const RelaxTail& a, cudaStream_t stream) {
     const int point_blocks = (int)ceil_div(a.N, kTailPoints);
     const int pose_blocks = (int)ceil_div((int64_t)a.T * a.P, threads);
     if (a.world > 1 && a.phase == 0 && (a.world > threads || !a.peer_base || !a.epoch)) return kErrInvalidArg;
+    // smem grows with H (through Hpad), so the >48 KB opt-in is made once per device for the instantiation's LARGEST
+    // launch (Hpad = 256): a later call with a larger H than the first must not exceed what was opted in
 #define REART_TAIL(PM)                                                                                                 \
     do {                                                                                                               \
         const size_t smem = ((size_t)kTailPoints * (4 + PM) + (size_t)3 * Hpad * (4 + PM)) * sizeof(float);           \
+        const size_t smem_max = ((size_t)kTailPoints * (4 + PM) + (size_t)3 * 256 * (4 + PM)) * sizeof(float);        \
         static bool attr_done[64] = {};                                                                                \
         int devid = 0;                                                                                                 \
         cudaGetDevice(&devid);                                                                                         \
         if (smem > 48 * 1024 && (devid < 0 || devid >= 64 || !attr_done[devid])) {                                     \
-            if (cudaFuncSetAttribute(relax_tail_kernel<PM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) \
+            if (cudaFuncSetAttribute(relax_tail_kernel<PM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max) != cudaSuccess) \
                 return kErrUnsupported;                                                                                \
             if (devid >= 0 && devid < 64) attr_done[devid] = true;                                                     \
         }                                                                                                              \
