@@ -301,6 +301,35 @@ REART_API int reart_kin_assign(const float* skinned, const float* cano, const in
                                float lambda, int64_t T, int64_t N, int64_t n, int64_t P, float* gR, float* gtr,
                                double* loss, int accumulate, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* The flow loss of the kinematic model (run_robot.py:194-213, networks/loss.py:10-21) straight into the pose gradients,
+ * between the energy (or reart_skin_fwd) and reart_kin_tail.  Same premise as reart_kin_assign: one-hot skinning weights,
+ * so the gradient w.r.t. (R, tr) of part p in frame t is a sum over the points of part p.  The kernel works on a WINDOW
+ * of the complete sequence (canonical cloud inserted at cano_idx): win [K,N,3] holds K consecutive complete frames,
+ * tflow [K-1,N,3] / mask [K-1,N] (uint8, as reart_knn3_blend writes them) the blended target flow of pair k = (slot k,
+ * slot k+1), slot_frame [K] int32 the local frame of each slot (-1: the canonical cloud or a neighbour rank's frame).
+ *   pred_k = win[k+1] - win[k],  err_k = pred_k - tflow[k],  per point and component d_k = d flow_loss / d pred_k:
+ *     mask set, plain: 2 err;  mask set, robust: err where |err| < 1, else sign(err) (|err| == 1 takes the linear branch,
+ *     as torch.where(a < 1, ...) does);  mask clear: 2 * 0.01 * pred.
+ *   slot s holding local frame t, point i of part p, x = cano[i]:  g = lambda (d_{s-1} - d_s) (a pair outside the window
+ *   is dropped);  gR[t,p] += sum g x^T,  gtr[t,p] += sum g.
+ *   loss += lambda * sum over the pairs [q0, q1) of the window of the per-point terms (mask set: |err|^2, or the Huber
+ *   terms 0.5 e^2 / |e| - 0.5 when robust; mask clear: 0.01 |pred|^2).  Pair k is counted by slot k+1 when that slot
+ *   is local, else by slot k (a counted pair needs a local slot).
+ * A frame's gradient depends only on its own slot and the two adjacent ones: a sub-window that holds a frame's
+ * neighbours gives that frame the bits of the whole-sequence call.  point_order [N]: the point indices stably sorted by
+ * part, part_offsets [P+1]: part p owns point_order[part_offsets[p] .. part_offsets[p+1]).  gR [T,P,3,3], gtr [T,P,3],
+ * loss [1] double: accumulate != 0 adds to them, else overwrites them (every local frame's (t, p) is written; a part
+ * without points gets zeros, with accumulate it is left untouched).  No float atomics: bit-reproducible.  workspace:
+ * reart_kin_flow_workspace_bytes(K,P), zero before the FIRST call (the kernel re-arms it).  P <= 32, K >= 2,
+ * 0 <= q0 <= q1 <= K-1; T == 0 is an empty problem.
+ * ------------------------------------------------------------------------------------------- */
+REART_API int64_t reart_kin_flow_workspace_bytes(int64_t K, int64_t P);
+REART_API int reart_kin_flow(const float* win, const float* tflow, const uint8_t* mask, const int32_t* slot_frame,
+                             const float* cano, const int32_t* point_order, const int32_t* part_offsets, float lambda,
+                             int robust, int64_t K, int64_t N, int64_t P, int64_t T, int64_t q0, int64_t q1, float* gR,
+                             float* gtr, double* loss, int accumulate, void* workspace, int64_t workspace_bytes,
+                             void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * 6D rotation representation -> matrix (Gram-Schmidt).
  * Replaces screw_se3/geo_utils.py:632-651 (rotation_6d_to_matrix); d6 [B,6] -> R [B,3,3].

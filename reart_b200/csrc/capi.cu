@@ -549,6 +549,36 @@ int reart_kin_assign(const float* skinned, const float* cano, const int64_t* src
     return launch_kin_assign(a, static_cast<cudaStream_t>(stream_));
 }
 
+int64_t reart_kin_flow_workspace_bytes(int64_t K, int64_t P) {
+    if (K < 2 || P < 1 || P > 32) return -1;
+    return align_up(kin_flow_blocks(K, P) * 8) + align_up(4) + kAlign;
+}
+
+int reart_kin_flow(const float* win, const float* tflow, const uint8_t* mask, const int32_t* slot_frame, const float* cano,
+                   const int32_t* point_order, const int32_t* part_offsets, float lambda, int robust, int64_t K, int64_t N,
+                   int64_t P, int64_t T, int64_t q0, int64_t q1, float* gR, float* gtr, double* loss, int accumulate,
+                   void* workspace, int64_t workspace_bytes, void* stream_) {
+    REART_ENTRY();
+    if (T < 0 || K < 0 || N < 0 || P < 1 || !fits_int(T * P * 12) || !fits_int(K * N * 3) || !fits_int(K * P))
+        return REART_ERR_INVALID_ARG;
+    if (P > 32) return REART_ERR_UNSUPPORTED;
+    if (T == 0) return REART_OK;
+    if (K < 2 || N == 0 || q0 < 0 || q1 < q0 || q1 > K - 1) return REART_ERR_INVALID_ARG;
+    if (!win || !tflow || !mask || !slot_frame || !cano || !point_order || !part_offsets || !gR || !gtr || !loss)
+        return REART_ERR_INVALID_ARG;
+    Carver ws(workspace, workspace_bytes);
+    double* partials = ws.take<double>(kin_flow_blocks(K, P));
+    unsigned* ticket = ws.take<unsigned>(1);
+    if (!ws.ok) return REART_ERR_WORKSPACE;
+    KinFlow a = {};
+    a.win = win; a.tflow = tflow; a.mask = mask; a.slot_frame = slot_frame; a.cano = cano;
+    a.point_order = point_order; a.part_offsets = part_offsets; a.lambda = lambda; a.robust = robust ? 1 : 0;
+    a.gR = gR; a.gtr = gtr; a.loss = loss; a.accumulate = accumulate ? 1 : 0;
+    a.partials = partials; a.ticket = ticket;
+    a.K = (int)K; a.N = (int)N; a.P = (int)P; a.T = (int)T; a.q0 = (int)q0; a.q1 = (int)q1;
+    return launch_kin_flow(a, static_cast<cudaStream_t>(stream_));
+}
+
 int reart_rot6d_fwd(const float* d6, int64_t B, float* R, void* stream_) {
     REART_ENTRY();
     if (B < 0) return REART_ERR_INVALID_ARG;

@@ -258,6 +258,26 @@ struct KinAssign {
 };
 int64_t kin_assign_blocks(int64_t T, int64_t P);
 int launch_kin_assign(const KinAssign& a, cudaStream_t stream);
+// Flow loss of the kinematic model straight into the pose gradients, on a window of the complete sequence.
+struct KinFlow {
+    const float* win;             // [K,N,3] consecutive complete frames
+    const float* tflow;           // [K-1,N,3] blended target flow of pair k = (slot k, slot k+1)
+    const uint8_t* mask;          // [K-1,N]
+    const int32_t* slot_frame;    // [K] local frame of each slot, -1: canonical cloud or a neighbour rank's frame
+    const float* cano;            // [N,3]
+    const int32_t* point_order;   // [N] point indices grouped by part (stable)
+    const int32_t* part_offsets;  // [P+1]
+    float lambda;
+    int robust;
+    float* gR; float* gtr;        // [T,P,9], [T,P,3]
+    double* loss;                 // [1]
+    int accumulate;               // add to gR / gtr / loss, else overwrite them
+    double* partials;             // [kin_flow_blocks(K,P)]
+    unsigned* ticket;             // [1] zero before the FIRST call; the kernel re-arms it
+    int K, N, P, T, q0, q1;       // the loss counts the pairs [q0, q1) of the window
+};
+int64_t kin_flow_blocks(int64_t K, int64_t P);
+int launch_kin_flow(const KinFlow& a, cudaStream_t stream);
 
 int launch_allreduce_oneshot(const unsigned long long* peer_base, int rank, int world, int64_t n, int64_t n_pad,
                              unsigned* epoch, float* data, cudaStream_t stream);

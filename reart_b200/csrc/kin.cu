@@ -308,4 +308,145 @@ int launch_kin_assign(const KinAssign& a, cudaStream_t stream) {
     return kOk;
 }
 
+// ============================================================================================ flow loss
+// The flow loss of run_robot.py:194-213 (networks/loss.py:10-21) and its gradient w.r.t. the poses, on a window of K
+// consecutive frames of the complete sequence.  With one-hot skinning weights, slot s holding local frame t:
+//   pred_k = win[k+1] - win[k],  err_k = pred_k - tflow[k],  d_k = d flow_loss / d pred_k (per point, per component):
+//     mask set: 2 err (plain) | err if |err| < 1 else sign(err) (robust);  mask clear: 2 * 0.01 * pred
+//   g = lambda (d_{s-1} - d_s)  (a term outside the window is dropped);  gR[t,p] += sum g x^T,  gtr[t,p] += sum g.
+// One CTA per (slot, part): thread j takes the part's points j, j+256, ... (point_order groups them by part), then a fixed
+// xor tree per warp and the warps in order.  Pair k's loss is counted (if q0 <= k < q1) by the units of slot k+1 when
+// that slot is local, else of slot k.  The loss: per-CTA partials added in index order by the last CTA (ticket).
+constexpr int kKinFlowThreads = 256;
+constexpr float kFlowSmoothWeight = 1e-2f;                   // networks/loss.py:10 smooth_weight
+
+int64_t kin_flow_blocks(int64_t K, int64_t P) { return K * P; }
+
+// d flow_loss / d pred (one component) and the per-component loss term
+__device__ __forceinline__ float flow_term_grad(float pred, float tgt, bool keep, int robust, float& term) {
+    if (!keep) {
+        term = kFlowSmoothWeight * (pred * pred);
+        return 2.0f * kFlowSmoothWeight * pred;
+    }
+    const float e = pred - tgt;
+    if (!robust) {
+        term = e * e;
+        return 2.0f * e;
+    }
+    const float a = fabsf(e);
+    if (a < 1.0f) {                                           // torch.where(a < 1, ...): |err| == 1 is the linear branch
+        term = 0.5f * e * e;
+        return e;
+    }
+    term = a - 0.5f;
+    return e > 0.f ? 1.0f : -1.0f;
+}
+
+__global__ void __launch_bounds__(kKinFlowThreads) kin_flow_kernel(const KinFlow a) {
+    constexpr int kWarps = kKinFlowThreads / 32;
+    __shared__ float s_acc[kWarps][12];
+    __shared__ double s_loss[kWarps];
+    __shared__ bool s_last;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int s = blockIdx.x, p = blockIdx.y, K = a.K;
+    const int t = a.slot_frame[s];
+    double loss = 0.0;
+    const bool local = t >= 0 && t < a.T;
+    const int k0 = a.part_offsets[p], k1 = a.part_offsets[p + 1];
+    if (local && k1 > k0) {
+        // which of the two adjacent pairs this unit counts the loss of
+        const bool has_prev = s > 0, has_next = s < K - 1;
+        const bool count_prev = has_prev && s - 1 >= a.q0 && s - 1 < a.q1;           // slot s is the pair's second slot
+        const bool count_next = has_next && s >= a.q0 && s < a.q1 && a.slot_frame[s + 1] < 0;
+        const int64_t N = a.N;
+        float acc[12];
+#pragma unroll
+        for (int k = 0; k < 12; ++k) acc[k] = 0.f;
+        for (int k = k0 + threadIdx.x; k < k1; k += kKinFlowThreads) {
+            const int64_t i = a.point_order[k];
+            const float* ws = a.win + ((int64_t)s * N + i) * 3;
+            float g[3] = {0.f, 0.f, 0.f};
+            float lp = 0.f, ln = 0.f;
+            if (has_prev) {
+                const float* wp = ws - N * 3;
+                const float* tf = a.tflow + ((int64_t)(s - 1) * N + i) * 3;
+                const bool keep = a.mask[(int64_t)(s - 1) * N + i] != 0;
+#pragma unroll
+                for (int r = 0; r < 3; ++r) {
+                    float term;
+                    g[r] = flow_term_grad(ws[r] - wp[r], tf[r], keep, a.robust, term);
+                    lp += term;
+                }
+            }
+            if (has_next) {
+                const float* wn = ws + N * 3;
+                const float* tf = a.tflow + ((int64_t)s * N + i) * 3;
+                const bool keep = a.mask[(int64_t)s * N + i] != 0;
+#pragma unroll
+                for (int r = 0; r < 3; ++r) {
+                    float term;
+                    g[r] -= flow_term_grad(wn[r] - ws[r], tf[r], keep, a.robust, term);
+                    ln += term;
+                }
+            }
+            if (count_prev) loss += (double)lp;
+            if (count_next) loss += (double)ln;
+            const float* x = a.cano + i * 3;
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                const float gr = a.lambda * g[r];
+                acc[3 * r] += gr * x[0]; acc[3 * r + 1] += gr * x[1]; acc[3 * r + 2] += gr * x[2];
+                acc[9 + r] += gr;
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 12; ++k)
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], o);
+        if (lane == 0)
+#pragma unroll
+            for (int k = 0; k < 12; ++k) s_acc[w][k] = acc[k];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) loss += __shfl_xor_sync(0xffffffffu, loss, o);
+    if (lane == 0) s_loss[w] = loss;
+    __syncthreads();
+    if (local && threadIdx.x < 12 && (k1 > k0 || !a.accumulate)) {   // a part without points keeps its gradient (or gets zeros)
+        float v = 0.f;
+        if (k1 > k0)
+            for (int q = 0; q < kWarps; ++q) v += s_acc[q][threadIdx.x];
+        const int64_t tp = (int64_t)t * a.P + p;
+        float* o = threadIdx.x < 9 ? a.gR + tp * 9 + threadIdx.x : a.gtr + tp * 3 + (threadIdx.x - 9);
+        *o = a.accumulate ? *o + v : v;
+    }
+    const int nblk = gridDim.x * gridDim.y, blk = blockIdx.y * gridDim.x + blockIdx.x;
+    if (threadIdx.x == 0) {
+        double c = 0.0;
+#pragma unroll
+        for (int q = 0; q < kWarps; ++q) c += s_loss[q];
+        a.partials[blk] = c;
+        __threadfence();
+        s_last = atomicAdd(a.ticket, 1u) == (unsigned)nblk - 1u;
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x == 0) {
+        __threadfence();
+        const volatile double* v = a.partials;
+        double tot = 0.0;
+        for (int b = 0; b < nblk; ++b) tot += v[b];
+        *a.loss = a.accumulate ? *a.loss + (double)a.lambda * tot : (double)a.lambda * tot;
+        *a.ticket = 0u;                                       // re-armed for the next launch (graph replay)
+    }
+}
+
+int launch_kin_flow(const KinFlow& a, cudaStream_t stream) {
+    if (a.T <= 0) return kOk;
+    if (a.P <= 0 || a.P > 32) return kErrUnsupported;
+    if (a.K < 2) return kErrInvalidArg;
+    dim3 grid((unsigned)a.K, (unsigned)a.P);
+    kin_flow_kernel<<<grid, kKinFlowThreads, 0, stream>>>(a);
+    REART_CHECK_LAUNCH();
+    return kOk;
+}
+
 }  // namespace reart

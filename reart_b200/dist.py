@@ -199,6 +199,48 @@ def flow_pairs_for_rank(T: int, cano_idx: int, lo: int, hi: int):
     return pairs[0], pairs[-1] + 1, a_src, b_src
 
 
+def flow_window_plan(T: int, cano_idx: int, bounds: List[Tuple[int, int]]) -> List[dict]:
+    """The windows and the neighbour-frame exchange of the native kinematic flow step (``reart_kin_flow``), for every rank
+    at once: plain host arithmetic on (T skinned frames, cano_idx, shard bounds [(lo, hi)] per rank), so every rank
+    computes the same plan.
+
+    Rank r's window is complete indices [j0, j0 + K) with j0 = max(0, j(lo) - 1) and j0 + K - 1 = min(T, j(hi - 1) + 1),
+    j(g) the complete index of skinned frame g: its frames and both their neighbours.  Per rank a dict with
+      j0, K;  slots: per slot ("local", i) | ("cano",) | ("prev",) (rank r-1's last frame) | ("next",) (rank r+1's first);
+      q0, q1: the pairs of the window whose loss the rank counts (``flow_pairs_for_rank``'s, window-relative);
+      send_prev / send_next: send the first / last local frame to rank r-1 / r+1;  recv_prev / recv_next: the slot that
+      receives rank r-1's last / rank r+1's first frame, or None.
+    Frames only travel forward (no gradient comes back): where the canonical frame separates two shards, nothing is sent."""
+    def j(g):
+        return g if g < cano_idx else g + 1
+
+    plans = []
+    for lo, hi in bounds:
+        j0, j1 = max(0, j(lo) - 1), min(T, j(hi - 1) + 1)
+        slots = []
+        for k in range(j0, j1 + 1):
+            g = None if k == cano_idx else (k if k < cano_idx else k - 1)
+            if g is None:
+                slots.append(("cano",))
+            elif lo <= g < hi:
+                slots.append(("local", g - lo))
+            elif g == lo - 1:
+                slots.append(("prev",))
+            else:
+                assert g == hi, (g, lo, hi)
+                slots.append(("next",))
+        p0, p1, _, _ = flow_pairs_for_rank(T, cano_idx, lo, hi)
+        q0, q1 = (p0 - j0, p1 - j0) if p1 > p0 else (0, 0)
+        assert 0 <= q0 <= q1 <= len(slots) - 1
+        plans.append(dict(j0=j0, K=len(slots), slots=slots, q0=q0, q1=q1,
+                          recv_prev=next((s for s, x in enumerate(slots) if x[0] == "prev"), None),
+                          recv_next=next((s for s, x in enumerate(slots) if x[0] == "next"), None)))
+    for r, pl in enumerate(plans):
+        pl["send_prev"] = r > 0 and plans[r - 1]["recv_next"] is not None
+        pl["send_next"] = r + 1 < len(plans) and plans[r + 1]["recv_prev"] is not None
+    return plans
+
+
 class _HaloPrev(torch.autograd.Function):
     """Forward: every rank sends its last local skinned frame to the next rank and receives the previous rank's
     (rank 0 receives nothing and gets zeros).  Backward: the gradient of the received frame travels back.

@@ -279,6 +279,39 @@ class _EngineBase:
         self._nat["cull_stats"][2].zero_()
         return n
 
+    # ------------------------------------------------------------------------------------------ flow loss
+    def _flow_term(self, pc_trans_list):
+        """run_robot.py:194-209: k=3 blended anchor flow (no grad, ONE launch for all pairs) vs predicted flow."""
+        from .flow_utils import blend_anchor_motion_batched
+        from .loss import flow_loss
+        c = self.cano_idx
+        if self.ctx.world_size == 1:
+            complete = torch.cat((pc_trans_list[:c], self.cano[None], pc_trans_list[c:]), dim=0)
+            with torch.no_grad():
+                target_flow, mask = blend_anchor_motion_batched(complete[:-1].detach().contiguous(), self.flow_ref)
+            pred_flow = complete[1:] - complete[:-1]
+            return flow_loss(target_flow, pred_flow, flow_mask_list=mask, robust=self.robust_flow)
+        # frame-sharded: own pairs [p0, p1), sides taken from local frames, the canonical cloud or the halo frame
+        from .dist import flow_pairs_for_rank, halo_from_previous_rank
+        lo, hi = self.frame_range
+        halo = halo_from_previous_rank(pc_trans_list[-1], self.ctx)          # every rank takes part, even with no pairs
+        # the halo's backward is a matched send/recv: tie it into every rank's loss (weight 0) so it always runs,
+        # also on ranks that do not consume their halo (rank 0) or own no pair
+        anchor = halo.sum() * 0.0
+        p0, p1, a_src, b_src = flow_pairs_for_rank(self.total_frames, c, lo, hi)
+        if p1 <= p0:
+            return anchor
+
+        def pick(src):
+            return self.cano if src[0] == "cano" else (halo if src[0] == "halo" else pc_trans_list[src[1]])
+
+        A = torch.stack([pick(x) for x in a_src])
+        Bm = torch.stack([pick(x) for x in b_src])
+        with torch.no_grad():
+            sub = self.flow_ref.slice(p0, p1)
+            target_flow, mask = blend_anchor_motion_batched(A.detach().contiguous(), sub)
+        return flow_loss(target_flow, Bm - A, flow_mask_list=mask, robust=self.robust_flow) + anchor
+
 
 # search="auto" runs the culled search from this many points per cloud on (both clouds): the coarse bounds of cull.cu
 # start culling there
@@ -532,61 +565,38 @@ class RelaxationEngine(_EngineBase):
         self.skinned = skinned.detach()                         # keep the cloud, not the autograd graph
         return loss
 
-    def _flow_term(self, pc_trans_list):
-        """run_robot.py:194-209: k=3 blended anchor flow (no grad, ONE launch for all pairs) vs predicted flow."""
-        from .flow_utils import blend_anchor_motion_batched
-        from .loss import flow_loss
-        c = self.cano_idx
-        if self.ctx.world_size == 1:
-            complete = torch.cat((pc_trans_list[:c], self.cano[None], pc_trans_list[c:]), dim=0)
-            with torch.no_grad():
-                target_flow, mask = blend_anchor_motion_batched(complete[:-1].detach().contiguous(), self.flow_ref)
-            pred_flow = complete[1:] - complete[:-1]
-            return flow_loss(target_flow, pred_flow, flow_mask_list=mask, robust=self.robust_flow)
-        # frame-sharded: own pairs [p0, p1), sides taken from local frames, the canonical cloud or the halo frame
-        from .dist import flow_pairs_for_rank, halo_from_previous_rank
-        lo, hi = self.frame_range
-        halo = halo_from_previous_rank(pc_trans_list[-1], self.ctx)          # every rank takes part, even with no pairs
-        # the halo's backward is a matched send/recv: tie it into every rank's loss (weight 0) so it always runs,
-        # also on ranks that do not consume their halo (rank 0) or own no pair
-        anchor = halo.sum() * 0.0
-        p0, p1, a_src, b_src = flow_pairs_for_rank(self.total_frames, c, lo, hi)
-        if p1 <= p0:
-            return anchor
-
-        def pick(src):
-            return self.cano if src[0] == "cano" else (halo if src[0] == "halo" else pc_trans_list[src[1]])
-
-        A = torch.stack([pick(x) for x in a_src])
-        Bm = torch.stack([pick(x) for x in b_src])
-        with torch.no_grad():
-            sub = self.flow_ref.slice(p0, p1)
-            target_flow, mask = blend_anchor_motion_batched(A.detach().contiguous(), sub)
-        return flow_loss(target_flow, Bm - A, flow_mask_list=mask, robust=self.robust_flow) + anchor
-
 
 class KinematicEngine(_EngineBase):
-    """Projection model (networks/model.py KinematicModel) + recon loss (+ the optional assignment loss), frame-sharded.
-    axis/moment are shared (all-reduced); theta/distance/root pose are per frame."""
+    """Projection model (networks/model.py KinematicModel) + recon loss (+ the optional assignment and flow losses),
+    frame-sharded.  axis/moment are shared (all-reduced); theta/distance/root pose are per frame."""
 
     def __init__(self, model_kwargs: dict, seg_part: torch.Tensor, cano: torch.Tensor, frames: torch.Tensor,
                  ctx: Optional[DistContext] = None, lr: float = 1e-2, weight_decay: float = 0.0,
                  use_graph: bool = True, native: bool = False, search: str = "auto", betas=(0.9, 0.999), eps: float = 1e-8,
-                 assign: Optional[dict] = None):
+                 assign: Optional[dict] = None, flow_ref=None, cano_idx: int = 0, lambda_flow: float = 1.0,
+                 robust_flow: bool = False):
         """native=True runs the iteration on library kernels -- kin_head -> fused energy -> kin_tail (FK backward, frame
         sums in a fixed order, [all-reduce], the library's Adam) -- with no autograd: the same optimisation as the default
         autograd composition, bit-reproducible.  search: "brute" | "culled" | "auto" as for ``RelaxationEngine`` (native
         iteration only; "culled" is bit-identical to "brute").
         assign: the assignment loss, dict(downsample, assign_gap, lambda_assign, assign_iter, mode="add"|"replace") as for
         ``RelaxationEngine``; the native iteration adds its pose gradients with ``reart_kin_assign``.  The frames' samples are
-        taken once here, so ``step(ingest=...)`` is not available with it."""
+        taken once here, so ``step(ingest=...)`` is not available with it.
+        flow_ref, cano_idx, lambda_flow, robust_flow: the flow loss of run_robot.py:194-213, as for ``RelaxationEngine``; it is
+        added in every phase.  The native iteration adds its pose gradients with ``reart_kin_flow`` on a window of the
+        complete sequence; under frame sharding each rank receives the neighbour ranks' adjacent frames (``dist.flow_window_plan``)."""
         super().__init__(ctx, use_graph)
+        self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
         from .knn_module import KNN
         dev = cano.device
         if frames.shape[0] < self.ctx.world_size:
             raise ValueError(f"{frames.shape[0]} frames cannot be sharded over {self.ctx.world_size} ranks")
         lo, hi = self.ctx.frames(frames.shape[0])
         self.frame_range = (lo, hi)
+        self.total_frames = int(frames.shape[0])
+        if flow_ref is not None and (flow_ref.T != self.total_frames or not 0 <= cano_idx <= self.total_frames):
+            raise ValueError(f"the flow reference needs one set per pair of the complete sequence ({self.total_frames}) and "
+                             f"0 <= cano_idx <= {self.total_frames}")
         self.cano = cano.float().contiguous()
         self.frames = frames[lo:hi].float().contiguous()
         self.frames_packed = ops.pack_cloud(self.frames)
@@ -634,6 +644,8 @@ class KinematicEngine(_EngineBase):
             if refresh:
                 self.assign.refresh(skinned)
             loss = loss + self.assign.loss(skinned)
+        if self.flow_ref is not None:
+            loss = loss + self.lambda_flow * self._flow_term(skinned)
         self.skinned = skinned.detach()
         return loss
 
@@ -684,6 +696,8 @@ class KinematicEngine(_EngineBase):
             b["part_offsets"] = torch.cat((sample_part.new_zeros(1), torch.bincount(sample_part, minlength=P).cumsum(0))).int()
             b["assign_ws_bytes"] = int(L.reart_kin_assign_workspace_bytes(T, P))
             b["assign_ws"] = torch.zeros(b["assign_ws_bytes"], dtype=torch.uint8, device=dev)
+        if self.flow_ref is not None:
+            self._init_native_flow(L, b, N, P)
         self.weight = self.weight.contiguous()
         red = make_small_all_reduce(self.ctx, 6 * E + 1, dev)
         oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
@@ -708,6 +722,77 @@ class KinematicEngine(_EngineBase):
         b["args"] = a
         b["keep"] = (tree, oneshot)
 
+    def _init_native_flow(self, L, b, N, P):
+        """The window of the complete sequence this rank's ``reart_kin_flow`` works on (``dist.flow_window_plan``), its target
+        flows and masks, and the points grouped by part: every buffer once, here."""
+        from .dist import flow_window_plan, shard_bounds
+        dev = self.cano.device
+        W = self.ctx.world_size
+        plan = flow_window_plan(self.total_frames, self.cano_idx, [shard_bounds(self.total_frames, W, r) for r in range(W)])
+        pl = b["flow_plan"] = plan[self.ctx.rank]
+        K = pl["K"]
+        b["win"] = torch.zeros(K, N, 3, dtype=torch.float32, device=dev)
+        b["tflow"] = torch.empty(K - 1, N, 3, dtype=torch.float32, device=dev)
+        b["fmask"] = torch.empty(K - 1, N, dtype=torch.uint8, device=dev)
+        b["slot_frame"] = torch.tensor([x[1] if x[0] == "local" else -1 for x in pl["slots"]], dtype=torch.int32, device=dev)
+        runs = []                                                  # (first slot, first local frame, count) of local runs
+        for s, x in enumerate(pl["slots"]):
+            if x[0] != "local":
+                continue
+            if runs and runs[-1][0] + runs[-1][2] == s:
+                runs[-1][2] += 1
+            else:
+                runs.append([s, x[1], 1])
+        b["win_runs"] = [tuple(r) for r in runs]
+        b["cano_slot"] = next((s for s, x in enumerate(pl["slots"]) if x[0] == "cano"), None)
+        b["flow_ref"] = ref = self.flow_ref.slice(pl["j0"], pl["j0"] + K - 1)
+        # the choice of blend_anchor_motion_batched (both kernels give the same bits)
+        b["flow_sorted"] = ref.sorted_refs is not None and N >= 2048
+        b["query_order"] = torch.empty(K - 1, N, dtype=torch.int32, device=dev) if b["flow_sorted"] else None
+        b["point_order"] = torch.argsort(self.labels, stable=True).int()
+        b["point_offsets"] = torch.cat((self.labels.new_zeros(1), torch.bincount(self.labels, minlength=P).cumsum(0))).int()
+        b["flow_ws_bytes"] = int(L.reart_kin_flow_workspace_bytes(K, P))
+        b["flow_ws"] = torch.zeros(b["flow_ws_bytes"], dtype=torch.uint8, device=dev)
+        if W > 1:
+            self.ctx.barrier()                                     # the communicator exists before the first exchange
+
+    def _native_flow(self, L, b, T, N, P, accumulate):
+        """Window assembly (device copies, [neighbour frames from the adjacent ranks]) -> blend -> reart_kin_flow."""
+        from ._lib import check, ptr, stream_ptr
+        pl, win, sk = b["flow_plan"], b["win"], b["skinned"]
+        for s0, l0, n in b["win_runs"]:
+            win[s0:s0 + n].copy_(sk[l0:l0 + n])
+        if b["cano_slot"] is not None:
+            win[b["cano_slot"]].copy_(self.cano)                  # every step: step(ingest=...) replaces the cloud
+        if self.ctx.world_size > 1:
+            import torch.distributed as dist
+            r = self.ctx.rank
+            p2p = []
+            if pl["send_prev"]:
+                p2p.append(dist.P2POp(dist.isend, sk[0], r - 1))
+            if pl["send_next"]:
+                p2p.append(dist.P2POp(dist.isend, sk[T - 1], r + 1))
+            if pl["recv_prev"] is not None:
+                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_prev"]], r - 1))
+            if pl["recv_next"] is not None:
+                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_next"]], r + 1))
+            if p2p:
+                for req in dist.batch_isend_irecv(p2p):
+                    req.wait()
+        K, ref = pl["K"], b["flow_ref"]
+        if b["flow_sorted"]:
+            buf, soff = ref.sorted_refs
+            check(L.reart_knn3_blend_sorted(ptr(win), ptr(buf), ptr(soff), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N,
+                                            ptr(b["query_order"]), ptr(b["tflow"]), ptr(b["fmask"]), stream_ptr()),
+                  "reart_knn3_blend_sorted")
+        else:
+            check(L.reart_knn3_blend(ptr(win), ptr(ref.ref_cat), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N, ptr(b["tflow"]),
+                                     ptr(b["fmask"]), stream_ptr()), "reart_knn3_blend")
+        check(L.reart_kin_flow(ptr(win), ptr(b["tflow"]), ptr(b["fmask"]), ptr(b["slot_frame"]), ptr(self.cano),
+                               ptr(b["point_order"]), ptr(b["point_offsets"]), self.lambda_flow, int(self.robust_flow), K, N, P,
+                               T, pl["q0"], pl["q1"], ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), int(accumulate),
+                               ptr(b["flow_ws"]), b["flow_ws_bytes"], stream_ptr()), "reart_kin_flow")
+
     def _opt_params(self):
         if not self.native:
             return super()._opt_params()
@@ -723,7 +808,8 @@ class KinematicEngine(_EngineBase):
     def _run_iteration_native(self):
         """kin_head -> [memset, skin (x-sorted copy), (cull bounds,) search, energy columns, energy rows, skin backward,
         reduce] -> kin_tail.  With the assignment loss: kin_head -> energy ("add") or skin ("replace") -> [reart_lap on
-        refresh steps] -> kin_assign -> kin_tail."""
+        refresh steps] -> kin_assign -> kin_tail.  With the flow loss: ... energy or skin -> window copies, [neighbour
+        frames], blend -> kin_flow (overwrites the gradients after skin) -> [lap] -> [kin_assign] -> kin_tail."""
         import ctypes
         from . import _lib
         from ._lib import check, ptr, stream_ptr
@@ -738,13 +824,16 @@ class KinematicEngine(_EngineBase):
             else:                                                 # run_robot.py:164-192: the assignment loss REPLACES Chamfer
                 check(L.reart_skin_fwd(ptr(self.cano), ptr(self.weight), ptr(b["R"]), ptr(b["tr"]), T, N, P, ptr(b["skinned"]),
                                        stream_ptr()), "reart_skin_fwd")
+            flow = self.flow_ref is not None
+            if flow:
+                self._native_flow(L, b, T, N, P, accumulate=use_chamfer)
             if use_assign:
                 if refresh:
                     self.assign.refresh(b["skinned"])
                 s = self.assign
                 check(L.reart_kin_assign(ptr(b["skinned"]), ptr(self.cano), ptr(s.src_idx), ptr(s.pc_tgt), ptr(s.col4row),
                                          ptr(b["sample_order"]), ptr(b["part_offsets"]), s.lambda_assign, T, N, s.num_fps, P,
-                                         ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), 1 if use_chamfer else 0,
+                                         ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), 1 if use_chamfer or flow else 0,
                                          ptr(b["assign_ws"]), b["assign_ws_bytes"], stream_ptr()), "reart_kin_assign")
             a = b["args"]
             if not b["nccl"]:
