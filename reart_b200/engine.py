@@ -12,27 +12,47 @@ Frames are sharded across ranks by ``DistContext``; per-frame parameters stay lo
 """
 from __future__ import annotations
 
+import ctypes
 import math
 from typing import Optional
 
 import torch
 import torch.nn.functional as F
 
-from . import ops
-from .dist import DistContext, GradBucket, make_small_all_reduce
+from . import _lib, ops
+from ._lib import check, ptr, stream_ptr
+from .dist import (DistContext, GradBucket, OneShotAllReduce, flow_pairs_for_rank, flow_window_plan, halo_from_previous_rank,
+                   make_small_all_reduce, shard_bounds)
 from .model import BaseModel, KinematicModel
 
 
 class _EngineBase:
-    def __init__(self, ctx: Optional[DistContext], use_graph: bool):
+    def __init__(self, cano: torch.Tensor, frames: torch.Tensor, ctx: Optional[DistContext], use_graph: bool, flow_ref,
+                 cano_idx: int, lambda_flow: float, robust_flow: bool):
+        """The set-up both engines share: the local shard of the frames, the flow-loss settings, and every attribute this
+        class reads, at its default (each engine sets the ones that apply to it)."""
         self.ctx = ctx or DistContext()
         self.use_graph = use_graph
         self._graphs = {}
         self.iteration = 0
+        if frames.shape[0] < self.ctx.world_size:
+            raise ValueError(f"{frames.shape[0]} frames cannot be sharded over {self.ctx.world_size} ranks: every rank must "
+                             "own at least one frame (an empty shard would skip the step's collectives)")
+        lo, hi = self.ctx.frames(frames.shape[0])
+        self.frame_range = (lo, hi)
+        self.total_frames = int(frames.shape[0])
+        self.cano = cano.float().contiguous()
+        self.frames = frames[lo:hi].float().contiguous()          # local shard of the observed frames
+        self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
+        self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
+        self.tau = torch.ones((), device=self.cano.device)
+        self.native = self.cull = self.search_culled = False
+        self.sink = self.assign = self.optimizer = self.bucket = None
+        self._nat = self._ingest_src = self._cur_variant = None
 
-    # subclasses: _iteration() -> loss tensor (local part), self.optimizer, self.bucket
+    # subclasses: _weights_and_poses() for the autograd iteration, or _run_iteration_native() with native=True
     def _run_iteration(self):
-        src = getattr(self, "_ingest_src", None)
+        src = self._ingest_src
         if src is not None:
             # fresh clouds for this step (a caller streaming data in): device copies + re-pack as part of the iteration,
             # i.e. inside the captured graph -- one launch per step instead of four enqueues in front of it
@@ -40,12 +60,12 @@ class _EngineBase:
             self.cano.copy_(cano_src)
             self.frames.copy_(frames_src)
             ops.pack_cloud(self.frames, out=self.frames_packed)
-            if getattr(self, "search_culled", False):
+            if self.search_culled:
                 torch.gather(self.frames, 1, self._search_gather, out=self.frames_search)
                 ops.pack_cloud(self.frames_search, out=self.frames_search_packed)
-        if getattr(self, "native", False):
+        if self.native:
             return self._run_iteration_native()
-        if getattr(self, "sink", None) is not None:
+        if self.sink is not None:
             return self._run_iteration_sink()
         # set_to_none: AccumulateGrad then adopts the fresh gradient tensors (no zero-fill and no add kernels); inside a
         # captured graph their addresses are stable because they come from the graph's private pool
@@ -76,16 +96,38 @@ class _EngineBase:
         self.optimizer.step()
         return total
 
+    def _iteration(self):
+        """The autograd iteration: the local loss of the skinning weights and poses of ``_weights_and_poses()``."""
+        use_chamfer, use_assign, refresh = self._step_phase()
+        W, R, tr = self._weights_and_poses()
+        if use_chamfer:
+            loss, skinned = ops.skinned_chamfer_loss(self.cano, W, R, tr, self.frames, self.frames_packed, unit_grad=True)
+        else:                                                       # run_robot.py:164-192: assignment only
+            skinned = ops.skin(self.cano, W, R, tr)
+            loss = skinned.new_zeros(())
+        if use_assign:
+            if refresh:
+                self.assign.refresh(skinned)
+            loss = loss + self.assign.loss(skinned)
+        if self.flow_ref is not None:
+            loss = loss + self.lambda_flow * self._flow_term(skinned)
+        self.skinned = skinned.detach()                         # keep the cloud, not the autograd graph
+        return loss
+
     def _opt_params(self):
+        if self.native:
+            return self._nat["params"]
         return [p for g in self.optimizer.param_groups for p in g["params"]]
 
     def _opt_state_tensors(self):
+        if self.native:
+            return self._nat["adam"]
         return [v for st in self.optimizer.state.values() for v in st.values() if torch.is_tensor(v)]
 
     def _aux_state_tensors(self):
         """Other device state an iteration carries from step to step (restored after a capture's warm-up)."""
         aux = [self.assign.col4row, self.assign.dual_u] if self.assign is not None else []
-        if getattr(self, "native", False) and (getattr(self, "cull", False) or self.search_culled):
+        if self.native and (self.cull or self.search_culled):
             aux += [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
         return aux
 
@@ -94,7 +136,6 @@ class _EngineBase:
         """assign: None or dict(downsample, assign_gap, lambda_assign, assign_iter, mode="add"|"replace") -> self.assign
         (an ``AssignLoss`` on the engine's clouds), self.assign_iter, self.assign_mode.  ``sample(n)`` -> (src_idx, tgt_idx):
         the FPS samples when the engine's clouds are not in the caller's order."""
-        self.assign = None
         if assign is None:
             return
         from .assign import AssignLoss
@@ -116,12 +157,9 @@ class _EngineBase:
             return True, False, False
         return self.assign_mode == "add", True, self.assign.due(i, self.assign_iter)
 
-    def _variant(self):
-        """Which flavour of the iteration the NEXT step runs (hashable); one CUDA graph is captured per flavour."""
-        return self._phase()
-
     def _step_phase(self):
-        return getattr(self, "_cur_variant", None) or self._phase()
+        """The phase of the step that is running; ``_phase()`` when the iteration is run outside ``step()``."""
+        return self._cur_variant or self._phase()
 
     def _capture(self, variant):
         """Warm up (allocator, library handles, NCCL communicator, lazily created Adam state), capture one
@@ -177,12 +215,12 @@ class _EngineBase:
         if tau is not None:
             self.tau.fill_(float(tau))
         self.iteration += 1
-        variant = self._variant()
+        variant = self._phase()                                # the flavour of this step: one CUDA graph per flavour
         self._cur_variant = variant                            # fixed for this step (warm-up and capture included)
         self._ingest_src = None
         key = variant
         if ingest is not None:
-            if getattr(self, "cull", False):
+            if self.cull:
                 raise ValueError("ingest is not available with cull=True")
             slot, cano_src, frames_src = ingest
             assert cano_src.shape == self.cano.shape and frames_src.shape == self.frames.shape
@@ -247,7 +285,6 @@ class _EngineBase:
     def _search_energy(self, L, b, W, R, tr, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
         """The fused energy on skinning weights W and poses (R, tr): brute-force search, or the exact culled one in the
         search order seeded by the previous step's arg-mins (bit-identical results).  Writes b["skinned"], b["loss64"]."""
-        from ._lib import check, ptr, stream_ptr
         if self.search_culled:
             check(L.reart_skinned_chamfer_fwd_bwd_ordered(
                 ptr(self.cano), ptr(W), ptr(R), ptr(tr), ptr(self.frames), ptr(self.frames_search),
@@ -263,11 +300,10 @@ class _EngineBase:
 
     def culling_stats(self):
         """(evaluated, offered) (warp, 32-target chunk) pairs since the last call; resets the counters.  Host sync."""
-        b = getattr(self, "_nat", None)
-        if not getattr(self, "native", False) or b is None or "cull_stats" not in b:
+        if not self.native or "cull_stats" not in self._nat:
             return None
-        ev, off = (int(x) for x in b["cull_stats"][:2].tolist())
-        b["cull_stats"][:2].zero_()
+        ev, off = (int(x) for x in self._nat["cull_stats"][:2].tolist())
+        self._nat["cull_stats"][:2].zero_()
         return ev, off
 
     def flagged_ties(self):
@@ -278,6 +314,33 @@ class _EngineBase:
         n = int(self._nat["cull_stats"][2])
         self._nat["cull_stats"][2].zero_()
         return n
+
+    # ------------------------------------------------------------------------------------------ tail of the native iterations
+    def _init_tail(self, a, reducer, n):
+        """Fill the all-reduce fields of the tail's args ``a`` (``RelaxTailArgs`` or ``KinTailArgs``) for ``reducer`` (from
+        ``make_small_all_reduce`` on the ``n`` floats of the bucket).  A one-shot reducer runs inside the tail; without peer
+        memory the tail runs in two phases around an NCCL all-reduce (b["nccl"]).  Returns the one-shot reducer (or None),
+        which the caller keeps alive."""
+        oneshot = reducer if isinstance(reducer, OneShotAllReduce) else None
+        self._nat["nccl"] = reducer is not None and oneshot is None
+        a.rank, a.world = (self.ctx.rank, self.ctx.world_size) if oneshot is not None else (0, 1)
+        if oneshot is not None:
+            assert oneshot.n == n
+            a.peer_base, a.epoch, a.n_pad = ptr(oneshot.peer_base), ptr(oneshot.epoch), oneshot.n_pad
+        a.phase = 0
+        return oneshot
+
+    def _run_tail(self, fn):
+        """The tail ``fn`` (``reart_relax_tail`` or ``reart_kin_tail``) on b["args"]: one launch, or phase 1 -> NCCL -> phase 2."""
+        b = self._nat
+        a = b["args"]
+        if b["nccl"]:                                             # no peer memory: gradients -> bucket, NCCL, Adam
+            a.phase = 1
+            check(fn(ctypes.byref(a), stream_ptr()), fn.__name__)
+            self.ctx.all_reduce_sum_(b["bucket"])
+            a.phase = 2
+        check(fn(ctypes.byref(a), stream_ptr()), fn.__name__)
+        a.phase = 0
 
     # ------------------------------------------------------------------------------------------ flow loss
     def _flow_term(self, pc_trans_list):
@@ -292,7 +355,6 @@ class _EngineBase:
             pred_flow = complete[1:] - complete[:-1]
             return flow_loss(target_flow, pred_flow, flow_mask_list=mask, robust=self.robust_flow)
         # frame-sharded: own pairs [p0, p1), sides taken from local frames, the canonical cloud or the halo frame
-        from .dist import flow_pairs_for_rank, halo_from_previous_rank
         lo, hi = self.frame_range
         halo = halo_from_previous_rank(pc_trans_list[-1], self.ctx)          # every rank takes part, even with no pairs
         # the halo's backward is a matched send/recv: tie it into every rank's loss (weight 0) so it always runs,
@@ -337,33 +399,27 @@ class RelaxationEngine(_EngineBase):
         while everything else stays in the caller's order -- bit-identical to "brute" (native fused iteration only);
         "auto" picks "culled" from ``SEARCH_CULLED_MIN_POINTS`` points per cloud on, where the coarse bounds of cull.cu make
         it faster.  ``cull=True`` (the engine reorders the caller's clouds) and ``fuse_producer=True`` search brute force."""
-        super().__init__(ctx, use_graph)
-        self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
         # the flow loss couples consecutive frames: under frame sharding each rank evaluates the pairs whose second
         # frame it owns and receives ONE skinned frame (the previous rank's last) per iteration (dist.py)
-        dev = cano.device
-        if frames.shape[0] < self.ctx.world_size:
-            raise ValueError(f"{frames.shape[0]} frames cannot be sharded over {self.ctx.world_size} ranks: every rank must "
-                             "own at least one frame (an empty shard would skip the step's collectives)")
-        lo, hi = self.ctx.frames(frames.shape[0])
-        self.frame_range = (lo, hi)
-        self.total_frames = int(frames.shape[0])
-        self.cano = cano.float().contiguous()
-        self.frames = frames[lo:hi].float().contiguous()          # local shard of the observed frames
+        super().__init__(cano, frames, ctx, use_graph, flow_ref, cano_idx, lambda_flow, robust_flow)
+        dev = self.cano.device
+        lo, hi = self.frame_range
         # cull=True: the engine's own clouds are put into k-d leaf order ONCE here (256-point leaves for the canonical
         # cloud = one warp of the search, 32-point leaves for the observed frames = one target chunk); ``perm_cano`` /
         # ``perm_frames`` map engine order -> caller order (engine.skinned[:, k] is caller point perm_cano[k]).  Every
         # order-dependent float sum then associates differently: the same optimisation, not the same bits.  The default
         # (search="auto") culls without this: only the search runs on k-d ordered copies (search_order_rows / _tgt).
-        self.cull = bool(cull) if cull is not None else False
+        self.cull = bool(cull)
         # fuse_producer: skin inside the search kernel's prologue (reart_skinned_chamfer_fwd_bwd_fused; SURVEY N1).  Bit-identical,
         # one launch less, but measured SLOWER than the separate skin kernel on B200 (profiles/r02_fused_producer.md), so opt-in.
         self.fuse_producer = bool(fuse_producer) and not self.cull
         if self.cull and (flow_ref is not None or native is False):
             raise ValueError("exact tile culling runs on the native fused iteration (recon / assignment losses)")
         self.perm_cano = self.perm_frames = None
-        native_path = (flow_ref is None) if native is None else bool(native)
-        self._setup_search(search, native_path and not self.cull and not self.fuse_producer,
+        # recon-only iterations run on the fused head / energy / tail kernels with the library's own Adam (8 launches per
+        # step, no autograd); extra losses on the skinned cloud (flow) keep the autograd composition
+        self.native = (flow_ref is None) if native is None else bool(native)
+        self._setup_search(search, self.native and not self.cull and not self.fuse_producer,
                            "search='culled' runs on the native fused iteration, without cull=True or fuse_producer=True")
         cano_orig, frames_orig = self.cano, self.frames
         if self.cull:
@@ -377,19 +433,15 @@ class RelaxationEngine(_EngineBase):
         torch.manual_seed(seed)                                    # identical init + gumbel draws on every rank
         torch.cuda.manual_seed_all(seed)
         self.model = BaseModel(num_parts=num_parts, pose_len=hi - lo).to(dev)
-        self.tau = torch.ones((), device=dev)
         seg_params = [p for p in self.model.seg_head.parameters() if p.requires_grad]
         self.optimizer = torch.optim.Adam(
             [{"params": [self.model.proposal_6d, self.model.proposal_t], "lr": trans_lr},
              {"params": seg_params, "lr": seg_lr}], lr=1e-3, weight_decay=weight_decay, capturable=use_graph, fused=True)
-        self.bucket = None
         H = self.model.seg_head.model[0].weight.shape[0]
         reducer = make_small_all_reduce(self.ctx, 4 * H + num_parts * H + 1, dev)
         self.sink = ops.GradSink(H, num_parts, dev, extra_scalars=1, reducer=reducer)
         self.model.seg_head.grad_sink = self.sink
-        self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
-        # recon-only iterations run on the fused head / energy / tail kernels with the library's own Adam (8 launches per
-        # step, no autograd); extra losses on the skinned cloud (flow) keep the autograd composition
+
         def sample_in_caller_order(n_fps):
             # sample the clouds in the CALLER's order (FPS starts at the caller's point 0, like the reference's kernel),
             # then express the samples in engine order
@@ -401,7 +453,6 @@ class RelaxationEngine(_EngineBase):
                     torch.gather(inv_f, 1, farthest_point_sample(frames_orig, n_fps)))
 
         self._setup_assign(assign, sample_in_caller_order if self.cull else None)
-        self.native = (flow_ref is None) if native is None else bool(native)
         if self.native:
             if flow_ref is not None:
                 raise ValueError("the native fused iteration covers the recon loss only; pass native=False with a flow loss")
@@ -409,8 +460,6 @@ class RelaxationEngine(_EngineBase):
 
     # ------------------------------------------------------------------------------------------ native fused iteration
     def _init_native(self, trans_lr, seg_lr, weight_decay, betas, eps):
-        import ctypes
-        from . import _lib
         L = _lib.lib()
         dev = self.cano.device
         m = self.model
@@ -441,47 +490,29 @@ class RelaxationEngine(_EngineBase):
         b["bucket"] = torch.zeros(nseg + 1, **f32)
         b["loss_out"] = torch.zeros(1, **f32)
         b["dims"] = (T, N, M, P, H)
+        b["params"] = [m.proposal_6d, m.proposal_t] + [q for q in m.seg_head.parameters() if q.requires_grad]
+        b["adam"] = [b[k] for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr", "step")]
         if self.cull or self.search_culled:
             self._search_buffers(b, T, N, M)
-        red = self.sink.reducer if self.sink is not None else None
         self.model.seg_head.grad_sink = None                     # the autograd sink is not used on this path
-        oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
-        b["nccl"] = red is not None and oneshot is None
         a = _lib.RelaxTailArgs()
-        p = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
-        a.cano, a.w0, a.b0, a.w2 = p(self.cano), p(conv0.weight), p(conv0.bias), p(conv2.weight)
-        a.ysoft, a.tau, a.gW = p(b["ysoft"]), p(self.tau), p(b["gW"])
-        a.d6, a.tr, a.gR, a.gtr = p(m.proposal_6d), p(m.proposal_t), p(b["gR"]), p(b["gtr"])
-        a.m_seg, a.v_seg, a.m_d6, a.v_d6, a.m_tr, a.v_tr = (p(b[k]) for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr"))
-        a.step = p(b["step"])
+        a.cano, a.w0, a.b0, a.w2 = ptr(self.cano), ptr(conv0.weight), ptr(conv0.bias), ptr(conv2.weight)
+        a.ysoft, a.tau, a.gW = ptr(b["ysoft"]), ptr(self.tau), ptr(b["gW"])
+        a.d6, a.tr, a.gR, a.gtr = ptr(m.proposal_6d), ptr(m.proposal_t), ptr(b["gR"]), ptr(b["gtr"])
+        a.m_seg, a.v_seg, a.m_d6, a.v_d6, a.m_tr, a.v_tr = (ptr(b[k]) for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr"))
+        a.step = ptr(b["step"])
         a.lr_pose, a.lr_seg, a.beta1, a.beta2, a.eps, a.weight_decay = trans_lr, seg_lr, betas[0], betas[1], eps, weight_decay
-        a.partials, a.tickets, a.loss_local = p(b["tail_ws"]), p(b["tickets"]), p(b["loss64"])
-        a.bucket, a.loss_out = p(b["bucket"]), p(b["loss_out"])
-        a.rank, a.world = (self.ctx.rank, self.ctx.world_size) if oneshot is not None else (0, 1)
-        if oneshot is not None:
-            assert oneshot.n == nseg + 1
-            a.peer_base, a.epoch, a.n_pad = p(oneshot.peer_base), p(oneshot.epoch), oneshot.n_pad
-        a.phase = 0
+        a.partials, a.tickets, a.loss_local = ptr(b["tail_ws"]), ptr(b["tickets"]), ptr(b["loss64"])
+        a.bucket, a.loss_out = ptr(b["bucket"]), ptr(b["loss_out"])
+        oneshot = self._init_tail(a, self.sink.reducer, nseg + 1)
         a.N, a.H, a.P, a.T = N, H, P, T
         b["args"] = a
         b["keep"] = (conv0, conv2, oneshot)
         assert self.tau.dtype == torch.float32 and conv0.weight.is_contiguous() and conv2.weight.is_contiguous()
 
-    def _opt_params(self):
-        if self.native:
-            m = self.model
-            return [m.proposal_6d, m.proposal_t] + [q for q in m.seg_head.parameters() if q.requires_grad]
-        return super()._opt_params()
-
-    def _opt_state_tensors(self):
-        if self.native:
-            return [self._nat[k] for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr", "step")]
-        return super()._opt_state_tensors()
-
     def _energy_call(self, L, b, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
         """The fused energy evaluation of this step: brute-force or culled search (``_search_energy``), the culled search on
         the engine's own k-d order (cull=True), or the skinning fused into the search (fuse_producer=True)."""
-        from ._lib import check, ptr, stream_ptr
         m = self.model
         if self.cull:
             check(L.reart_skinned_chamfer_fwd_bwd_culled(
@@ -500,9 +531,6 @@ class RelaxationEngine(_EngineBase):
 
     def _run_iteration_native(self):
         """head -> [memset, skin (x-sorted copy), search, energy columns, energy rows, skin backward, reduce] -> tail."""
-        import ctypes
-        from . import _lib
-        from ._lib import check, ptr, stream_ptr
         L = _lib.lib()
         b = self._nat
         T, N, M, P, H = b["dims"]
@@ -534,36 +562,14 @@ class RelaxationEngine(_EngineBase):
                 check(L.reart_skin_bwd(ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(b["gs"]), T, N, P,
                                        ptr(b["gW"]), ptr(b["gR"]), ptr(b["gtr"]), ptr(b["bwd_ws"]), b["bwd_ws_bytes"], stream_ptr()),
                       "reart_skin_bwd")
-            a = b["args"]
-            if not b["nccl"]:
-                check(L.reart_relax_tail(ctypes.byref(a), stream_ptr()), "reart_relax_tail")
-            else:                                                 # no peer memory: gradients -> bucket, NCCL, Adam
-                a.phase = 1
-                check(L.reart_relax_tail(ctypes.byref(a), stream_ptr()), "reart_relax_tail")
-                self.ctx.all_reduce_sum_(b["bucket"])
-                a.phase = 2
-                check(L.reart_relax_tail(ctypes.byref(a), stream_ptr()), "reart_relax_tail")
+            self._run_tail(L.reart_relax_tail)
         self.skinned = b["skinned"]
         return b["loss_out"][0]
 
-    def _iteration(self):
-        use_chamfer, use_assign, refresh = self._step_phase()
-        seg, weight = self.model.weights(self.cano, tau=self.tau)
+    def _weights_and_poses(self):
+        _, weight = self.model.weights(self.cano, tau=self.tau)     # draws the gumbel noise
         R, tr = self.model.pose()
-        if use_chamfer:
-            loss, skinned = ops.skinned_chamfer_loss(self.cano, weight, R, tr, self.frames, self.frames_packed,
-                                                     unit_grad=True)
-        else:
-            skinned = ops.skin(self.cano, weight, R, tr)
-            loss = skinned.new_zeros(())
-        if use_assign:
-            if refresh:
-                self.assign.refresh(skinned)
-            loss = loss + self.assign.loss(skinned)
-        if self.flow_ref is not None:
-            loss = loss + self.lambda_flow * self._flow_term(skinned)
-        self.skinned = skinned.detach()                         # keep the cloud, not the autograd graph
-        return loss
+        return weight, R, tr
 
 
 class KinematicEngine(_EngineBase):
@@ -585,20 +591,13 @@ class KinematicEngine(_EngineBase):
         flow_ref, cano_idx, lambda_flow, robust_flow: the flow loss of run_robot.py:194-213, as for ``RelaxationEngine``; it is
         added in every phase.  The native iteration adds its pose gradients with ``reart_kin_flow`` on a window of the
         complete sequence; under frame sharding each rank receives the neighbour ranks' adjacent frames (``dist.flow_window_plan``)."""
-        super().__init__(ctx, use_graph)
-        self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
+        super().__init__(cano, frames, ctx, use_graph, flow_ref, cano_idx, lambda_flow, robust_flow)
         from .knn_module import KNN
-        dev = cano.device
-        if frames.shape[0] < self.ctx.world_size:
-            raise ValueError(f"{frames.shape[0]} frames cannot be sharded over {self.ctx.world_size} ranks")
-        lo, hi = self.ctx.frames(frames.shape[0])
-        self.frame_range = (lo, hi)
-        self.total_frames = int(frames.shape[0])
+        dev = self.cano.device
+        lo, hi = self.frame_range
         if flow_ref is not None and (flow_ref.T != self.total_frames or not 0 <= cano_idx <= self.total_frames):
             raise ValueError(f"the flow reference needs one set per pair of the complete sequence ({self.total_frames}) and "
                              f"0 <= cano_idx <= {self.total_frames}")
-        self.cano = cano.float().contiguous()
-        self.frames = frames[lo:hi].float().contiguous()
         self.frames_packed = ops.pack_cloud(self.frames)
         self.native = bool(native)
         self._setup_search(search, self.native, "search='culled' runs on the native fused iteration (native=True)")
@@ -608,16 +607,13 @@ class KinematicEngine(_EngineBase):
                 kw[k] = kw[k][lo:hi].clone()
         self.model = KinematicModel(pose_len=hi - lo, seg_part=seg_part, cano_pc=self.cano,
                                     knn=KNN(k=1, transpose_mode=True), **kw).to(dev)
-        self.tau = torch.ones((), device=dev)
         with torch.no_grad():                                       # constant label transfer (SURVEY Q27)
             self.labels = self.model._labels(self.model.cano_pc)
             self.weight = F.one_hot(self.labels, num_classes=self.model.num_parts).float()
-        self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
         if assign is not None and self.cano.shape[0] // int(assign.get("downsample", 4)) < 1:
             raise ValueError(f"downsample leaves no assignment samples of {self.cano.shape[0]} points")
         self._setup_assign(assign)
         if self.native:
-            self.optimizer = self.bucket = None
             self._init_native(lr, weight_decay, betas, eps)
         else:
             params = [p for p in self.model.parameters() if p.requires_grad]
@@ -630,29 +626,12 @@ class KinematicEngine(_EngineBase):
             raise ValueError("ingest is not available with the assignment loss: the frames' samples are taken once at set-up")
         return super().step(tau, ingest)
 
-    def _iteration(self):
-        use_chamfer, use_assign, refresh = self._step_phase()
+    def _weights_and_poses(self):
         trans = self.model.transforms()
-        R, tr = trans[:, :, :3, :3].contiguous(), trans[:, :, :3, 3].contiguous()
-        if use_chamfer:
-            loss, skinned = ops.skinned_chamfer_loss(self.cano, self.weight, R, tr, self.frames, self.frames_packed,
-                                                     unit_grad=True)
-        else:                                                       # run_robot.py:164-192: assignment only
-            skinned = ops.skin(self.cano, self.weight, R, tr)
-            loss = skinned.new_zeros(())
-        if use_assign:
-            if refresh:
-                self.assign.refresh(skinned)
-            loss = loss + self.assign.loss(skinned)
-        if self.flow_ref is not None:
-            loss = loss + self.lambda_flow * self._flow_term(skinned)
-        self.skinned = skinned.detach()
-        return loss
+        return self.weight, trans[:, :, :3, :3].contiguous(), trans[:, :, :3, 3].contiguous()
 
     # ------------------------------------------------------------------------------------------ native fused iteration
     def _init_native(self, lr, weight_decay, betas, eps):
-        from . import _lib
-        from ._lib import ptr
         L = _lib.lib()
         m = self.model
         dev = self.cano.device
@@ -662,7 +641,8 @@ class KinematicEngine(_EngineBase):
         tree = m.tree(dev)
         if P > 32:
             raise ValueError("the native kinematic iteration supports up to 32 parts")
-        params = self._opt_params()
+        names = ["axis_list", "moment_list", "theta_list", "distance_list", "root_6d", "root_t"]
+        params = [getattr(m, n) for n in names if hasattr(m, n)]
         for q in params:                                            # raw pointers below: float32, contiguous, updated in place
             if q.dtype != torch.float32 or not q.is_contiguous():
                 q.data = q.data.float().contiguous()
@@ -671,6 +651,7 @@ class KinematicEngine(_EngineBase):
         f32 = dict(dtype=torch.float32, device=dev)
         b = self._nat = {}
         b["dims"] = (T, N, M, P)
+        b["params"] = params
         b["fk"] = torch.empty(T, P, 12, **f32)
         b["R"], b["tr"] = torch.empty(T, P, 3, 3, **f32), torch.empty(T, P, 3, **f32)
         b["gpose"] = torch.empty(T * P * 12, **f32)
@@ -686,6 +667,7 @@ class KinematicEngine(_EngineBase):
         b["grad"], b["m"], b["v"] = torch.zeros(n_grad, **f32), torch.zeros(n_grad, **f32), torch.zeros(n_grad, **f32)
         b["bucket"] = b["grad"][:6 * E + 1]
         b["step"] = torch.zeros(1, **f32)
+        b["adam"] = [b["m"], b["v"], b["step"]]
         b["loss_out"] = torch.zeros(1, **f32)
         if self.search_culled:
             self._search_buffers(b, T, N, M)
@@ -700,8 +682,6 @@ class KinematicEngine(_EngineBase):
             self._init_native_flow(L, b, N, P)
         self.weight = self.weight.contiguous()
         red = make_small_all_reduce(self.ctx, 6 * E + 1, dev)
-        oneshot = red if (red is not None and hasattr(red, "peer_base")) else None
-        b["nccl"] = red is not None and oneshot is None
         b["head"] = (ptr(m.axis_list), ptr(m.moment_list), ptr(m.theta_list), ptr(distance), ptr(tree.order), ptr(tree.parent),
                      ptr(tree.edge), ptr(tree.joint_type), ptr(m.root_6d) if has_root else None,
                      ptr(m.root_t) if has_root else None, T, P, ptr(b["R"]), ptr(b["tr"]), ptr(b["fk"]))
@@ -713,11 +693,7 @@ class KinematicEngine(_EngineBase):
         a.grad, a.m, a.v, a.step = ptr(b["grad"]), ptr(b["m"]), ptr(b["v"]), ptr(b["step"])
         a.lr, a.beta1, a.beta2, a.eps, a.weight_decay = lr, betas[0], betas[1], eps, weight_decay
         a.partials, a.loss_out = ptr(b["tail_ws"]), ptr(b["loss_out"])
-        a.rank, a.world = (self.ctx.rank, self.ctx.world_size) if oneshot is not None else (0, 1)
-        if oneshot is not None:
-            assert oneshot.n == 6 * E + 1
-            a.peer_base, a.epoch, a.n_pad = ptr(oneshot.peer_base), ptr(oneshot.epoch), oneshot.n_pad
-        a.phase = 0
+        oneshot = self._init_tail(a, red, 6 * E + 1)
         a.T, a.P = T, P
         b["args"] = a
         b["keep"] = (tree, oneshot)
@@ -725,7 +701,6 @@ class KinematicEngine(_EngineBase):
     def _init_native_flow(self, L, b, N, P):
         """The window of the complete sequence this rank's ``reart_kin_flow`` works on (``dist.flow_window_plan``), its target
         flows and masks, and the points grouped by part: every buffer once, here."""
-        from .dist import flow_window_plan, shard_bounds
         dev = self.cano.device
         W = self.ctx.world_size
         plan = flow_window_plan(self.total_frames, self.cano_idx, [shard_bounds(self.total_frames, W, r) for r in range(W)])
@@ -758,7 +733,6 @@ class KinematicEngine(_EngineBase):
 
     def _native_flow(self, L, b, T, N, P, accumulate):
         """Window assembly (device copies, [neighbour frames from the adjacent ranks]) -> blend -> reart_kin_flow."""
-        from ._lib import check, ptr, stream_ptr
         pl, win, sk = b["flow_plan"], b["win"], b["skinned"]
         for s0, l0, n in b["win_runs"]:
             win[s0:s0 + n].copy_(sk[l0:l0 + n])
@@ -793,26 +767,11 @@ class KinematicEngine(_EngineBase):
                                T, pl["q0"], pl["q1"], ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), int(accumulate),
                                ptr(b["flow_ws"]), b["flow_ws_bytes"], stream_ptr()), "reart_kin_flow")
 
-    def _opt_params(self):
-        if not self.native:
-            return super()._opt_params()
-        m = self.model
-        names = ["axis_list", "moment_list", "theta_list", "distance_list", "root_6d", "root_t"]
-        return [getattr(m, n) for n in names if hasattr(m, n)]
-
-    def _opt_state_tensors(self):
-        if self.native:
-            return [self._nat[k] for k in ("m", "v", "step")]
-        return super()._opt_state_tensors()
-
     def _run_iteration_native(self):
         """kin_head -> [memset, skin (x-sorted copy), (cull bounds,) search, energy columns, energy rows, skin backward,
         reduce] -> kin_tail.  With the assignment loss: kin_head -> energy ("add") or skin ("replace") -> [reart_lap on
         refresh steps] -> kin_assign -> kin_tail.  With the flow loss: ... energy or skin -> window copies, [neighbour
         frames], blend -> kin_flow (overwrites the gradients after skin) -> [lap] -> [kin_assign] -> kin_tail."""
-        import ctypes
-        from . import _lib
-        from ._lib import check, ptr, stream_ptr
         L = _lib.lib()
         b = self._nat
         T, N, M, P = b["dims"]
@@ -835,16 +794,7 @@ class KinematicEngine(_EngineBase):
                                          ptr(b["sample_order"]), ptr(b["part_offsets"]), s.lambda_assign, T, N, s.num_fps, P,
                                          ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), 1 if use_chamfer or flow else 0,
                                          ptr(b["assign_ws"]), b["assign_ws_bytes"], stream_ptr()), "reart_kin_assign")
-            a = b["args"]
-            if not b["nccl"]:
-                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
-            else:                                                 # no peer memory: gradients -> bucket, NCCL, Adam
-                a.phase = 1
-                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
-                self.ctx.all_reduce_sum_(b["bucket"])
-                a.phase = 2
-                check(L.reart_kin_tail(ctypes.byref(a), stream_ptr()), "reart_kin_tail")
-                a.phase = 0
+            self._run_tail(L.reart_kin_tail)
         self.skinned = b["skinned"]
         return b["loss_out"][0]
 

@@ -136,7 +136,7 @@ def main():
                     for arm in ARMS:
                         eng = make(arm, c, assign)
                         eng.iteration = 1
-                        eng._cur_variant = eng._variant()
+                        eng._cur_variant = eng._phase()
                         ours, names = kernels_of_one_step(eng)
                         emit({"census": True, "T": T, "N": N, "P": P, "cano_idx": c, "assign": assign is not None, "arm": arm,
                               "our_kernels": ours, "all_kernels": sum(names.values()) if names else None,
