@@ -259,7 +259,8 @@ REART_API int reart_relax_tail(const reart_relax_tail_args* args, void* stream);
  *       grad (written) = [g_axis 3E | g_moment 3E | loss | g_theta T*E | g_distance T*E (with distance) | g_root_6d 6T,
  *       g_root_t 3T (with a root pose)]; m, v: Adam moments in the same layout; step [1] counts completed steps.
  *       phase 0: everything; 1: gradients only (the caller reduces grad[0 .. 6E], e.g. with NCCL); 2: Adam from grad.
- * P <= 32; joint_type values as in reart_fk_fwd.
+ * P <= 32; joint_type values as in reart_fk_fwd.  A one-part model (P = 1) has no joints: axis, moment and theta may be
+ * NULL in both calls, and only the root pose (if any) trains.
  * ------------------------------------------------------------------------------------------- */
 REART_API int reart_kin_head(const float* axis, const float* moment, const float* theta, const float* distance,
                              const int32_t* order, const int32_t* parent, const int32_t* edge, const int32_t* joint_type,

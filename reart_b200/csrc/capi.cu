@@ -501,8 +501,9 @@ int reart_kin_tail(const reart_kin_tail_args* x, void* stream_) {
     REART_ENTRY();
     if (!x || x->T <= 0 || x->P < 1 || !fits_int(x->T * x->P * 12)) return REART_ERR_INVALID_ARG;
     if (x->P > 32) return REART_ERR_UNSUPPORTED;
-    if (!x->fk || !x->gR || !x->gtr || !x->loss_local || !x->order || !x->parent || !x->edge || !x->theta ||
-        (x->P > 1 && (!x->axis || !x->moment)) || (!x->root_6d != !x->root_t) || !x->grad || !x->m || !x->v || !x->step ||
+    // a one-part model has no joints (E = 0): axis, moment and theta may be null there, as in reart_kin_head
+    if (!x->fk || !x->gR || !x->gtr || !x->loss_local || !x->order || !x->parent || !x->edge ||
+        (x->P > 1 && (!x->axis || !x->moment || !x->theta)) || (!x->root_6d != !x->root_t) || !x->grad || !x->m || !x->v || !x->step ||
         !x->partials || !x->loss_out || x->phase < 0 || x->phase > 2 || x->world < 1 || x->rank < 0 || x->rank >= x->world)
         return REART_ERR_INVALID_ARG;
     KinTail a = {};

@@ -71,6 +71,32 @@ def test_kin_entry_points_reject_bad_arguments_without_touching_the_gpu():
     assert L.reart_kin_tail_workspace_bytes(-1, 8) == -1
 
 
+def test_kin_entry_points_take_a_one_part_model_without_joint_arrays():
+    """A one-part model has no joints (E = 0): axis, moment and theta may be null in both the head and the tail, while a
+    model with joints still needs all three.  Without a device, a call that passes the argument check fails at the
+    launch (REART_ERR_LAUNCH) instead of REART_ERR_INVALID_ARG; on a GPU machine the one-part launch itself is
+    test_kinematic_se3_float64_gpu.py's."""
+    import torch
+    from reart_b200 import _lib
+    L = _lib.lib()
+    fake, null = ctypes.c_void_p(0x1000), None
+    for P in (2, 5):
+        for drop in ("axis", "moment", "theta"):
+            a = _tail_args(P=P); setattr(a, drop, None)
+            assert L.reart_kin_tail(ctypes.byref(a), null) == -1, (P, drop)
+            ptrs = {"axis": fake, "moment": fake, "theta": fake}
+            ptrs[drop] = null
+            assert L.reart_kin_head(ptrs["axis"], ptrs["moment"], ptrs["theta"], null, fake, fake, fake, null, null, null,
+                                    4, P, fake, fake, fake, null) == -1, (P, drop)
+    a = _tail_args(P=1); a.root_6d = fake                                    # still both parts of the root pose or neither
+    a.axis = a.moment = a.theta = None
+    assert L.reart_kin_tail(ctypes.byref(a), null) == -1
+    if not torch.cuda.is_available():
+        a = _tail_args(P=1); a.axis = a.moment = a.theta = None
+        assert L.reart_kin_tail(ctypes.byref(a), null) == -3
+        assert L.reart_kin_head(null, null, null, null, fake, fake, fake, null, null, null, 4, 1, fake, fake, fake, null) == -3
+
+
 def test_kin_kernels_carry_no_float_atomics():
     """The SASS of kin_head_kernel / kin_tail_kernel has no float RED/ATOM: the frame sums are fixed-order, so the native
     kinematic step is bit-reproducible (fk_bwd_kernel of the autograd path does use them)."""
