@@ -331,6 +331,32 @@ REART_API int reart_kin_flow(const float* win, const float* tflow, const uint8_t
                              float* gtr, double* loss, int accumulate, void* workspace, int64_t workspace_bytes,
                              void* stream);
 
+/* The flow loss (run_robot.py:194-213, networks/loss.py:10-21) and its gradient w.r.t. the SKINNED cloud, for a model
+ * whose skinning weights train (the relaxation model: reart_skin_bwd takes the gradient on to gW, gR, gtr).  Between the
+ * energy (compute_grad = 0, g_skinned set) or reart_skin_fwd and reart_skin_bwd.  Same window as reart_kin_flow: win [K,N,3]
+ * holds K consecutive frames of the complete sequence (canonical cloud inserted at cano_idx), tflow [K-1,N,3] / mask [K-1,N]
+ * (uint8, as reart_knn3_blend writes them) the blended target flow of pair k = (slot k, slot k+1), slot_frame [K] int32 the
+ * local frame of each slot (-1: the canonical cloud or a neighbour rank's frame).
+ *   pred_k = win[k+1] - win[k],  err_k = pred_k - tflow[k],  per point and component d_k = d flow_loss / d pred_k:
+ *     mask set, plain: 2 err;  mask set, robust: err where |err| < 1, else sign(err) (|err| == 1 takes the linear branch);
+ *     mask clear: 2 * 0.01 * pred   (the per-component rule of reart_kin_flow, the same operations).
+ *   slot s holding local frame t, point i, component r:  g_skinned[t,i,r] (+)= lambda (d_{s-1} - d_s)  (a pair outside the
+ *   window is dropped).
+ *   loss += lambda * sum over the pairs [q0, q1) of the window of the per-point terms, each pair counted by slot k+1 when
+ *   that slot is local, else by slot k, exactly as reart_kin_flow counts it.
+ * A frame's gradient depends only on its own slot and the two adjacent ones: a sub-window that holds a frame's neighbours
+ * gives that frame the bits of the whole-sequence call.  g_skinned [T,N,3] in the caller's point order, loss [1] double:
+ * accumulate != 0 adds to them (one float add per element), else overwrites them (every point of every local frame that
+ * has a slot is written, the loss slot is set).  No float atomics: bit-reproducible.  workspace:
+ * reart_flow_grad_workspace_bytes(K,N), zero before the FIRST call (the kernel re-arms it).  K >= 2, N >= 1,
+ * 0 <= q0 <= q1 <= K-1; T == 0 is an empty problem.
+ * ------------------------------------------------------------------------------------------- */
+REART_API int64_t reart_flow_grad_workspace_bytes(int64_t K, int64_t N);
+REART_API int reart_flow_grad(const float* win, const float* tflow, const uint8_t* mask, const int32_t* slot_frame,
+                              float lambda, int robust, int64_t K, int64_t N, int64_t T, int64_t q0, int64_t q1,
+                              float* g_skinned, double* loss, int accumulate, void* workspace, int64_t workspace_bytes,
+                              void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * 6D rotation representation -> matrix (Gram-Schmidt).
  * Replaces screw_se3/geo_utils.py:632-651 (rotation_6d_to_matrix); d6 [B,6] -> R [B,3,3].

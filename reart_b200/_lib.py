@@ -100,6 +100,8 @@ SIGNATURES.update({
     "reart_kin_assign": (_c_int, [_vp] * 7 + [ctypes.c_float] + [_c_i64] * 4 + [_vp] * 3 + [_c_int, _vp, _c_i64, _vp]),
     "reart_kin_flow_workspace_bytes": (_c_i64, [_c_i64, _c_i64]),
     "reart_kin_flow": (_c_int, [_vp] * 7 + [ctypes.c_float, _c_int] + [_c_i64] * 6 + [_vp] * 3 + [_c_int, _vp, _c_i64, _vp]),
+    "reart_flow_grad_workspace_bytes": (_c_i64, [_c_i64, _c_i64]),
+    "reart_flow_grad": (_c_int, [_vp] * 4 + [ctypes.c_float, _c_int] + [_c_i64] * 5 + [_vp] * 2 + [_c_int, _vp, _c_i64, _vp]),
     "reart_relax_head": (_c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _c_i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "reart_skinned_chamfer_fwd_bwd_fused": (_c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _c_i64, _vp, _vp, _vp,
                                                      _vp, _vp, _vp, _c_int, _vp, _c_i64, _vp]),

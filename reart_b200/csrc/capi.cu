@@ -580,6 +580,32 @@ int reart_kin_flow(const float* win, const float* tflow, const uint8_t* mask, co
     return launch_kin_flow(a, static_cast<cudaStream_t>(stream_));
 }
 
+int64_t reart_flow_grad_workspace_bytes(int64_t K, int64_t N) {
+    if (K < 2 || N < 1 || !fits_int(K * N * 3)) return -1;
+    return align_up(flow_grad_blocks(K, N) * 8) + align_up(4) + kAlign;
+}
+
+int reart_flow_grad(const float* win, const float* tflow, const uint8_t* mask, const int32_t* slot_frame, float lambda,
+                    int robust, int64_t K, int64_t N, int64_t T, int64_t q0, int64_t q1, float* g_skinned, double* loss,
+                    int accumulate, void* workspace, int64_t workspace_bytes, void* stream_) {
+    REART_ENTRY();
+    if (T < 0 || K < 0 || N < 0 || !fits_int(K * N * 3) || !fits_int(T * N * 3)) return REART_ERR_INVALID_ARG;
+    if (T == 0) return REART_OK;
+    if (K < 2 || N == 0 || q0 < 0 || q1 < q0 || q1 > K - 1) return REART_ERR_INVALID_ARG;
+    if (!win || !tflow || !mask || !slot_frame || !g_skinned || !loss) return REART_ERR_INVALID_ARG;
+    Carver ws(workspace, workspace_bytes);
+    double* partials = ws.take<double>(flow_grad_blocks(K, N));
+    unsigned* ticket = ws.take<unsigned>(1);
+    if (!ws.ok) return REART_ERR_WORKSPACE;
+    FlowGrad a = {};
+    a.win = win; a.tflow = tflow; a.mask = mask; a.slot_frame = slot_frame;
+    a.lambda = lambda; a.robust = robust ? 1 : 0;
+    a.g_skinned = g_skinned; a.loss = loss; a.accumulate = accumulate ? 1 : 0;
+    a.partials = partials; a.ticket = ticket;
+    a.K = (int)K; a.N = (int)N; a.T = (int)T; a.q0 = (int)q0; a.q1 = (int)q1;
+    return launch_flow_grad(a, static_cast<cudaStream_t>(stream_));
+}
+
 int reart_rot6d_fwd(const float* d6, int64_t B, float* R, void* stream_) {
     REART_ENTRY();
     if (B < 0) return REART_ERR_INVALID_ARG;

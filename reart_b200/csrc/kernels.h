@@ -278,6 +278,23 @@ struct KinFlow {
 };
 int64_t kin_flow_blocks(int64_t K, int64_t P);
 int launch_kin_flow(const KinFlow& a, cudaStream_t stream);
+// Flow loss and its gradient w.r.t. the skinned cloud, per point, on a window of the complete sequence (flow.cu).
+struct FlowGrad {
+    const float* win;             // [K,N,3] consecutive complete frames
+    const float* tflow;           // [K-1,N,3] blended target flow of pair k = (slot k, slot k+1)
+    const uint8_t* mask;          // [K-1,N]
+    const int32_t* slot_frame;    // [K] local frame of each slot, -1: canonical cloud or a neighbour rank's frame
+    float lambda;
+    int robust;
+    float* g_skinned;             // [T,N,3]
+    double* loss;                 // [1]
+    int accumulate;               // add to g_skinned / loss, else overwrite them
+    double* partials;             // [flow_grad_blocks(K,N)]
+    unsigned* ticket;             // [1] zero before the FIRST call; the kernel re-arms it
+    int K, N, T, q0, q1;          // the loss counts the pairs [q0, q1) of the window
+};
+int64_t flow_grad_blocks(int64_t K, int64_t N);
+int launch_flow_grad(const FlowGrad& a, cudaStream_t stream);
 
 int launch_allreduce_oneshot(const unsigned long long* peer_base, int rank, int world, int64_t n, int64_t n_pad,
                              unsigned* epoch, float* data, cudaStream_t stream);

@@ -11,6 +11,7 @@
 // The work is T*P small dependent steps: the tail is ONE CTA striding over frames.  No float atomics anywhere, so a step
 // is bit-reproducible (fk_bwd_kernel's atomicAdd over frames is what the autograd path does instead).
 #include "common.cuh"
+#include "flow_device.cuh"
 #include "kernels.h"
 #include "se3_device.cuh"
 #include "tail_device.cuh"
@@ -317,30 +318,10 @@ int launch_kin_assign(const KinAssign& a, cudaStream_t stream) {
 // One CTA per (slot, part): thread j takes the part's points j, j+256, ... (point_order groups them by part), then a fixed
 // xor tree per warp and the warps in order.  Pair k's loss is counted (if q0 <= k < q1) by the units of slot k+1 when
 // that slot is local, else of slot k.  The loss: per-CTA partials added in index order by the last CTA (ticket).
+// flow_term_grad (flow_device.cuh) is the per-component rule, shared with flow_grad_kernel (flow.cu).
 constexpr int kKinFlowThreads = 256;
-constexpr float kFlowSmoothWeight = 1e-2f;                   // networks/loss.py:10 smooth_weight
 
 int64_t kin_flow_blocks(int64_t K, int64_t P) { return K * P; }
-
-// d flow_loss / d pred (one component) and the per-component loss term
-__device__ __forceinline__ float flow_term_grad(float pred, float tgt, bool keep, int robust, float& term) {
-    if (!keep) {
-        term = kFlowSmoothWeight * (pred * pred);
-        return 2.0f * kFlowSmoothWeight * pred;
-    }
-    const float e = pred - tgt;
-    if (!robust) {
-        term = e * e;
-        return 2.0f * e;
-    }
-    const float a = fabsf(e);
-    if (a < 1.0f) {                                           // torch.where(a < 1, ...): |err| == 1 is the linear branch
-        term = 0.5f * e * e;
-        return e;
-    }
-    term = a - 0.5f;
-    return e > 0.f ? 1.0f : -1.0f;
-}
 
 __global__ void __launch_bounds__(kKinFlowThreads) kin_flow_kernel(const KinFlow a) {
     constexpr int kWarps = kKinFlowThreads / 32;

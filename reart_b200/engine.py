@@ -6,6 +6,9 @@ seg MLP -> straight-through gumbel weights -> 6D -> R -> fused [skin -> bidirect
 captured once in a CUDA graph (NCCL all-reduce included) and replayed, so neither Python nor the ~4 host syncs
 per iteration of the reference loop (SURVEY Q20) sit on the critical path.
 
+With ``native=True`` the iteration is relax_head -> fused energy -> relax_tail on library kernels, with the assignment
+and flow losses on the skinned cloud in between (``reart_assign_loss_grad``, ``reart_flow_grad``, then ``reart_skin_bwd``).
+
 ``KinematicEngine.step`` is the same for ``--model=kinematic`` (fused tree FK instead of the 6D proposals); its native
 iteration (``native=True``) is kin_head -> fused energy -> kin_tail on library kernels.
 Frames are sharded across ranks by ``DistContext``; per-frame parameters stay local to their rank.
@@ -44,6 +47,9 @@ class _EngineBase:
         self.cano = cano.float().contiguous()
         self.frames = frames[lo:hi].float().contiguous()          # local shard of the observed frames
         self.pairs_per_step_local = 2 * (hi - lo) * self.cano.shape[0] * self.frames.shape[1]
+        if flow_ref is not None and (flow_ref.T != self.total_frames or not 0 <= cano_idx <= self.total_frames):
+            raise ValueError(f"the flow reference needs one set per pair of the complete sequence ({self.total_frames}) and "
+                             f"0 <= cano_idx <= {self.total_frames}")
         self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
         self.tau = torch.ones((), device=self.cano.device)
         self.native = self.cull = self.search_culled = False
@@ -343,6 +349,66 @@ class _EngineBase:
         a.phase = 0
 
     # ------------------------------------------------------------------------------------------ flow loss
+    def _init_flow_window(self, b, N):
+        """The window of the complete sequence this rank's native flow kernel works on (``dist.flow_window_plan``), its target
+        flows and masks: every buffer once, here, in the native buffers ``b``."""
+        dev = self.cano.device
+        W = self.ctx.world_size
+        plan = flow_window_plan(self.total_frames, self.cano_idx, [shard_bounds(self.total_frames, W, r) for r in range(W)])
+        pl = b["flow_plan"] = plan[self.ctx.rank]
+        K = pl["K"]
+        b["win"] = torch.zeros(K, N, 3, dtype=torch.float32, device=dev)
+        b["tflow"] = torch.empty(K - 1, N, 3, dtype=torch.float32, device=dev)
+        b["fmask"] = torch.empty(K - 1, N, dtype=torch.uint8, device=dev)
+        b["slot_frame"] = torch.tensor([x[1] if x[0] == "local" else -1 for x in pl["slots"]], dtype=torch.int32, device=dev)
+        runs = []                                                  # (first slot, first local frame, count) of local runs
+        for s, x in enumerate(pl["slots"]):
+            if x[0] != "local":
+                continue
+            if runs and runs[-1][0] + runs[-1][2] == s:
+                runs[-1][2] += 1
+            else:
+                runs.append([s, x[1], 1])
+        b["win_runs"] = [tuple(r) for r in runs]
+        b["cano_slot"] = next((s for s, x in enumerate(pl["slots"]) if x[0] == "cano"), None)
+        b["flow_ref"] = ref = self.flow_ref.slice(pl["j0"], pl["j0"] + K - 1)
+        # the choice of blend_anchor_motion_batched (both kernels give the same bits)
+        b["flow_sorted"] = ref.sorted_refs is not None and N >= 2048
+        b["query_order"] = torch.empty(K - 1, N, dtype=torch.int32, device=dev) if b["flow_sorted"] else None
+
+    def _flow_window(self, L, b, T, N):
+        """Window assembly (device copies, [neighbour frames from the adjacent ranks]) -> blend: b["win"], b["tflow"],
+        b["fmask"] for this step's b["skinned"]."""
+        pl, win, sk = b["flow_plan"], b["win"], b["skinned"]
+        for s0, l0, n in b["win_runs"]:
+            win[s0:s0 + n].copy_(sk[l0:l0 + n])
+        if b["cano_slot"] is not None:
+            win[b["cano_slot"]].copy_(self.cano)                  # every step: step(ingest=...) replaces the cloud
+        if self.ctx.world_size > 1:
+            import torch.distributed as dist
+            r = self.ctx.rank
+            p2p = []
+            if pl["send_prev"]:
+                p2p.append(dist.P2POp(dist.isend, sk[0], r - 1))
+            if pl["send_next"]:
+                p2p.append(dist.P2POp(dist.isend, sk[T - 1], r + 1))
+            if pl["recv_prev"] is not None:
+                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_prev"]], r - 1))
+            if pl["recv_next"] is not None:
+                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_next"]], r + 1))
+            if p2p:
+                for req in dist.batch_isend_irecv(p2p):
+                    req.wait()
+        K, ref = pl["K"], b["flow_ref"]
+        if b["flow_sorted"]:
+            buf, soff = ref.sorted_refs
+            check(L.reart_knn3_blend_sorted(ptr(win), ptr(buf), ptr(soff), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N,
+                                            ptr(b["query_order"]), ptr(b["tflow"]), ptr(b["fmask"]), stream_ptr()),
+                  "reart_knn3_blend_sorted")
+        else:
+            check(L.reart_knn3_blend(ptr(win), ptr(ref.ref_cat), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N, ptr(b["tflow"]),
+                                     ptr(b["fmask"]), stream_ptr()), "reart_knn3_blend")
+
     def _flow_term(self, pc_trans_list):
         """run_robot.py:194-209: k=3 blended anchor flow (no grad, ONE launch for all pairs) vs predicted flow."""
         from .flow_utils import blend_anchor_motion_batched
@@ -381,7 +447,8 @@ SEARCH_CULLED_MIN_POINTS = 8192
 
 
 class RelaxationEngine(_EngineBase):
-    """Relaxation model (networks/model.py BaseModel) + recon loss, frame-sharded."""
+    """Relaxation model (networks/model.py BaseModel) + recon loss (+ the optional assignment and flow losses),
+    frame-sharded."""
 
     def __init__(self, cano: torch.Tensor, frames: torch.Tensor, num_parts: int, ctx: Optional[DistContext] = None,
                  trans_lr: float = 1e-2, seg_lr: float = 1e-3, weight_decay: float = 0.0, use_graph: bool = True,
@@ -393,8 +460,13 @@ class RelaxationEngine(_EngineBase):
         loss (run_real.py / run_sapien.py) or REPLACES it (run_robot.py's if/else, SURVEY Q12); assignments are refreshed
         on the GPU (``reart_lap``) at ``assign_iter`` and whenever ``i % assign_gap == 0``, inside the captured iteration.
         flow_ref: optional ``flow_utils.FlowReference`` (run_robot.py:78-84) enabling the flow loss of
-        run_robot.py:194-213.  Consecutive frames couple across shard boundaries: under frame sharding each rank
-        receives one skinned frame per iteration from the previous rank (``dist.halo_from_previous_rank``).
+        run_robot.py:194-213 (with cano_idx, lambda_flow, robust_flow).  Consecutive frames couple across shard boundaries.
+        By default (native=None) a flow fit runs the autograd composition: under frame sharding each rank receives one
+        skinned frame per iteration from the previous rank (``dist.halo_from_previous_rank``) and sends its gradient back.
+        native=True runs it on the fused iteration instead, bit-reproducible: ``reart_flow_grad`` writes the gradient w.r.t.
+        the skinned cloud on a window of the complete sequence, ``reart_skin_bwd`` takes it on to the weights and poses;
+        under frame sharding each rank receives the neighbour ranks' adjacent frames (``dist.flow_window_plan``), forward
+        only.  Not with cull=True.
         search: "brute" evaluates every pair; "culled" runs the exact culled search on k-d ordered copies of the clouds
         while everything else stays in the caller's order -- bit-identical to "brute" (native fused iteration only);
         "auto" picks "culled" from ``SEARCH_CULLED_MIN_POINTS`` points per cloud on, where the coarse bounds of cull.cu make
@@ -417,7 +489,7 @@ class RelaxationEngine(_EngineBase):
             raise ValueError("exact tile culling runs on the native fused iteration (recon / assignment losses)")
         self.perm_cano = self.perm_frames = None
         # recon-only iterations run on the fused head / energy / tail kernels with the library's own Adam (8 launches per
-        # step, no autograd); extra losses on the skinned cloud (flow) keep the autograd composition
+        # step, no autograd); with the flow loss the autograd composition stays the default (native=True opts in)
         self.native = (flow_ref is None) if native is None else bool(native)
         self._setup_search(search, self.native and not self.cull and not self.fuse_producer,
                            "search='culled' runs on the native fused iteration, without cull=True or fuse_producer=True")
@@ -454,8 +526,6 @@ class RelaxationEngine(_EngineBase):
 
         self._setup_assign(assign, sample_in_caller_order if self.cull else None)
         if self.native:
-            if flow_ref is not None:
-                raise ValueError("the native fused iteration covers the recon loss only; pass native=False with a flow loss")
             self._init_native(trans_lr, seg_lr, weight_decay, betas, eps)
 
     # ------------------------------------------------------------------------------------------ native fused iteration
@@ -494,6 +564,16 @@ class RelaxationEngine(_EngineBase):
         b["adam"] = [b[k] for k in ("m_seg", "v_seg", "m_d6", "v_d6", "m_tr", "v_tr", "step")]
         if self.cull or self.search_culled:
             self._search_buffers(b, T, N, M)
+        if self.flow_ref is not None:
+            # the flow loss takes the route of the assignment loss: d loss / d skinned in b["gs"], then reart_skin_bwd
+            b["gs"] = torch.zeros(T, N, 3, **f32)
+            b["bwd_ws_bytes"] = int(L.reart_skin_bwd_workspace_bytes(T, N, P))
+            b["bwd_ws"] = _lib.workspace(b["bwd_ws_bytes"], dev)
+            self._init_flow_window(b, N)
+            b["flow_ws_bytes"] = int(L.reart_flow_grad_workspace_bytes(b["flow_plan"]["K"], N))
+            b["flow_ws"] = torch.zeros(b["flow_ws_bytes"], dtype=torch.uint8, device=dev)
+            if self.ctx.world_size > 1:
+                self.ctx.barrier()                                 # the communicator exists before the first exchange
         self.model.seg_head.grad_sink = None                     # the autograd sink is not used on this path
         a = _lib.RelaxTailArgs()
         a.cano, a.w0, a.b0, a.w2 = ptr(self.cano), ptr(conv0.weight), ptr(conv0.bias), ptr(conv2.weight)
@@ -530,19 +610,23 @@ class RelaxationEngine(_EngineBase):
                 b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_fused")
 
     def _run_iteration_native(self):
-        """head -> [memset, skin (x-sorted copy), search, energy columns, energy rows, skin backward, reduce] -> tail."""
+        """head -> [memset, skin (x-sorted copy), search, energy columns, energy rows, skin backward, reduce] -> tail.
+        With the assignment or the flow loss the gradient goes through the skinned cloud: head -> energy (compute_grad = 0,
+        d loss / d skinned into b["gs"]) or skin ("replace" phases) -> [window copies, [neighbour frames], blend -> flow_grad
+        (overwrites b["gs"] and the loss after skin)] -> [reart_lap on refresh steps] -> [assignment] -> skin_bwd -> tail."""
         L = _lib.lib()
         b = self._nat
         T, N, M, P, H = b["dims"]
         m = self.model
         conv0, conv2 = m.seg_head.model[0], m.seg_head.model[2]
         use_chamfer, use_assign, refresh = self._step_phase()
+        flow = self.flow_ref is not None
         b["expo"].exponential_()                                  # the same RNG draw F.gumbel_softmax makes
         with torch.cuda.device(self.cano.device):
             check(L.reart_relax_head(ptr(self.cano), ptr(conv0.weight), ptr(conv0.bias), ptr(conv2.weight), ptr(b["expo"]),
                                      ptr(self.perm_cano), ptr(self.tau), ptr(m.proposal_6d), N, H, P, T, None, ptr(b["W"]), ptr(b["ysoft"]),
                                      ptr(b["R"]), ptr(b["hot"]), stream_ptr()), "reart_relax_head")
-            if not use_assign:
+            if not use_assign and not flow:
                 self._energy_call(L, b, T, N, M, P, b["gW"], b["gR"], b["gtr"], None, 1)
             else:
                 if "gs" not in b:
@@ -554,11 +638,19 @@ class RelaxationEngine(_EngineBase):
                 else:                                             # run_robot.py:164-192: the assignment loss REPLACES Chamfer
                     check(L.reart_skin_fwd(ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), T, N, P, ptr(b["skinned"]),
                                            stream_ptr()), "reart_skin_fwd")
-                    b["gs"].zero_()
-                    b["loss64"].zero_()
-                if refresh:
-                    self.assign.refresh(b["skinned"])
-                self.assign.add_loss_and_grad(b["skinned"], b["gs"], b["loss64"], accumulate=True)
+                    if not flow:
+                        b["gs"].zero_()
+                        b["loss64"].zero_()
+                if flow:
+                    self._flow_window(L, b, T, N)
+                    pl = b["flow_plan"]
+                    check(L.reart_flow_grad(ptr(b["win"]), ptr(b["tflow"]), ptr(b["fmask"]), ptr(b["slot_frame"]), self.lambda_flow,
+                                            int(self.robust_flow), pl["K"], N, T, pl["q0"], pl["q1"], ptr(b["gs"]), ptr(b["loss64"]),
+                                            int(use_chamfer), ptr(b["flow_ws"]), b["flow_ws_bytes"], stream_ptr()), "reart_flow_grad")
+                if use_assign:
+                    if refresh:
+                        self.assign.refresh(b["skinned"])
+                    self.assign.add_loss_and_grad(b["skinned"], b["gs"], b["loss64"], accumulate=True)
                 check(L.reart_skin_bwd(ptr(self.cano), ptr(b["W"]), ptr(b["R"]), ptr(m.proposal_t), ptr(b["gs"]), T, N, P,
                                        ptr(b["gW"]), ptr(b["gR"]), ptr(b["gtr"]), ptr(b["bwd_ws"]), b["bwd_ws_bytes"], stream_ptr()),
                       "reart_skin_bwd")
@@ -595,9 +687,6 @@ class KinematicEngine(_EngineBase):
         from .knn_module import KNN
         dev = self.cano.device
         lo, hi = self.frame_range
-        if flow_ref is not None and (flow_ref.T != self.total_frames or not 0 <= cano_idx <= self.total_frames):
-            raise ValueError(f"the flow reference needs one set per pair of the complete sequence ({self.total_frames}) and "
-                             f"0 <= cano_idx <= {self.total_frames}")
         self.frames_packed = ops.pack_cloud(self.frames)
         self.native = bool(native)
         self._setup_search(search, self.native, "search='culled' runs on the native fused iteration (native=True)")
@@ -699,72 +788,23 @@ class KinematicEngine(_EngineBase):
         b["keep"] = (tree, oneshot)
 
     def _init_native_flow(self, L, b, N, P):
-        """The window of the complete sequence this rank's ``reart_kin_flow`` works on (``dist.flow_window_plan``), its target
-        flows and masks, and the points grouped by part: every buffer once, here."""
-        dev = self.cano.device
-        W = self.ctx.world_size
-        plan = flow_window_plan(self.total_frames, self.cano_idx, [shard_bounds(self.total_frames, W, r) for r in range(W)])
-        pl = b["flow_plan"] = plan[self.ctx.rank]
-        K = pl["K"]
-        b["win"] = torch.zeros(K, N, 3, dtype=torch.float32, device=dev)
-        b["tflow"] = torch.empty(K - 1, N, 3, dtype=torch.float32, device=dev)
-        b["fmask"] = torch.empty(K - 1, N, dtype=torch.uint8, device=dev)
-        b["slot_frame"] = torch.tensor([x[1] if x[0] == "local" else -1 for x in pl["slots"]], dtype=torch.int32, device=dev)
-        runs = []                                                  # (first slot, first local frame, count) of local runs
-        for s, x in enumerate(pl["slots"]):
-            if x[0] != "local":
-                continue
-            if runs and runs[-1][0] + runs[-1][2] == s:
-                runs[-1][2] += 1
-            else:
-                runs.append([s, x[1], 1])
-        b["win_runs"] = [tuple(r) for r in runs]
-        b["cano_slot"] = next((s for s, x in enumerate(pl["slots"]) if x[0] == "cano"), None)
-        b["flow_ref"] = ref = self.flow_ref.slice(pl["j0"], pl["j0"] + K - 1)
-        # the choice of blend_anchor_motion_batched (both kernels give the same bits)
-        b["flow_sorted"] = ref.sorted_refs is not None and N >= 2048
-        b["query_order"] = torch.empty(K - 1, N, dtype=torch.int32, device=dev) if b["flow_sorted"] else None
+        """The flow window (``_init_flow_window``), the points grouped by part and ``reart_kin_flow``'s workspace: every buffer
+        once, here."""
+        self._init_flow_window(b, N)
         b["point_order"] = torch.argsort(self.labels, stable=True).int()
         b["point_offsets"] = torch.cat((self.labels.new_zeros(1), torch.bincount(self.labels, minlength=P).cumsum(0))).int()
-        b["flow_ws_bytes"] = int(L.reart_kin_flow_workspace_bytes(K, P))
-        b["flow_ws"] = torch.zeros(b["flow_ws_bytes"], dtype=torch.uint8, device=dev)
-        if W > 1:
+        b["flow_ws_bytes"] = int(L.reart_kin_flow_workspace_bytes(b["flow_plan"]["K"], P))
+        b["flow_ws"] = torch.zeros(b["flow_ws_bytes"], dtype=torch.uint8, device=self.cano.device)
+        if self.ctx.world_size > 1:
             self.ctx.barrier()                                     # the communicator exists before the first exchange
 
     def _native_flow(self, L, b, T, N, P, accumulate):
-        """Window assembly (device copies, [neighbour frames from the adjacent ranks]) -> blend -> reart_kin_flow."""
-        pl, win, sk = b["flow_plan"], b["win"], b["skinned"]
-        for s0, l0, n in b["win_runs"]:
-            win[s0:s0 + n].copy_(sk[l0:l0 + n])
-        if b["cano_slot"] is not None:
-            win[b["cano_slot"]].copy_(self.cano)                  # every step: step(ingest=...) replaces the cloud
-        if self.ctx.world_size > 1:
-            import torch.distributed as dist
-            r = self.ctx.rank
-            p2p = []
-            if pl["send_prev"]:
-                p2p.append(dist.P2POp(dist.isend, sk[0], r - 1))
-            if pl["send_next"]:
-                p2p.append(dist.P2POp(dist.isend, sk[T - 1], r + 1))
-            if pl["recv_prev"] is not None:
-                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_prev"]], r - 1))
-            if pl["recv_next"] is not None:
-                p2p.append(dist.P2POp(dist.irecv, win[pl["recv_next"]], r + 1))
-            if p2p:
-                for req in dist.batch_isend_irecv(p2p):
-                    req.wait()
-        K, ref = pl["K"], b["flow_ref"]
-        if b["flow_sorted"]:
-            buf, soff = ref.sorted_refs
-            check(L.reart_knn3_blend_sorted(ptr(win), ptr(buf), ptr(soff), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N,
-                                            ptr(b["query_order"]), ptr(b["tflow"]), ptr(b["fmask"]), stream_ptr()),
-                  "reart_knn3_blend_sorted")
-        else:
-            check(L.reart_knn3_blend(ptr(win), ptr(ref.ref_cat), ptr(ref.flow_cat), ptr(ref.offsets), K - 1, N, ptr(b["tflow"]),
-                                     ptr(b["fmask"]), stream_ptr()), "reart_knn3_blend")
-        check(L.reart_kin_flow(ptr(win), ptr(b["tflow"]), ptr(b["fmask"]), ptr(b["slot_frame"]), ptr(self.cano),
-                               ptr(b["point_order"]), ptr(b["point_offsets"]), self.lambda_flow, int(self.robust_flow), K, N, P,
-                               T, pl["q0"], pl["q1"], ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), int(accumulate),
+        """Window assembly and blend (``_flow_window``) -> reart_kin_flow."""
+        self._flow_window(L, b, T, N)
+        pl = b["flow_plan"]
+        check(L.reart_kin_flow(ptr(b["win"]), ptr(b["tflow"]), ptr(b["fmask"]), ptr(b["slot_frame"]), ptr(self.cano),
+                               ptr(b["point_order"]), ptr(b["point_offsets"]), self.lambda_flow, int(self.robust_flow), pl["K"], N,
+                               P, T, pl["q0"], pl["q1"], ptr(b["gR"]), ptr(b["gtr"]), ptr(b["loss64"]), int(accumulate),
                                ptr(b["flow_ws"]), b["flow_ws_bytes"], stream_ptr()), "reart_kin_flow")
 
     def _run_iteration_native(self):
