@@ -155,8 +155,10 @@ REART_API int reart_skinned_chamfer_fwd_bwd_culled(const float* cano, const floa
  * search marks every point whose minimum is reached in two of its chunks, and those take the lowest caller index among
  * all points at exactly that distance -- the brute force's answer.  Points ordered by caller index inside every 256-row
  * block and 32-target chunk of the search order are required for the others: a chunk's first match is then its lowest
- * caller index.  nn_rows [T,N] / nn_cols [T,M] (device, int32, SEARCH order and search indices) are the culling seeds as in
- * reart_skinned_chamfer_fwd_bwd_culled (-1 / any value: still exact) and are overwritten with this evaluation's arg-mins.
+ * caller index.  nn_rows [T,N] / nn_cols [T,M] (device, int32, by CALLER index: nn_rows[t][i] the arg-min caller target
+ * of caller row i, nn_cols[t][j] the arg-min caller row of caller target j) are the culling seeds as in
+ * reart_skinned_chamfer_fwd_bwd_culled (-1 / any value: still exact) and are overwritten with this evaluation's arg-mins;
+ * they do not depend on the search order, so they carry over when the order changes.
  * stats (optional, device, [3] uint64, caller-zeroed): += (warp, chunk) pairs evaluated, offered, points resolved by the
  * tie path. */
 REART_API int reart_skinned_chamfer_fwd_bwd_ordered(const float* cano, const float* W, const float* R, const float* tr,
@@ -167,6 +169,23 @@ REART_API int reart_skinned_chamfer_fwd_bwd_ordered(const float* cano, const flo
                                                     float* g_skinned, int compute_grad, float* d_fwd, int64_t* i_fwd,
                                                     float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
                                                     uint64_t* stats, void* workspace, int64_t workspace_bytes, void* stream);
+/* reart_skinned_chamfer_fwd_bwd_ordered with a row order the call computes itself, per frame, on the skinned cloud
+ * (csrc/order.cu): a sort-tile-recursive order -- the frame's axes by decreasing extent; rows sorted by (coordinate, caller
+ * index) along the first into slabs of 2048, each slab along the second into pieces of 512, each piece along the third into
+ * leaves of 256 (the last leaf of a frame may be short); every leaf then in ascending caller index.  Once the parts of a fit
+ * move apart, the skinned rows of one canonical neighbourhood land in many places of a frame, and blocks grouped on the
+ * posed cloud stay compact where a fixed order does not.  row_order / row_inv [T,N] (device, int32) are written: search
+ * position -> caller row and its inverse.  Every other argument and result as in reart_skinned_chamfer_fwd_bwd_ordered;
+ * bit-identical to reart_skinned_chamfer_fwd_bwd_ex.  N <= reart_posed_order_max_points() (else REART_ERR_UNSUPPORTED). */
+REART_API int reart_skinned_chamfer_fwd_bwd_posed(const float* cano, const float* W, const float* R, const float* tr,
+                                                  const float* tgt, const float* tgt_search, const float* tgt_search_packed,
+                                                  int64_t T, int64_t N, int64_t M, int64_t P, const int32_t* tgt_order,
+                                                  const int32_t* tgt_inv, int32_t* row_order, int32_t* row_inv,
+                                                  float* skinned, double* loss, float* gW, float* gR, float* gtr,
+                                                  float* g_skinned, int compute_grad, float* d_fwd, int64_t* i_fwd,
+                                                  float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
+                                                  uint64_t* stats, void* workspace, int64_t workspace_bytes, void* stream);
+REART_API int64_t reart_posed_order_max_points(void);
 /* The same energy with the skinning FUSED INTO THE PRODUCER SIDE OF THE SEARCH (the composition networks/model.py:63-69 ->
  * utils/chamfer.py:78-94 in one kernel): every search CTA skins its own 2048 canonical points in its prologue and the
  * skinned cloud / x-sorted copy are emitted as by-products, so there is no skinning launch and the cloud is not re-read.

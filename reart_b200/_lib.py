@@ -45,6 +45,9 @@ SIGNATURES = {
                                                       _vp]),
     "reart_skinned_chamfer_fwd_bwd_ordered": (_c_int, [_vp] * 7 + [_c_i64] * 4 + [_vp] * 10 + [_c_int] + [_vp] * 8 +
                                               [_c_i64, _vp]),
+    "reart_skinned_chamfer_fwd_bwd_posed": (_c_int, [_vp] * 7 + [_c_i64] * 4 + [_vp] * 10 + [_c_int] + [_vp] * 8 +
+                                            [_c_i64, _vp]),
+    "reart_posed_order_max_points": (_c_i64, []),
     "reart_segmlp_fwd": (_c_int, [_vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _vp, _vp]),
     "reart_segmlp_bwd": (_c_int, [_vp, _vp, _vp, _vp, _vp, _c_i64, _c_i64, _c_i64, _vp, _vp, _vp, _vp]),
     "reart_gumbel_st_fwd": (_c_int, [_vp, _vp, _vp, _c_i64, _c_i64, _vp, _vp, _vp]),

@@ -251,10 +251,12 @@ int reart_skinned_chamfer_fwd_bwd_ex(const float* cano, const float* W, const fl
                                                 workspace_bytes, stream_);
 }
 
-// The search order of reart_skinned_chamfer_fwd_bwd_ordered (null everywhere else).
+// The search order of reart_skinned_chamfer_fwd_bwd_ordered / _posed (null everywhere else).
 struct SearchOrder {
-    const int32_t* row_order; const int32_t* row_inv; const int32_t* tgt_order; const int32_t* tgt_inv;
+    int32_t* row_order; int32_t* row_inv;      // [N] given (ordered), or [T,N] written by the pipeline (posed)
+    const int32_t* tgt_order; const int32_t* tgt_inv;
     const float* tgt_search;      // [T,M,3] the observed frames in tgt_order (tgt_packed is then its packed copy)
+    bool posed;                   // rows: a per-frame STR order of the skinned cloud, computed every call (order.cu)
 };
 
 static int energy_pipeline(const float* cano, const float* W, const float* hot, const float* R, const float* tr,
@@ -286,7 +288,27 @@ int reart_skinned_chamfer_fwd_bwd_ordered(const float* cano, const float* W, con
                                           int64_t workspace_bytes, void* stream_) {
     REART_ENTRY();
     if (!tgt_search || !row_order || !row_inv || !tgt_order || !tgt_inv || !nn_rows || !nn_cols) return REART_ERR_INVALID_ARG;
-    const SearchOrder order = {row_order, row_inv, tgt_order, tgt_inv, tgt_search};
+    // the shared row order is only read (SearchOrder holds the posed entry's outputs too)
+    const SearchOrder order = {const_cast<int32_t*>(row_order), const_cast<int32_t*>(row_inv), tgt_order, tgt_inv, tgt_search,
+                               false};
+    return energy_pipeline(cano, W, nullptr, R, tr, tgt, tgt_search_packed, T, N, M, P, skinned, loss, gW, gR, gtr, g_skinned,
+                           compute_grad, d_fwd, i_fwd, d_bwd, i_bwd, nn_rows, nn_cols, stats, workspace, workspace_bytes,
+                           stream_, &order);
+}
+
+int64_t reart_posed_order_max_points(void) { return posed_order_max_points(); }
+
+int reart_skinned_chamfer_fwd_bwd_posed(const float* cano, const float* W, const float* R, const float* tr,
+                                        const float* tgt, const float* tgt_search, const float* tgt_search_packed, int64_t T,
+                                        int64_t N, int64_t M, int64_t P, const int32_t* tgt_order, const int32_t* tgt_inv,
+                                        int32_t* row_order, int32_t* row_inv, float* skinned, double* loss, float* gW,
+                                        float* gR, float* gtr, float* g_skinned, int compute_grad, float* d_fwd,
+                                        int64_t* i_fwd, float* d_bwd, int64_t* i_bwd, int32_t* nn_rows, int32_t* nn_cols,
+                                        uint64_t* stats, void* workspace, int64_t workspace_bytes, void* stream_) {
+    REART_ENTRY();
+    if (!tgt_search || !row_order || !row_inv || !tgt_order || !tgt_inv || !nn_rows || !nn_cols) return REART_ERR_INVALID_ARG;
+    if (N > posed_order_max_points()) return REART_ERR_UNSUPPORTED;
+    const SearchOrder order = {row_order, row_inv, tgt_order, tgt_inv, tgt_search, true};
     return energy_pipeline(cano, W, nullptr, R, tr, tgt, tgt_search_packed, T, N, M, P, skinned, loss, gW, gR, gtr, g_skinned,
                            compute_grad, d_fwd, i_fwd, d_bwd, i_bwd, nn_rows, nn_cols, stats, workspace, workspace_bytes,
                            stream_, &order);
@@ -353,6 +375,13 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
         if (cull) return REART_ERR_INVALID_ARG;
         sp.sk_cano = cano; sp.sk_hot = hot; sp.sk_R = R; sp.sk_tr = tr; sp.sk_P = (int)P; sp.sk_npad = (int)n_pad_sorted;
         sp.sk_out = skinned; sp.sk_sorted = psrc; sp.sk_perm = perm; sp.sk_xq = xq;
+    } else if (order && order->posed) {
+        // skin in caller order, then order the skinned rows per frame and write the search's copies in that order
+        rc = launch_skin_fwd(cano, W, R, tr, T, N, P, skinned, nullptr, stream);
+        if (rc) return rc;
+        rc = launch_posed_order(skinned, T, N, n_pad_sorted, order->row_order, order->row_inv, skinned_search, psrc, perm, xq,
+                                stream);
+        if (rc) return rc;
     } else {
         rc = launch_skin_fwd_sorted(cano, W, R, tr, T, N, P, skinned, psrc, perm, xq, n_pad_sorted, stream,
                                     order ? order->row_order : nullptr, skinned_search);
@@ -366,6 +395,10 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
         // seeds = the arg-mins of the previous evaluation (nn_* = -1: none, brute force); bounds, then the culled search
         CullParams cp = {};
         cp.a = sp.a; cp.b = order ? order->tgt_search : tgt; cp.nn_rows = nn_rows; cp.nn_cols = nn_cols;
+        if (order) {
+            cp.row_order = order->row_order; cp.row_inv = order->row_inv; cp.tgt_order = order->tgt_order;
+            cp.tgt_inv = order->tgt_inv; cp.row_stride = order->posed ? N : 0;
+        }
         cp.B = (int)T; cp.na = (int)N; cp.nb = (int)M; cp.nb_pad = (int)padded_points(M);
         cp.colbox = colbox; cp.rowbound = rowbound;
         cp.coarse = (N >= 8192 && M >= 8192 && N <= 800000 && M <= 800000) ? 1 : 0;   // small clouds: the pass costs more than it saves
@@ -382,10 +415,11 @@ static int energy_pipeline(const float* cano, const float* W, const float* hot, 
     ep.row_chunk_pts = kChunk; ep.col_chunk_pts = sp.col_chunk_pts; ep.gscale = 1.0f; ep.g_src = gs; ep.loss = loss;
     if (sp.col_chunk_pts != 256) return REART_ERR_UNSUPPORTED;       // the sorted copy is built per 256-point chunk
     ep.d_fwd = d_fwd; ep.i_fwd = i_fwd; ep.d_bwd = d_bwd; ep.i_bwd = i_bwd;
-    ep.nn_rows = nn_rows; ep.nn_cols = nn_cols;                      // the next evaluation's seeds
+    ep.nn_rows = nn_rows; ep.nn_cols = nn_cols;                      // the next evaluation's seeds, by caller index
     ep.src_perm = perm; ep.src_xq = xq; ep.acc = acc; ep.col_bound = col_bound; ep.partials = partials; ep.ticket = ticket;
     if (order) {
         ep.row_order = order->row_order; ep.row_inv = order->row_inv; ep.tgt_order = order->tgt_order; ep.tgt_inv = order->tgt_inv;
+        ep.row_stride = order->posed ? N : 0;
         ep.tie_a = sp.tie_a; ep.tie_b = sp.tie_b;
         ep.ties = cull_stats ? reinterpret_cast<unsigned long long*>(cull_stats) + 2 : nullptr;
     }

@@ -13,8 +13,9 @@
 // pair distance in it -- is STRICTLY above both bounds: such a pair can hold neither a minimum nor a tie.  Without seeds
 // (nn = -1) and below 8192 points the bounds are infinite and the search is the brute force.  The distances here use the
 // very arithmetic of the search (sqdist_scalar), so the bounds bound the COMPUTED minima and the culled keys are
-// bit-identical.  How much is skipped depends on how compact the chunks are: callers that control the point order
-// (engine.py) sort both clouds into a k-d order once; any order is correct.
+// bit-identical.  How much is skipped depends on how compact the chunks are: the ordered entries of capi.cu run the search
+// on copies in a compact order (fixed, or per frame on the posed cloud), and the seeds, kept by caller index, are
+// translated through it here; any order is correct.
 #include "common.cuh"
 #include "kernels.h"
 #include <algorithm>
@@ -114,15 +115,18 @@ __global__ void __launch_bounds__(kCullRowChunk) cull_row_bounds_kernel(const Cu
             if (!(ub >= 0.f)) ub = INFINITY;                   // NaN input: no culling
         }
         if (p.nn_rows) {
+            // seeds are kept by caller index: the neighbours' caller rows, their seeds translated into the search order
             int jprev = -2;
 #pragma unroll
             for (int d = -kCullSeeds; d <= kCullSeeds; ++d) {
                 const int in = min(max(i + d, 0), p.na - 1);
-                const int j = p.nn_rows[(int64_t)b * p.na + in];
+                const int cr = p.row_order ? p.row_order[(int64_t)b * p.row_stride + in] : in;
+                const int j = p.nn_rows[(int64_t)b * p.na + cr];
                 if (j == jprev) continue;                      // neighbours very often share a seed
                 jprev = j;
                 if (j >= 0 && j < p.nb) {
-                    const float* t = p.b + ((int64_t)b * p.nb + j) * 3;
+                    const int js = p.tgt_inv ? p.tgt_inv[(int64_t)b * p.nb + j] : j;
+                    const float* t = p.b + ((int64_t)b * p.nb + js) * 3;
                     const float c = sqdist_scalar(ax, ay, az, t[0], t[1], t[2]);
                     if (c < ub) ub = c;                        // NaN never passes: no culling on NaN input
                 }
@@ -171,8 +175,10 @@ __global__ void __launch_bounds__(256) cull_col_boxes_kernel(const CullParams p,
 #pragma unroll
             for (int d = -kCullSeeds; d <= kCullSeeds; ++d) {
                 const int jn = min(max(j + d, 0), p.nb - 1);
-                const int i0 = p.nn_cols[(int64_t)b * p.nb + jn];
-                if (i0 < 0 || i0 >= p.na) continue;
+                const int cj = p.tgt_order ? p.tgt_order[(int64_t)b * p.nb + jn] : jn;
+                const int ic = p.nn_cols[(int64_t)b * p.nb + cj];
+                if (ic < 0 || ic >= p.na) continue;
+                const int i0 = p.row_inv ? p.row_inv[(int64_t)b * p.row_stride + ic] : ic;
 #pragma unroll
                 for (int e = -1; e <= 1; ++e) {
                     if (d != 0 && e != 0) continue;            // row neighbours only around the target's own seed

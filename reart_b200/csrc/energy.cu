@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(kEnergyThreads) energy_cols_kernel(const Energ
                                           p.src_xq + b * (int64_t)(p.n_pad / kSortedChunk) * kQuantiles,
                                           (unsigned)(key & 0xffffffffu), ax, ay, az, dmin);
                 if (i >= p.N) i = 0;
-                if (ORDERED) i = p.row_order[i];
+                if (ORDERED) i = p.row_order[b * p.row_stride + i];
             }
         }
         if (ORDERED) resolve_flagged(flagged, p.src, p.N, ax, ay, az, dmin, b, i, p.ties);
@@ -121,7 +121,7 @@ __global__ void __launch_bounds__(kEnergyThreads) energy_cols_kernel(const Energ
         local += (double)dmin;
         if (p.d_bwd) p.d_bwd[f] = dmin;
         if (p.i_bwd) p.i_bwd[f] = i;
-        if (p.nn_cols) p.nn_cols[s] = ORDERED ? p.row_inv[i] : i;
+        if (p.nn_cols) p.nn_cols[f] = i;                         // seeds by caller index
     }
     const double s = block_sum(local, sh);
     if (threadIdx.x == 0) p.partials[blockIdx.x] = s;
@@ -146,7 +146,7 @@ __global__ void __launch_bounds__(kEnergyThreads) energy_rows_kernel(const Energ
         bool flagged = false;
         if (valid) {
             b = e / p.N;
-            s = ORDERED ? b * p.N + p.row_inv[e - b * p.N] : e;  // the search's position of this point
+            s = ORDERED ? b * p.N + p.row_inv[b * p.row_stride + e - b * p.N] : e;  // the search's position of this point
             const u64 key = p.keys_a[s];
             dmin = __uint_as_float((unsigned)(key >> 32));
             const float* a = p.src + e * 3;
@@ -169,7 +169,7 @@ __global__ void __launch_bounds__(kEnergyThreads) energy_rows_kernel(const Energ
         local += (double)dmin;
         if (p.d_fwd) p.d_fwd[e] = dmin;
         if (p.i_fwd) p.i_fwd[e] = j;
-        if (p.nn_rows) p.nn_rows[s] = ORDERED ? p.tgt_inv[b * p.M + j] : j;
+        if (p.nn_rows) p.nn_rows[e] = j;
     }
     const double s = block_sum(local, sh);
     if (threadIdx.x == 0) {

@@ -66,8 +66,14 @@ struct SymParams {
 struct CullParams {
     const float* a;               // [B,na,3] rows (skinned cloud)
     const float* b;               // [B,nb,3] columns (observed frames)
-    const int32_t* nn_rows;       // [B,na] arg-min column of every row from an EARLIER evaluation, -1: unknown
-    const int32_t* nn_cols;       // [B,nb] arg-min row of every column, -1: unknown
+    // seeds from an EARLIER evaluation, by caller index (-1: unknown): nn_rows [B,na] the arg-min caller target of every
+    // caller row, nn_cols [B,nb] the arg-min caller row of every caller target
+    const int32_t* nn_rows;
+    const int32_t* nn_cols;
+    // a, b in a search order (null: caller order): row_order / row_inv [row_stride ? B : 1, na] (search position <-> caller
+    // row; row_stride 0: one order for all frames, na: one per frame), tgt_order / tgt_inv [B,nb]
+    const int32_t* row_order; const int32_t* row_inv; const int32_t* tgt_order; const int32_t* tgt_inv;
+    int64_t row_stride;
     int B, na, nb, nb_pad;
     float* colbox;                // out [B, nb_pad/32, 8]
     float* rowbound;              // out [B, ceil(na/256)]
@@ -93,6 +99,10 @@ int launch_skin_fwd(const float* cano, const float* W, const float* R, const flo
                     float* out, float* out_packed, cudaStream_t stream);
 // order != null: the sorted copy (and out_search [T,N,3], AoS) holds the points in the order `order` [N] (search position ->
 // caller point); `out` stays in caller order
+// per-frame STR row order of the skinned cloud [T,N,3] and the search's copies in it (order.cu; N <= posed_order_max_points())
+int posed_order_max_points();
+int launch_posed_order(const float* skinned, int64_t T, int64_t N, int64_t n_pad, int32_t* row_order, int32_t* row_inv,
+                       float* out_search, float* out_packed, unsigned char* perm, float* xq, cudaStream_t stream);
 int launch_skin_fwd_sorted(const float* cano, const float* W, const float* R, const float* tr, int64_t T, int64_t N,
                            int64_t P, float* out, float* out_packed, unsigned char* perm, float* xq, int64_t n_pad,
                            cudaStream_t stream, const int32_t* order = nullptr, float* out_search = nullptr);
@@ -142,13 +152,14 @@ struct EnergyParams {
     const unsigned* col_bound;    // [1] float bits >= every column minimum (SymParams::col_bound)
     double* partials;             // [2 * energy_max_blocks()] per-block loss partials (no initialisation needed)
     unsigned* ticket;             // [1] ZERO on entry
-    int32_t* nn_rows; int32_t* nn_cols;   // optional [B,N] / [B,M]: the arg-mins, kept as the next evaluation's culling seeds
+    int32_t* nn_rows; int32_t* nn_cols;   // optional [B,N] / [B,M]: the arg-mins by caller index, the next evaluation's seeds
     float* d_fwd; int64_t* i_fwd; // optional [B,N]
     float* d_bwd; int64_t* i_bwd; // optional [B,M]
     // search in a permuted order (all null: the keys are in caller order).  The search ran on row_order / tgt_order copies
-    // (src_packed, tgt_packed, keys, tie words and nn_* are in that order); both passes still iterate in caller order.
-    const int32_t* row_order;     // [N]   search position -> caller row
-    const int32_t* row_inv;       // [N]   caller row -> search position
+    // (src_packed, tgt_packed, keys and tie words are in that order); both passes still iterate in caller order.
+    const int32_t* row_order;     // [N] or [B,N] (row_stride 0 / N): search position -> caller row
+    const int32_t* row_inv;       // same shape: caller row -> search position
+    int64_t row_stride;
     const int32_t* tgt_order;     // [B,M] per frame: search position -> caller target
     const int32_t* tgt_inv;       // [B,M]
     const unsigned* tie_a;        // [B,N] / [B,M] tie words of the search (SymParams::tie_a)

@@ -52,7 +52,7 @@ class _EngineBase:
                              f"0 <= cano_idx <= {self.total_frames}")
         self.flow_ref, self.cano_idx, self.lambda_flow, self.robust_flow = flow_ref, cano_idx, lambda_flow, robust_flow
         self.tau = torch.ones((), device=self.cano.device)
-        self.native = self.cull = self.search_culled = False
+        self.native = self.cull = self.search_culled = self.search_posed = False
         self.sink = self.assign = self.optimizer = self.bucket = None
         self._nat = self._ingest_src = self._cur_variant = None
 
@@ -263,16 +263,21 @@ class _EngineBase:
         self.search_culled = can_order and (search == "culled" or (
             search == "auto" and min(self.cano.shape[0], self.frames.shape[1]) >= SEARCH_CULLED_MIN_POINTS))
         self.search_order_rows = self.search_order_tgt = None
+        # rows: up to reart_posed_order_max_points() the search groups them per frame on the skinned cloud, every step
+        # (reart_skinned_chamfer_fwd_bwd_posed: compact blocks once the parts move apart); larger clouds keep one k-d
+        # order of the canonical cloud, fixed here
+        self.search_posed = self.search_culled and self.cano.shape[0] <= _lib.lib().reart_posed_order_max_points()
         if self.search_culled:
-            # the culled search's own order, fixed here (256-row blocks = one warp of the search, 32-target chunks); the
-            # engine's clouds, outputs and every sum stay in the caller's order.  Any order is exact, a stale one (after
+            # the culled search's own order (256-row blocks = one warp of the search, 32-target chunks); the engine's
+            # clouds, outputs and every sum stay in the caller's order.  Any order is exact, a stale one (after
             # step(ingest=...)) only culls less.
             dev = self.cano.device
-            self.search_order_rows = ops.search_order(self.cano[None], 256)[0].int()
+            if not self.search_posed:
+                self.search_order_rows = ops.search_order(self.cano[None], 256)[0].int()
+                self.search_inv_rows = torch.empty_like(self.search_order_rows)
+                self.search_inv_rows[self.search_order_rows.long()] = torch.arange(
+                    self.cano.shape[0], dtype=torch.int32, device=dev)
             self.search_order_tgt = ops.search_order(self.frames, 32).int()
-            self.search_inv_rows = torch.empty_like(self.search_order_rows)
-            self.search_inv_rows[self.search_order_rows.long()] = torch.arange(
-                self.cano.shape[0], dtype=torch.int32, device=dev)
             self.search_inv_tgt = torch.empty_like(self.search_order_tgt)
             self.search_inv_tgt.scatter_(1, self.search_order_tgt.long(), torch.arange(
                 self.frames.shape[1], dtype=torch.int32, device=dev)[None].expand_as(self.search_order_tgt).contiguous())
@@ -285,13 +290,23 @@ class _EngineBase:
         dev = self.cano.device
         b["nn_rows"] = torch.full((T, N), -1, dtype=torch.int32, device=dev)      # arg-mins of the last step (-1: none yet)
         b["nn_cols"] = torch.full((T, M), -1, dtype=torch.int32, device=dev)
+        if self.search_culled and self.search_posed:                                # this step's row order, per frame
+            b["row_order"] = torch.empty((T, N), dtype=torch.int32, device=dev)
+            b["row_inv"] = torch.empty((T, N), dtype=torch.int32, device=dev)
         # evaluated / offered (warp, chunk) pairs; ordered search: + points resolved by the exact tie path
         b["cull_stats"] = torch.zeros(3 if self.search_culled else 2, dtype=torch.int64, device=dev)
 
     def _search_energy(self, L, b, W, R, tr, T, N, M, P, gW, gR, gtr, g_skinned, compute_grad):
         """The fused energy on skinning weights W and poses (R, tr): brute-force search, or the exact culled one in the
         search order seeded by the previous step's arg-mins (bit-identical results).  Writes b["skinned"], b["loss64"]."""
-        if self.search_culled:
+        if self.search_culled and self.search_posed:
+            check(L.reart_skinned_chamfer_fwd_bwd_posed(
+                ptr(self.cano), ptr(W), ptr(R), ptr(tr), ptr(self.frames), ptr(self.frames_search),
+                ptr(self.frames_search_packed), T, N, M, P, ptr(self.search_order_tgt), ptr(self.search_inv_tgt),
+                ptr(b["row_order"]), ptr(b["row_inv"]), ptr(b["skinned"]), ptr(b["loss64"]), ptr(gW), ptr(gR), ptr(gtr),
+                ptr(g_skinned), compute_grad, None, None, None, None, ptr(b["nn_rows"]), ptr(b["nn_cols"]),
+                ptr(b["cull_stats"]), ptr(b["ws"]), b["ws_bytes"], stream_ptr()), "reart_skinned_chamfer_fwd_bwd_posed")
+        elif self.search_culled:
             check(L.reart_skinned_chamfer_fwd_bwd_ordered(
                 ptr(self.cano), ptr(W), ptr(R), ptr(tr), ptr(self.frames), ptr(self.frames_search),
                 ptr(self.frames_search_packed), T, N, M, P, ptr(self.search_order_rows), ptr(self.search_inv_rows),
@@ -480,7 +495,7 @@ class RelaxationEngine(_EngineBase):
         # cloud = one warp of the search, 32-point leaves for the observed frames = one target chunk); ``perm_cano`` /
         # ``perm_frames`` map engine order -> caller order (engine.skinned[:, k] is caller point perm_cano[k]).  Every
         # order-dependent float sum then associates differently: the same optimisation, not the same bits.  The default
-        # (search="auto") culls without this: only the search runs on k-d ordered copies (search_order_rows / _tgt).
+        # (search="auto") culls without this: only the search runs on ordered copies (_EngineBase._setup_search).
         self.cull = bool(cull)
         # fuse_producer: skin inside the search kernel's prologue (reart_skinned_chamfer_fwd_bwd_fused; SURVEY N1).  Bit-identical,
         # one launch less, but measured SLOWER than the separate skin kernel on B200 (profiles/r02_fused_producer.md), so opt-in.
