@@ -166,6 +166,20 @@ def make_small_all_reduce(ctx: DistContext, numel: int, device):
     return lambda flat: ctx.all_reduce_sum_(flat)
 
 
+def gather_frames(ctx: DistContext, x: torch.Tensor, total: int) -> torch.Tensor:
+    """The complete [total, ...] tensor of a per-frame tensor whose rows [lo, hi) each rank holds (``shard_bounds``), on
+    every rank: the uneven shards are padded to the largest one, all-gathered and trimmed.  Collective."""
+    if ctx.world_size <= 1:
+        return x
+    bounds = [shard_bounds(total, ctx.world_size, r) for r in range(ctx.world_size)]
+    rows = max(hi - lo for lo, hi in bounds)
+    pad = x.new_zeros((rows,) + tuple(x.shape[1:]))
+    pad[:x.shape[0]] = x
+    out = [torch.empty_like(pad) for _ in bounds]
+    dist.all_gather(out, pad)
+    return torch.cat([o[:hi - lo] for o, (lo, hi) in zip(out, bounds)])
+
+
 def flow_pairs_for_rank(T: int, cano_idx: int, lo: int, hi: int):
     """Which consecutive pairs of the COMPLETE sequence (canonical frame inserted at cano_idx, run_robot.py:204-207)
     a rank owning skinned frames [lo, hi) evaluates, and where each side comes from.

@@ -24,12 +24,45 @@ import torch.nn.functional as F
 
 from . import _lib, ops
 from ._lib import check, ptr, stream_ptr
-from .dist import (DistContext, GradBucket, OneShotAllReduce, flow_pairs_for_rank, flow_window_plan, halo_from_previous_rank,
-                   make_small_all_reduce, shard_bounds)
+from .dist import (DistContext, GradBucket, OneShotAllReduce, flow_pairs_for_rank, flow_window_plan, gather_frames,
+                   halo_from_previous_rank, make_small_all_reduce, shard_bounds)
 from .model import BaseModel, KinematicModel
 
 
+# ------------------------------------------------------------------------------------------ flat moment layouts
+# The native tails keep their Adam moments in flat buffers; a checkpoint stores them per parameter (state_dict name and
+# shape).  A layout is the list of (name, shape) in buffer order; name None marks a slot that is not parameter state.
+def relax_seg_layout(H: int, P: int):
+    """relax_tail_kernel's seg buffers (m_seg, v_seg, bucket): [w0 (3H) | b0 (H) | w2 (P H)] -- its e < 3H / e < 4H split."""
+    return [("seg_head.model.0.weight", (H, 3, 1)), ("seg_head.model.0.bias", (H,)), ("seg_head.model.2.weight", (P, H, 1))]
+
+
+def kin_layout(E: int, T: int, distance: bool, root: bool):
+    """kin_tail_kernel's gradient / moment buffers: [axis | moment | loss slot | theta | (distance) | (root_6d, root_t)]."""
+    spec = [("axis_list", (E, 3)), ("moment_list", (E, 3)), (None, (1,)), ("theta_list", (T, E))]
+    if distance:
+        spec.append(("distance_list", (T, E)))
+    if root:
+        spec += [("root_6d", (T, 6)), ("root_t", (T, 3))]
+    return spec
+
+
+def split_flat(flat: torch.Tensor, layout) -> dict:
+    """{name: view of ``flat`` in the parameter's shape} for a ``layout``; views, so writing them writes the buffer."""
+    out, off = {}, 0
+    for name, shape in layout:
+        n = math.prod(shape)
+        if name is not None:
+            out[name] = flat[off:off + n].view(shape)
+        off += n
+    assert off == flat.numel(), (off, flat.numel())
+    return out
+
+
 class _EngineBase:
+    KIND = None                 # "relaxation" | "kinematic": the checkpoint's engine kind
+    FRAME_KEYS = ()             # state_dict entries with one row per frame (sharded over the ranks)
+
     def __init__(self, cano: torch.Tensor, frames: torch.Tensor, ctx: Optional[DistContext], use_graph: bool, flow_ref,
                  cano_idx: int, lambda_flow: float, robust_flow: bool):
         """The set-up both engines share: the local shard of the frames, the flow-loss settings, and every attribute this
@@ -136,6 +169,132 @@ class _EngineBase:
         if self.native and (self.cull or self.search_culled):
             aux += [self._nat["nn_rows"], self._nat["nn_cols"], self._nat["cull_stats"]]
         return aux
+
+    # ------------------------------------------------------------------------------------------ checkpoint / resume
+    def _moments(self, create: bool):
+        """({parameter name: (exp_avg, exp_avg_sq)}, [step counters]): the live optimiser state in the parameters' own
+        shapes -- views of the native tail's buffers, or torch Adam's state.  torch creates that state lazily in the first
+        step: ``create`` makes it now, in place and as fused capturable Adam would (float32 device ``step``), so a later
+        capture sees existing state and snapshots it instead of zeroing it; without ``create`` missing state reads as zeros."""
+        if self.native:
+            return self._native_moments()
+        names = {id(p): n for n, p in self.model.named_parameters()}
+        out, steps = {}, []
+        for p in self._opt_params():
+            st = self.optimizer.state[p] if create else self.optimizer.state.get(p, {})
+            if create and not st:
+                st["step"] = torch.zeros((), dtype=torch.float32, device=p.device)
+                st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+                st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+            if st:
+                out[names[id(p)]] = (st["exp_avg"], st["exp_avg_sq"])
+                steps.append(st["step"])
+            else:
+                out[names[id(p)]] = (torch.zeros_like(p), torch.zeros_like(p))
+        return out, steps
+
+    def _dims(self) -> dict:
+        return dict(N=int(self.cano.shape[0]), M=int(self.frames.shape[1]), P=int(self.model.num_parts), H=None)
+
+    def _reference_extras(self) -> dict:
+        return {}
+
+    def checkpoint(self) -> dict:
+        """The state of the fit after the last completed step, as a dict of tensors (on the host), numbers, strings, lists
+        and dicts: ``torch.save`` it, and ``torch.load(..., weights_only=True)`` gives it back.
+
+        ``"state_dict"`` is ``model.state_dict()`` of the complete sequence in the reference's keys and shapes (per-frame
+        parameters gathered from the ranks), next to the reference's extras (relaxation: ``tau``, ``cano_idx``;
+        kinematic: ``seg_part``, ``cano_pc``, ``edge_index``, ``paths_to_base``, ``reverse_topo``), so code written for
+        the run scripts' ``model.pth.tar`` reads it.  ``"engine"`` holds the rest of the iteration's state: kind,
+        iteration, sizes, Adam's moments per parameter name in the complete-sequence layout (one layout for the native
+        and the autograd path) with the step count, the CUDA RNG state and the assignment's matches and duals.
+
+        Not saved: the culled search's seeds and counters (any seed gives the same search result, so a resumed step has
+        the same bits; only the first step's culling counters differ) and the clouds (the caller's, as at construction).
+        Under frame sharding every rank calls it and gets the whole dict.  Host sync; ``step()`` is unchanged by it."""
+        T = self.total_frames
+
+        def host(x, per_frame):
+            x = x.detach()
+            return (gather_frames(self.ctx, x.contiguous(), T) if per_frame else x).cpu()
+
+        sd = {k: host(v, k in self.FRAME_KEYS) for k, v in self.model.state_dict().items()}
+        moments, steps = self._moments(create=False)
+        adam = dict(step=int(round(float(steps[0]))) if steps else 0,
+                    exp_avg={k: host(m, k in self.FRAME_KEYS) for k, (m, _) in moments.items()},
+                    exp_avg_sq={k: host(v, k in self.FRAME_KEYS) for k, (_, v) in moments.items()})
+        # every rank draws the same gumbel noise from the same seed: the local generator state is every rank's
+        eng = dict(kind=self.KIND, iteration=int(self.iteration), T_total=T, **self._dims(), adam=adam,
+                   rng=torch.cuda.get_rng_state(self.cano.device))
+        if self.assign is not None:
+            a = self.assign
+            eng["assign"] = dict(num_fps=int(a.num_fps), col4row=host(a.col4row, True), dual_u=host(a.dual_u, True),
+                                 have_assignment=bool(a.have_assignment))
+        return dict(state_dict=sd, **self._reference_extras(), engine=eng)
+
+    def load_checkpoint(self, ck: dict) -> None:
+        """Continue the fit a ``checkpoint()`` dict describes: parameters, Adam's moments and step count, the RNG state,
+        the assignment's state and the iteration counter, each rank taking its own frames (a checkpoint of any world size
+        loads on any other).  Everything is copied into the engine's existing tensors, so graphs captured before stay
+        valid; it works before the first step too.  A reference-layout dict without ``"engine"`` (a shipped
+        ``model.pth.tar``) loads the parameters and starts the optimiser afresh at iteration 0, as the run scripts'
+        ``--resume`` does.  Raises ValueError, naming the field, when the checkpoint does not fit this engine."""
+        eng = ck.get("engine")
+        sd = ck["state_dict"]
+        T = self.total_frames
+        if eng is not None:
+            mine = dict(kind=self.KIND, T_total=T, **self._dims())
+            for field, want in mine.items():
+                if eng.get(field) != want:
+                    raise ValueError(f"checkpoint {field} is {eng.get(field)!r}, this engine's is {want!r}")
+        own = self.model.state_dict(keep_vars=True)
+        if set(sd) != set(own):
+            raise ValueError(f"checkpoint parameter set differs from this engine's: missing {sorted(set(own) - set(sd))}, "
+                             f"extra {sorted(set(sd) - set(own))}")
+        for k, v in own.items():
+            want = ((T,) + tuple(v.shape[1:])) if k in self.FRAME_KEYS else tuple(v.shape)
+            if tuple(sd[k].shape) != want:
+                raise ValueError(f"checkpoint {k} has shape {tuple(sd[k].shape)}, this engine needs {want}")
+        if eng is not None:
+            names = sorted(self._moments(create=False)[0])
+            for part in ("exp_avg", "exp_avg_sq"):
+                if sorted(eng["adam"][part]) != names:
+                    raise ValueError(f"checkpoint adam {part} holds {sorted(eng['adam'][part])}, this engine optimises {names}")
+            if ("assign" in eng) != (self.assign is not None):
+                raise ValueError("checkpoint assign state " + ("is present but this engine has no assignment loss"
+                                                              if "assign" in eng else "is missing for this engine's assignment loss"))
+            if self.assign is not None and eng["assign"]["num_fps"] != self.assign.num_fps:
+                raise ValueError(f"checkpoint assign num_fps is {eng['assign']['num_fps']}, this engine's is {self.assign.num_fps}")
+        moments, steps = self._moments(create=True)
+        lo, hi = self.frame_range
+
+        def local(x, key):
+            return x[lo:hi] if key in self.FRAME_KEYS else x
+
+        with torch.no_grad():
+            for k, v in own.items():
+                v.copy_(local(sd[k], k))
+            for k, (m, v) in moments.items():
+                if eng is None:
+                    m.zero_(); v.zero_()
+                else:
+                    m.copy_(local(eng["adam"]["exp_avg"][k], k)); v.copy_(local(eng["adam"]["exp_avg_sq"][k], k))
+            for s in steps:
+                s.fill_(0 if eng is None else float(eng["adam"]["step"]))
+            if self.assign is not None:
+                a = self.assign
+                if eng is None:
+                    a.col4row.zero_(); a.dual_u.zero_(); a.have_assignment = False
+                else:
+                    a.col4row.copy_(eng["assign"]["col4row"][lo:hi]); a.dual_u.copy_(eng["assign"]["dual_u"][lo:hi])
+                    a.have_assignment = bool(eng["assign"]["have_assignment"])
+            if "tau" in ck:
+                self.tau.fill_(float(ck["tau"]))
+        self.iteration = 0 if eng is None else int(eng["iteration"])
+        if eng is not None:
+            torch.cuda.set_rng_state(eng["rng"], self.cano.device)
+        torch.cuda.synchronize()
 
     # ------------------------------------------------------------------------------------------ iteration flavours
     def _setup_assign(self, assign: Optional[dict], sample=None):
@@ -464,6 +623,8 @@ SEARCH_CULLED_MIN_POINTS = 8192
 class RelaxationEngine(_EngineBase):
     """Relaxation model (networks/model.py BaseModel) + recon loss (+ the optional assignment and flow losses),
     frame-sharded."""
+    KIND = "relaxation"
+    FRAME_KEYS = ("proposal_6d", "proposal_t")
 
     def __init__(self, cano: torch.Tensor, frames: torch.Tensor, num_parts: int, ctx: Optional[DistContext] = None,
                  trans_lr: float = 1e-2, seg_lr: float = 1e-3, weight_decay: float = 0.0, use_graph: bool = True,
@@ -678,10 +839,28 @@ class RelaxationEngine(_EngineBase):
         R, tr = self.model.pose()
         return weight, R, tr
 
+    # ------------------------------------------------------------------------------------------ checkpoint layout
+    def _native_moments(self):
+        b = self._nat
+        _, _, _, P, H = b["dims"]
+        lay = relax_seg_layout(H, P)
+        out = {k: (m, v) for (k, m), v in zip(split_flat(b["m_seg"], lay).items(), split_flat(b["v_seg"], lay).values())}
+        out["proposal_6d"] = (b["m_d6"], b["v_d6"])
+        out["proposal_t"] = (b["m_tr"], b["v_tr"])
+        return out, [b["step"]]
+
+    def _dims(self) -> dict:
+        return dict(super()._dims(), H=int(self.model.seg_head.model[0].weight.shape[0]))
+
+    def _reference_extras(self) -> dict:
+        return dict(tau=float(self.tau), cano_idx=int(self.cano_idx))
+
 
 class KinematicEngine(_EngineBase):
     """Projection model (networks/model.py KinematicModel) + recon loss (+ the optional assignment and flow losses),
     frame-sharded.  axis/moment are shared (all-reduced); theta/distance/root pose are per frame."""
+    KIND = "kinematic"
+    FRAME_KEYS = ("theta_list", "distance_list", "root_6d", "root_t")
 
     def __init__(self, model_kwargs: dict, seg_part: torch.Tensor, cano: torch.Tensor, frames: torch.Tensor,
                  ctx: Optional[DistContext] = None, lr: float = 1e-2, weight_decay: float = 0.0,
@@ -733,6 +912,25 @@ class KinematicEngine(_EngineBase):
     def _weights_and_poses(self):
         trans = self.model.transforms()
         return self.weight, trans[:, :, :3, :3].contiguous(), trans[:, :, :3, 3].contiguous()
+
+    # ------------------------------------------------------------------------------------------ checkpoint layout
+    def _native_moments(self):
+        b, m = self._nat, self.model
+        T, _, _, P = b["dims"]
+        lay = kin_layout(P - 1, T, hasattr(m, "distance_list"), hasattr(m, "root_6d") and hasattr(m, "root_t"))
+        ms, vs = split_flat(b["m"], lay), split_flat(b["v"], lay)
+        return {k: (ms[k], vs[k]) for k in ms}, [b["step"]]
+
+    def _reference_extras(self) -> dict:
+        m = self.model
+        key = lambda k: k if isinstance(k, str) else int(k)
+        ex = dict(seg_part=m.seg_part.detach().cpu(), cano_pc=self.cano.detach().cpu(),
+                  edge_index={key(k): int(v) for k, v in m.edge_index.items()},
+                  paths_to_base={key(k): [int(x) for x in v] for k, v in m.paths_to_base.items()},
+                  reverse_topo=[int(x) for x in m.reverse_topo])
+        if m.joint_type_list is not None:
+            ex["joint_type_list"] = [str(j) for j in m.joint_type_list]
+        return ex
 
     # ------------------------------------------------------------------------------------------ native fused iteration
     def _init_native(self, lr, weight_decay, betas, eps):
@@ -860,14 +1058,18 @@ def tau_schedule(i: int, n_iter: int, start_tau: float, end_tau: float) -> float
 
 
 def fit_relaxation(cano: torch.Tensor, frames: torch.Tensor, num_parts: int, n_iter: int, ctx: Optional[DistContext] = None,
-                   start_tau: float = 5.0, end_tau: float = 1.0, log_every: int = 0, **engine_kwargs):
+                   start_tau: float = 5.0, end_tau: float = 1.0, log_every: int = 0, resume: Optional[dict] = None,
+                   **engine_kwargs):
     """The relaxation optimisation of run_robot.py:153-221 (recon loss, cosine tau schedule :86,157) on the engine.
     Returns (engine, losses) where ``losses`` holds the all-rank loss every ``log_every`` iterations (0: only the
-    last) -- reading it is the only host sync."""
+    last) -- reading it is the only host sync.  ``resume``: a ``checkpoint()`` dict; the fit loads it and runs the
+    remaining iterations ``resume["engine"]["iteration"] .. n_iter - 1`` of the same schedule."""
     eng = RelaxationEngine(cano, frames, num_parts, ctx=ctx, **engine_kwargs)
+    if resume is not None:
+        eng.load_checkpoint(resume)
     losses = []
     loss = None
-    for i in range(n_iter):
+    for i in range(eng.iteration, n_iter):
         loss = eng.step(tau_schedule(i, n_iter, start_tau, end_tau))
         if log_every and (i % log_every == 0):
             losses.append(float(loss))
